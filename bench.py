@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: 512x512 Unet-VGG16 (21 classes) training throughput, batch 16 per GPU, data parallel.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one iteration of the reference's fit_one_epoch body (utils/utils_fit.py:26-97): forward, CE + Dice
 (+ f_score), backward, gradient all-reduce (N > 1), Adam step, on one synthetic batch of 16 images per GPU.
@@ -15,6 +15,8 @@ Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for every key.
   cpu_baseline the oracle (a torch-CPU restatement of the reference path; the reference itself is Python and does
                not travel to the GPU box) timed on this box's host cores on a bounded sample
   --impl reference   times that same CPU path with all host threads and prints the reference-arm line
+  --dump-outputs DIR writes what the last timed step computed as DIR/<name>.npy (see dump_outputs), so that two builds
+                     can be compared output for output on identical seeded inputs
 """
 import argparse
 import json
@@ -36,6 +38,8 @@ WORKLOAD = ("Unet-VGG16 21-class 512x512 training step (fwd + CE + Dice + f_scor
             "batch 16 per GPU, BASELINE configs[1]")
 # fprop + dgrad + wgrad conv FLOPs per image (SURVEY.md 8d)
 TRAIN_GFLOP_PER_IMG = 1351.99
+# parameter / gradient values per --dump-outputs array: 16 MB each in float32
+DUMP_SAMPLE = 1 << 22
 
 
 def _peaks():
@@ -143,6 +147,22 @@ class OperandBytes:
     def __exit__(self, *exc):
         for name, fn in self.saved.items():
             setattr(self.ops, name, fn)
+
+
+def dump_outputs(trainer, out, path):
+    """What the last timed step hands its caller: the [loss, f_score] it returns and the model state it leaves behind --
+    the updated parameters and the gradients it applied (summed over ranks), concatenated in state_dict order.  Of those
+    24.9 M values, DUMP_SAMPLE fixed positions (numpy Generator seeded 0, sorted) are written."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    params = torch.cat([trainer.params[n].reshape(-1) for n in trainer.names])
+    grads = torch.cat([trainer.grads[n].reshape(-1) for n in trainer.names])
+    idx = np.sort(np.random.default_rng(0).choice(params.numel(), size=min(DUMP_SAMPLE, params.numel()), replace=False))
+    idx = torch.from_numpy(idx).to(params.device)
+    arrays = {"loss": out[0], "f_score": out[1], "params_sample": params[idx], "grads_sample": grads[idx]}
+    for name, t in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), t.detach().float().cpu().numpy())
 
 
 def _ev_ms(fn, iters, warm):
@@ -376,7 +396,7 @@ def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    steps = max(1, min(args.steps, 3))
+    steps = args.steps
     warmup = 1 if args.warmup > 0 else 0
     v, s_per_step, threads, batch, kind = cpu_path_img_per_s(steps, warmup)
     cpu_model = ""
@@ -465,6 +485,8 @@ def run_ours(args):
     launches = int(lib.b2u_launch_count())
     clocks = sampler.stop() if rank == 0 else None
     loss_val = out.tolist()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(trainer, out, args.dump_outputs)
     if args.kernels_only:
         if rank == 0:
             print(json.dumps({"kernels_only": True, "note": "profiling pass, not a bench value", "steps": K, "warmup": W,
@@ -617,7 +639,14 @@ def main():
     ap.add_argument("--kernels-only", action="store_true",
                     help="profiling pass (ncu): warm-up + the K device-resident steps, nothing else; prints a reduced line that is NOT a bench value")
     ap.add_argument("--detail", default=None, help="write the per-layer conv kernel timing table (JSON) here")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last timed step's loss, f_score and a fixed sample of the updated "
+                         "parameters and of the gradients as DIR/<name>.npy (float32, 32 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the product path (--impl ours)")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.impl == "reference":

@@ -717,6 +717,57 @@ def ulu_train_step(sd, imgs, pngs, cls_weights, num_classes, variant, dice=True,
     return loss.detach(), logits.detach(), dict(zip(names, grads)), stats
 
 
+# ----------------------------------------------------------------------------------------------- ImprovedSegNet (RepVGG_Unet)
+def _isn_block(sd, stats, p, x, training, deploy):
+    """LightweightConvBlock(use_repvgg=True) (nets/RepVGG_Unet.py): 1x1 conv (+bias), BN, ReLU, then RepVGGBlock(mid -> out).
+    Training form: relu(bn1(conv3x3(y)) + bn2(conv1x1(y))), both convs bias-free (no identity branch: mid != out in every
+    block); deploy form: relu(reparam_conv(y))."""
+    y = _rn_bn(sd, stats, p + ".conv.1", F.conv2d(x, sd[p + ".conv.0.weight"], sd[p + ".conv.0.bias"]), training, True)
+    r = p + ".conv.3"
+    if deploy:
+        return F.relu(F.conv2d(y, sd[r + ".reparam_conv.weight"], sd[r + ".reparam_conv.bias"], padding=1))
+    b3 = _rn_bn(sd, stats, r + ".bn1", F.conv2d(y, sd[r + ".conv1.weight"], padding=1), training, False)
+    b1 = _rn_bn(sd, stats, r + ".bn2", F.conv2d(y, sd[r + ".conv2.weight"]), training, False)
+    return F.relu(b3 + b1)
+
+
+def isn_forward(sd, x, training=True, stats=None, deploy=False):
+    """ImprovedSegNet(use_repvgg=True).forward without Dropout: the topology of UltraLightweightUnet_large_optimized
+    (ulu_forward: widths 44-88-176-352-704, SE after each encoder stage, cat[upsampled, skip]) with LightweightConvBlock in
+    place of LightConvBlock.  deploy=True runs the re-parameterised blocks (isn_deploy_params)."""
+    if stats is None:
+        stats = {k: v.clone() for k, v in sd.items() if "running_" in k or "num_batches" in k}
+    skips = []
+    for i in range(1, 5):
+        if i > 1:
+            x = _pinned_max_pool(x, f"p{i}")
+        x = _ulu_se(sd, f"se{i}", _isn_block(sd, stats, f"enc{i}", x, training, deploy), False)
+        skips.append(x)
+    x = _isn_block(sd, stats, "bridge", _pinned_max_pool(x, "p5"), training, deploy)
+    for k in (4, 3, 2, 1):
+        skip = skips[k - 1]
+        up = F.interpolate(x, size=skip.shape[2:], mode="bilinear", align_corners=True)
+        x = _isn_block(sd, stats, f"dec{k}", torch.cat([up, skip], 1), training, deploy)
+    return F.conv2d(x, sd["final.weight"], sd["final.bias"]), stats
+
+
+def isn_deploy_params(sd, eps=1e-5):
+    """switch_to_deploy (nets/RepVGG_Unet.py): every RepVGGBlock's conv3x3 + BN and conv1x1 + BN branches, the BatchNorms in
+    eval form, become one conv3x3 with bias (`reparam_conv`); the 1x1 kernel sits at the centre tap.  The training-form
+    tensors stay in the state_dict."""
+    out = dict(sd)
+    for key in [k for k in sd if k.endswith(".conv.3.conv1.weight")]:
+        r = key[:-len(".conv1.weight")]
+        folded = []
+        for conv, bn in ((".conv1", ".bn1"), (".conv2", ".bn2")):
+            scale = sd[r + bn + ".weight"] / torch.sqrt(sd[r + bn + ".running_var"] + eps)
+            w = sd[r + conv + ".weight"] * scale.view(-1, 1, 1, 1)
+            folded.append((F.pad(w, (1, 1, 1, 1)) if w.shape[-1] == 1 else w, sd[r + bn + ".bias"] - sd[r + bn + ".running_mean"] * scale))
+        out[r + ".reparam_conv.weight"] = folded[0][0] + folded[1][0]
+        out[r + ".reparam_conv.bias"] = folded[0][1] + folded[1][1]
+    return out
+
+
 # ----------------------------------------------------------------------------------------------- LightweightUnet
 LW_WIDTHS = (24, 48, 96, 192, 384)                     # nets/LightWeightUnet.py:62-90
 

@@ -9,7 +9,7 @@ dev = torch.device("cuda:0")
 fam, C, med = sys.argv[1] if len(sys.argv) > 1 else "unet_vgg", 2, True
 model, T = WP.build_reference(fam, C); model = model.to(dev)
 WP.warm_up(model, T, C, 512, 4, 200, dev, medical=med)
-sd = {k: v.detach().clone() for k, v in model.state_dict().items()}
+sd = {k: v.detach().clone() for k, v in model.reference_state_dict().items()}
 imgs, pngs = WP.make_batch(8, C, 512, 7, med, dev)
 z64, g64, l64 = WP.run_reference(model, T, imgs, pngs, C, torch.float64)
 za, ga, la = WP.run_reference(model, T, imgs, pngs, C, torch.float32, autocast=True)

@@ -43,6 +43,26 @@ class RoundBwd(torch.autograd.Function):
         return g.to(torch.bfloat16).to(g.dtype)
 
 
+# family -> module and class of the reference (the rounding sites are hooked on its nn.Conv2d / nn.Linear modules)
+REFERENCE_CLASSES = {"unet_vgg": ("nets.unet", "Unet"), "unet_resnet50": ("nets.unet", "Unet"),
+                     "traditional": ("nets.TraditionalUnet", "TraditionalUnet"), "lightweight": ("nets.LightWeightUnet", "LightweightUnet"),
+                     "ultralight": ("nets.UltraLightweightUnet", "UltraLightweightUnet"),
+                     "ultralight_large": ("nets.UltraLightweightUnet_large", "UltraLightweightUnet_large"),
+                     "ultralight_large_optimized": ("nets.UltraLightweightUnet_large_optimized", "UltraLightweightUnet_large_optimized")}
+
+
+def build_reference(fam, C, WP, seed=11):
+    """The unmodified reference module staged under baseline/_ref (baseline/stage_ref.py), Dropout disabled, and its losses."""
+    from baseline import stage_ref
+    mod, cls = REFERENCE_CLASSES[fam]
+    torch.manual_seed(seed)
+    model = getattr(stage_ref.import_reference(mod), cls)(**WP.FAMILIES[fam][0](C))
+    for m in model.modules():
+        if isinstance(m, (torch.nn.Dropout, torch.nn.Dropout2d)):
+            m.p = 0.0
+    return model, stage_ref.import_reference("nets.unet_training")
+
+
 def run(model, T, imgs, pngs, C, sites, WP):
     m = copy.deepcopy(model).double().train()
     convs = [mod for mod in m.modules() if isinstance(mod, torch.nn.Conv2d)]
@@ -98,7 +118,7 @@ def main():
         fam, C = item.split(":")
         C = int(C)
         medical = C == 2
-        model, T = WP.build_reference(fam, C)
+        model, T = build_reference(fam, C, WP)
         model = model.to(dev)
         WP.warm_up(model, T, C, args.hw, 4, args.warm, dev, lr=args.lr, medical=medical)
         imgs, pngs = WP.make_batch(args.batch, C, args.hw, 7, medical, dev)

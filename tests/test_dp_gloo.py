@@ -71,8 +71,10 @@ def test_gradient_sync_is_mean_of_shards():
 
 
 def _ddp_reference_worker(rank, world, port, out):
-    """The UNMODIFIED reference model under DistributedDataParallel (gloo, CPU) exactly as train.py:346 wraps it, next to this
-    package's GradientSync fed with the same per-shard gradients: both must produce the mean of the shard gradients."""
+    """The reference model under DistributedDataParallel (gloo, CPU) exactly as train.py:346 wraps it, next to this package's
+    GradientSync fed with the same per-shard gradients: both must produce the mean of the shard gradients.  The reference
+    model and losses are the oracle's restatement (nets/unet.py::Unet, CE_Loss, Dice_loss), which tests/test_oracle.py pins
+    to the reference's own outputs stored under tests/golden/."""
     os.environ["MASTER_ADDR"] = "127.0.0.1"
     os.environ["MASTER_PORT"] = str(port)
     dist.init_process_group("gloo", rank=rank, world_size=world)
@@ -81,26 +83,30 @@ def _ddp_reference_worker(rank, world, port, out):
         root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
         if root not in sys.path:
             sys.path.insert(0, root)
-        from baseline import stage_ref
         from oracle import unet_oracle as O
-        import unet_pytorch_b200 as b2u
         from unet_pytorch_b200.trainer import FlatBuckets, GradientSync, _backward_order
+
+        class RefUnet(torch.nn.Module):
+            def __init__(self, params):
+                super().__init__()
+                self.names = list(params)
+                self.weights = torch.nn.ParameterList(torch.nn.Parameter(v.clone()) for v in params.values())
+
+            def forward(self, x):
+                return O.unet_forward(dict(zip(self.names, self.weights)), x)
+
         C = 3
-        RefUnet = stage_ref.import_reference("nets.unet").Unet
-        T = stage_ref.import_reference("nets.unet_training")
         params = O.make_params(C, seed=11)
-        torch.manual_seed(0)
-        model = RefUnet(num_classes=C, pretrained=False, backbone="vgg")
-        model.load_state_dict(params)
+        model = RefUnet(params)
         ddp = torch.nn.parallel.DistributedDataParallel(model, find_unused_parameters=True)      # train.py:346
         imgs, pngs = O.make_inputs(4, C, 32, 32, seed=21)
         n = imgs.shape[0] // world
         xs, ys = imgs[rank * n:(rank + 1) * n], pngs[rank * n:(rank + 1) * n]      # DistributedSampler shard (train.py:425-427)
         w = torch.ones(C)
         out_logits = ddp(xs)
-        loss = T.CE_Loss(out_logits, ys, w, num_classes=C) + T.Dice_loss(out_logits, O.one_hot(ys, C))
+        loss = O.ce_loss(out_logits, ys, w, C) + O.dice_loss(out_logits, O.one_hot(ys, C))
         loss.backward()
-        ddp_grads = {k: p.grad.detach().clone() for k, p in model.named_parameters()}
+        ddp_grads = {k: p.grad.detach().clone() for k, p in zip(model.names, model.weights)}
         # oracle gradient of THIS shard alone (each rank normalises CE / Dice over its own shard, utils_fit.py:70-81)
         _, _, shard = O.train_step(params, xs, ys, w, C, dice=True)
         shapes = {k: tuple(v.shape) for k, v in params.items()}
@@ -122,13 +128,8 @@ def _ddp_reference_worker(rank, world, port, out):
 
 
 def test_reference_under_ddp_equals_bucketed_mean_of_shards():
-    import sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    sys.path.insert(0, root)
-    from baseline import stage_ref
-    import pytest
-    if stage_ref.stage() is None or not stage_ref.available():
-        pytest.skip("baseline/_ref is not staged")
+    """Runs the oracle's restatement of the reference Unet-VGG16 (not the reference module itself) under gloo-DDP: its
+    averaged gradients must equal GradientSync's bucketed mean of the per-shard oracle gradients."""
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
     port = _free_port()

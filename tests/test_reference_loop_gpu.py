@@ -129,33 +129,30 @@ def test_lightweight_unet_non_rgb_inputs(b2u, cuda_device, cin, build):
     graph engine zero-pads the image to one 64-channel block (two-term bf16 split while 2C <= 64).  Tiny random-init fixture in
     training mode (BatchNorm over 2 x 4 x 4 samples at the bridge): the fp32 validation build pins the engine's logic to the
     reference (1e-4), the product bf16 path is held to the noise level such fixtures show for every BatchNorm family
-    (tests/test_model_gpu.py, `_direct`)."""
-    S = _staged()
-    if S is None:
-        pytest.skip("baseline/_ref is not staged")
+    (tests/test_model_gpu.py, `_direct`).  The reference is the oracle's restatement of LightweightUnet.forward (pinned to the
+    reference's own outputs by tests/test_oracle.py) in training mode without Dropout, on the weights the module's
+    constructor draws (the drop-in keeps the reference's module tree and init)."""
     zb, gb = (1e-1, 1.0) if build == "bf16" else (1e-4, 2e-2)      # measured: 4.0-5.4e-2 / 6.0-6.2e-1 (bf16), 1.3e-5 / 9.3e-3 (fp32)
     torch.manual_seed(3)
-    ref = S.import_reference("nets.LightWeightUnet").LightweightUnet(num_classes=3, in_channels=cin)
-    for m in ref.modules():
-        if isinstance(m, torch.nn.Dropout2d):
-            m.p = 0.0
-    ref = ref.to(cuda_device).train()
+    sd = b2u.LightweightUnet(num_classes=3, in_channels=cin).state_dict()
+    ref = {k: (v.to(cuda_device).requires_grad_(True) if v.is_floating_point() and "running_" not in k else v.to(cuda_device))
+           for k, v in sd.items()}
     with _build(b2u, build):
         ours = b2u.LightweightUnet(num_classes=3, in_channels=cin)
-        ours.load_state_dict(ref.state_dict())
+        ours.load_state_dict(sd)
         ours = ours.to(cuda_device).train()
         for ins in ours._engine_for(cuda_device).program:
             if ins["op"] == "drop":
                 ins["p"] = 0.0
         x = torch.rand(2, cin, 64, 64, device=cuda_device)
-        zr = ref(x)
+        zr, _ = O.lw_forward(ref, x, training=True)
         zo = ours(x)
         assert zo.shape == zr.shape
         zerr = ((zo - zr).norm() / zr.norm()).item()
         zr.square().mean().backward()
         zo.square().mean().backward()
         w = "backbone.stage1.0.conv.0.weight"
-        gr = dict(ref.named_parameters())[w].grad
+        gr = ref[w].grad
         go = dict(ours.named_parameters())[w].grad
         gerr = ((go - gr).norm() / gr.norm()).item()
         print(f"\n[LightweightUnet in_channels={cin} {build}] logits {zerr:.2e} first-conv gradient {gerr:.2e}")
@@ -166,64 +163,65 @@ def test_lightweight_unet_non_rgb_inputs(b2u, cuda_device, cin, build):
 @pytest.mark.parametrize("build", ["bf16", "fp32"])
 def test_repvgg_improved_segnet_train_and_deploy(b2u, cuda_device, build):
     """nets/RepVGG_Unet.py::ImprovedSegNet (SURVEY 8(f) rank 4): the training form (two conv + BatchNorm branches per RepVGGBlock)
-    against the staged reference in fp32 on the GPU -- logits, loss gradients, BatchNorm running statistics -- and the deploy form
-    after `switch_to_deploy()` (one re-parameterised conv3x3 + bias + ReLU per block, eval mode) against the reference's own
-    deployed model.  The training form sums two BatchNorm branches per block over as few as 4 x 4 x 4 samples on this tiny
-    random-init fixture, which amplifies bf16 rounding far beyond the other families: the fp32 validation build pins the
-    program's logic (logits 2e-5, gradients 1.4e-3 measured), the product path is a regression guard there and is held to
-    5e-2 in the deploy form, where no batch statistics are involved."""
-    S = _staged()
-    if S is None:
-        pytest.skip("baseline/_ref is not staged")
+    against the reference in fp32 on the GPU -- logits, loss gradients, BatchNorm running statistics -- and the deploy form
+    after `switch_to_deploy()` (one re-parameterised conv3x3 + bias + ReLU per block, eval mode) against the reference's
+    deployed model.  The reference is the oracle's restatement (oracle.isn_forward / isn_deploy_params: the topology, SE
+    blocks, BatchNorm and pooling of ulu_forward, which tests/test_oracle.py pins to the reference's own outputs, with the
+    RepVGG block in place of the depthwise one).  The training form sums two BatchNorm branches per block over as few as
+    4 x 4 x 4 samples on this tiny random-init fixture, which amplifies bf16 rounding far beyond the other families: the fp32
+    validation build pins the program's logic (logits 2e-5, gradients 1.4e-3 measured), the product path is a regression guard
+    there and is held to 5e-2 in the deploy form, where no batch statistics are involved."""
     with _build(b2u, build):
-        _repvgg_case(b2u, cuda_device, S, build)
+        _repvgg_case(b2u, cuda_device, build)
 
 
-def _repvgg_case(b2u, cuda_device, S, build):
+def _repvgg_case(b2u, cuda_device, build):
     zb, gb, sb, db_, ab = (5e-1, 1.0, 1e-1, 5e-2, 0.95) if build == "bf16" else (1e-4, 5e-3, 1e-4, 1e-4, 0.999)
     dev = cuda_device
     C = 4
     torch.manual_seed(5)
-    ref = S.import_reference("nets.RepVGG_Unet").ImprovedSegNet(num_classes=C)
-    ref.dropout.p = 0.0
-    ref = ref.to(dev).train()
+    sd = b2u.ImprovedSegNet(num_classes=C).state_dict()          # the module's own init (the reference's module tree)
+    ref = {k: (v.to(dev).requires_grad_(True) if v.is_floating_point() and "running_" not in k else v.to(dev))
+           for k, v in sd.items()}
     ours = b2u.ImprovedSegNet(num_classes=C)
-    assert list(ours.state_dict().keys()) == list(ref.state_dict().keys())
-    ours.load_state_dict(ref.state_dict())
+    ours.load_state_dict(sd)
     ours = ours.to(dev).train()
     for ins in ours._engine_for(dev).program:
         if ins["op"] == "drop":
             ins["p"] = 0.0
     imgs, pngs = O.make_inputs(4, C, 64, 64, seed=17)
     imgs, pngs = imgs.to(dev), pngs.to(dev)
-    T = S.import_reference("nets.unet_training")
     w = torch.ones(C, device=dev)
     labels = O.one_hot(pngs.cpu(), C).to(dev)
-    zr = ref(imgs)
-    (T.CE_Loss(zr, pngs, w, num_classes=C) + T.Dice_loss(zr, labels)).backward()
+    zr, stats = O.isn_forward(ref, imgs, training=True)
+    live_names = [k for k, v in ref.items() if v.requires_grad]
+    gr = dict(zip(live_names, torch.autograd.grad(O.ce_loss(zr, pngs, w, C) + O.dice_loss(zr, labels), [ref[k] for k in live_names])))
     zo = ours(imgs)
     (b2u.CE_Loss(zo, pngs, w, num_classes=C) + b2u.Dice_loss(zo, labels)).backward()
     zerr = ((zo - zr).norm() / zr.norm()).item()
-    gr = {k: p.grad for k, p in ref.named_parameters()}
     go = {k: p.grad for k, p in ours.named_parameters()}
-    live = [k for k in gr if gr[k] is not None and gr[k].norm().item() > 1e-9]
+    live = [k for k in gr if gr[k].norm().item() > 1e-9]
     num = sum((go[k] - gr[k]).double().pow(2).sum().item() for k in live)
     den = sum(gr[k].double().pow(2).sum().item() for k in live)
     gerr = (num / den) ** 0.5
     print(f"\n[ImprovedSegNet train {build}] logits {zerr:.2e} grads {gerr:.2e}")
     assert zerr <= zb and gerr <= gb
-    for (k, a), (_, b) in zip(ours.named_buffers(), ref.named_buffers()):
+    for k, a in ours.named_buffers():
         if k.endswith("running_mean") or k.endswith("running_var"):
+            b = stats[k]
             assert ((a - b).norm() / (b.norm() + 1e-12)).item() <= sb, k
     # deploy: fold every RepVGGBlock, eval mode
     # (the deploy form is built from identical states: the training step above left bf16-level differences in the running statistics)
-    ours.load_state_dict(ref.state_dict())
-    ref.eval(); ref.switch_to_deploy()
+    ref_sd = {k: v.detach() for k, v in ref.items()}
+    ref_sd.update(stats)
+    ours.load_state_dict(ref_sd)
     ours.eval(); ours.switch_to_deploy()
-    for k in ref.state_dict():
-        assert torch.allclose(ours.state_dict()[k], ref.state_dict()[k], rtol=1e-5, atol=1e-6), k
+    deployed = O.isn_deploy_params(ref_sd)
+    assert sorted(ours.state_dict()) == sorted(deployed)
+    for k in deployed:
+        assert torch.allclose(ours.state_dict()[k], deployed[k], rtol=1e-5, atol=1e-6), k
     with torch.no_grad():
-        dr = ref(imgs)
+        dr, _ = O.isn_forward(deployed, imgs, training=False, deploy=True)
         do = ours(imgs)
     derr = ((do - dr).norm() / dr.norm()).item()
     print(f"[ImprovedSegNet deploy {build}] logits {derr:.2e}")

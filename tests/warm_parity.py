@@ -1,7 +1,7 @@
 """Warm, structured 512x512 parity fixtures (VERDICT r1 item 1, SURVEY.md 8c(5) / section 7 hard part 6).
 
-For one model family: build the REFERENCE model (the staged, unmodified reference under baseline/_ref when present, the
-oracle restatement otherwise) on the GPU in fp32 (TF32 off), train it for a few hundred Adam steps on structured
+For one model family: build the REFERENCE model (the oracle's restatement of the reference, oracle/unet_oracle.py, which
+tests/test_oracle.py pins to the reference's own outputs stored under tests/golden/) on the GPU in fp32 (TF32 off), train it for a few hundred Adam steps on structured
 synthetic batches so the logits have margins (a mid-training state instead of near-tied random init), then on one held-out
 structured batch compare, against the reference evaluated in FLOAT64 on the same weights:
 
@@ -17,6 +17,7 @@ import copy
 import os
 import sys
 import time
+import types
 
 import torch
 import torch.nn.functional as F
@@ -27,40 +28,75 @@ if ROOT not in sys.path:
 
 from oracle import unet_oracle as O  # noqa: E402
 
-# family -> (reference module, class, ctor kwargs builder, product class name, medical inputs?)
+# family -> (ctor kwargs builder, class name of the reference module and of its drop-in)
 FAMILIES = {
-    "unet_vgg": ("nets.unet", "Unet", lambda C: dict(num_classes=C, pretrained=False, backbone="vgg"), "Unet"),
-    "unet_resnet50": ("nets.unet", "Unet", lambda C: dict(num_classes=C, pretrained=False, backbone="resnet50"), "Unet"),
-    "traditional": ("nets.TraditionalUnet", "TraditionalUnet", lambda C: dict(in_channels=3, num_classes=C), "TraditionalUnet"),
-    "lightweight": ("nets.LightWeightUnet", "LightweightUnet", lambda C: dict(num_classes=C), "LightweightUnet"),
-    "ultralight": ("nets.UltraLightweightUnet", "UltraLightweightUnet", lambda C: dict(num_classes=C), "UltraLightweightUnet"),
-    "ultralight_large": ("nets.UltraLightweightUnet_large", "UltraLightweightUnet_large", lambda C: dict(num_classes=C),
-                         "UltraLightweightUnet_large"),
-    "ultralight_large_optimized": ("nets.UltraLightweightUnet_large_optimized", "UltraLightweightUnet_large_optimized",
-                                   lambda C: dict(num_classes=C), "UltraLightweightUnet_large_optimized"),
+    "unet_vgg": (lambda C: dict(num_classes=C, pretrained=False, backbone="vgg"), "Unet"),
+    "unet_resnet50": (lambda C: dict(num_classes=C, pretrained=False, backbone="resnet50"), "Unet"),
+    "traditional": (lambda C: dict(in_channels=3, num_classes=C), "TraditionalUnet"),
+    "lightweight": (lambda C: dict(num_classes=C), "LightweightUnet"),
+    "ultralight": (lambda C: dict(num_classes=C), "UltraLightweightUnet"),
+    "ultralight_large": (lambda C: dict(num_classes=C), "UltraLightweightUnet_large"),
+    "ultralight_large_optimized": (lambda C: dict(num_classes=C), "UltraLightweightUnet_large_optimized"),
 }
 
 
-def reference_available():
-    try:
-        from baseline import stage_ref
-        return stage_ref.stage() is not None and stage_ref.available()
-    except Exception:
-        return False
+def _oracle_forward(family):
+    """(state_dict, x, training, stats) -> (logits, stats): the oracle's forward of the family."""
+    if family == "unet_vgg":
+        return lambda sd, x, training, stats: (O.unet_forward(sd, x), stats)
+    if family.startswith("ultralight"):
+        return lambda sd, x, training, stats: O.ulu_forward(sd, x, family, training=training, stats=stats)
+    fwd = {"unet_resnet50": O.resnet_unet_forward, "traditional": O.trad_forward, "lightweight": O.lw_forward}[family]
+    return lambda sd, x, training, stats: fwd(sd, x, training=training, stats=stats)
+
+
+class OracleReference(torch.nn.Module):
+    """One model family of the reference as the oracle computes it, without Dropout: the trainable tensors of its state_dict
+    are parameters, the BatchNorm statistics buffers (updated in training mode like torch's BatchNorm2d)."""
+
+    def __init__(self, family, state_dict):
+        super().__init__()
+        self.fwd = _oracle_forward(family)
+        self.names = [k for k, v in state_dict.items() if v.is_floating_point() and "running_" not in k]
+        self.buffer_names = [k for k in state_dict if k not in self.names]
+        self.weights = torch.nn.ParameterList(torch.nn.Parameter(state_dict[k].clone()) for k in self.names)
+        for i, k in enumerate(self.buffer_names):
+            self.register_buffer(f"stat{i}", state_dict[k].clone())
+
+    def reference_state_dict(self):
+        """The state_dict of the reference module (its own key names)."""
+        sd = dict(zip(self.names, self.weights))
+        sd.update((k, getattr(self, f"stat{i}")) for i, k in enumerate(self.buffer_names))
+        return sd
+
+    def forward(self, x):
+        sd = self.reference_state_dict()
+        logits, stats = self.fwd(sd, x, self.training, {k: sd[k] for k in self.buffer_names})
+        with torch.no_grad():
+            for i, k in enumerate(self.buffer_names):
+                if stats[k] is not sd[k]:           # num_batches_tracked is replaced, the running statistics update in place
+                    getattr(self, f"stat{i}").copy_(stats[k])
+        return logits
+
+    def grads(self):
+        return {k: p.grad.detach() for k, p in zip(self.names, self.weights) if p.grad is not None}
+
+
+# CE_Loss / Dice_loss (nets/unet_training.py) as the oracle restates them, logits resized to the label size first
+ORACLE_LOSSES = types.SimpleNamespace(
+    CE_Loss=lambda inputs, target, cls_weights, num_classes=21: O.ce_loss(
+        O.resize_logits(inputs, target.shape[1], target.shape[2]), target, cls_weights, num_classes),
+    Dice_loss=lambda inputs, target: O.dice_loss(O.resize_logits(inputs, target.shape[1], target.shape[2]), target))
 
 
 def build_reference(family, C, seed=11):
-    """The reference nn.Module (unmodified, from baseline/_ref) with dropout disabled (BASELINE config 4: 'train mode with
-    Dropout disabled') and its loss functions."""
-    from baseline import stage_ref
-    mod, cls, kw, _ = FAMILIES[family]
+    """The reference model (OracleReference) and its loss functions.  Its initial weights are those the module's own
+    constructor draws after torch.manual_seed(seed); the drop-in module keeps the reference's module tree and init."""
+    import unet_pytorch_b200 as b2u
+    kw, cls = FAMILIES[family]
     torch.manual_seed(seed)
-    model = getattr(stage_ref.import_reference(mod), cls)(**kw(C))
-    for m in model.modules():
-        if isinstance(m, (torch.nn.Dropout, torch.nn.Dropout2d)):
-            m.p = 0.0
-    T = stage_ref.import_reference("nets.unet_training")
-    return model, T
+    sd = getattr(b2u, cls)(**kw(C)).state_dict()
+    return OracleReference(family, sd), ORACLE_LOSSES
 
 
 def make_batch(n, C, hw, seed, medical=False, device="cpu"):
@@ -141,13 +177,12 @@ def run_reference(model, T, imgs, pngs, C, dtype, autocast=False):
         logits = m(x)
     loss = loss_of(T, logits, pngs, C, w)
     loss.backward()
-    grads = {k: p.grad.detach() for k, p in m.named_parameters() if p.grad is not None}
-    return logits.detach(), grads, loss.item()
+    return logits.detach(), m.grads(), loss.item()
 
 
 def run_product(b2u, family, state_dict, imgs, pngs, C):
     """The product bf16 path through the drop-in module API (the calls of utils_fit.py:70-92)."""
-    _, _, kw, cls = FAMILIES[family]
+    kw, cls = FAMILIES[family]
     model = getattr(b2u, cls)(**kw(C))
     model.load_state_dict(state_dict)
     model = model.train().to(imgs.device)
@@ -185,7 +220,7 @@ def measure(b2u, family, C, hw=512, batch=8, warm_steps=200, warm_batch=4, devic
         if cache:
             os.makedirs(cache_dir, exist_ok=True)
             torch.save(model.state_dict(), cache)
-    sd = {k: v.detach().clone() for k, v in model.state_dict().items()}
+    sd = {k: v.detach().clone() for k, v in model.reference_state_dict().items()}
     imgs, pngs = make_batch(batch, C, hw, 7, medical, dev)
     z64, g64, l64 = run_reference(model, T, imgs, pngs, C, torch.float64)
     out = {"family": family, "classes": C, "hw": hw, "batch": batch, "warm_steps": warm_steps, "warm_loss": warm_loss, "loss_fp64": l64}

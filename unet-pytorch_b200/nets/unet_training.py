@@ -3,6 +3,9 @@ helpers (weights_init :58-76, get_lr_scheduler :78-108, set_optimizer_lr :110-11
 
 CE_Loss / Focal_Loss / Dice_loss keep the reference signatures and run the fused CUDA loss kernels
 (csrc/head_loss.cu); `ce_dice_loss` is the one-pass combination the training loop uses (utils_fit.py:74-81)."""
+import math
+from functools import partial
+
 import torch
 
 from .. import ops
@@ -107,31 +110,62 @@ def ce_dice_loss(inputs, target, cls_weights, num_classes=21, dice=True, focal=F
 
 
 # ---------------------------------------------------------------------------------------- host helpers
-# weights_init / get_lr_scheduler / set_optimizer_lr (nets/unet_training.py:58-113) are host-side helpers outside the hot
-# path; they are not restated here.  A loop that imports them from this module gets the reference's own, unmodified
-# functions: from the reference checkout on sys.path order, else from the staged copy under baseline/_ref/
-# (baseline/stage_ref.py).
-_REFERENCE_HELPERS = ("weights_init", "get_lr_scheduler", "set_optimizer_lr")
+# weights_init / get_lr_scheduler / set_optimizer_lr (nets/unet_training.py:58-113): host-side helpers outside the hot
+# path, restated with the reference's signatures and arithmetic so that the training scripts can import them from here.
+def weights_init(net, init_type="normal", init_gain=0.02):
+    """Every module whose class name contains 'Conv' and that has a weight: N(0, init_gain) (or the named init);
+    BatchNorm2d: weight N(1, 0.02), bias 0."""
+    def init_func(m):
+        classname = m.__class__.__name__
+        if hasattr(m, "weight") and classname.find("Conv") != -1:
+            if init_type == "normal":
+                torch.nn.init.normal_(m.weight.data, 0.0, init_gain)
+            elif init_type == "xavier":
+                torch.nn.init.xavier_normal_(m.weight.data, gain=init_gain)
+            elif init_type == "kaiming":
+                torch.nn.init.kaiming_normal_(m.weight.data, a=0, mode="fan_in")
+            elif init_type == "orthogonal":
+                torch.nn.init.orthogonal_(m.weight.data, gain=init_gain)
+            else:
+                raise NotImplementedError("initialization method [%s] is not implemented" % init_type)
+        elif classname.find("BatchNorm2d") != -1:
+            torch.nn.init.normal_(m.weight.data, 1.0, 0.02)
+            torch.nn.init.constant_(m.bias.data, 0.0)
+    print("initialize network with %s type" % init_type)
+    net.apply(init_func)
 
 
-def _reference_unet_training():
-    import importlib.util
-    import os
-    root = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-    for cand in (os.environ.get("B2U_REFERENCE_SRC", "/root/reference"), os.path.join(root, "baseline", "_ref")):
-        path = os.path.join(cand, "nets", "unet_training.py")
-        if os.path.exists(path):
-            spec = importlib.util.spec_from_file_location("_b2u_reference_unet_training", path)
-            mod = importlib.util.module_from_spec(spec)
-            spec.loader.exec_module(mod)
-            return mod
-    raise ImportError("weights_init / get_lr_scheduler / set_optimizer_lr are the reference's own host helpers: put the "
-                      "reference checkout at $B2U_REFERENCE_SRC or stage it with `python -m baseline.stage_ref`")
+def get_lr_scheduler(lr_decay_type, lr, min_lr, total_iters, warmup_iters_ratio=0.05, warmup_lr_ratio=0.1,
+                     no_aug_iter_ratio=0.05, step_num=10):
+    """epoch -> learning rate.  "cos": quadratic warm-up, cosine decay, min_lr for the last epochs; otherwise step decay
+    from lr to min_lr in step_num steps."""
+    def yolox_warm_cos_lr(lr, min_lr, total_iters, warmup_total_iters, warmup_lr_start, no_aug_iter, iters):
+        if iters <= warmup_total_iters:
+            lr = (lr - warmup_lr_start) * pow(iters / float(warmup_total_iters), 2) + warmup_lr_start
+        elif iters >= total_iters - no_aug_iter:
+            lr = min_lr
+        else:
+            lr = min_lr + 0.5 * (lr - min_lr) * (
+                1.0 + math.cos(math.pi * (iters - warmup_total_iters) / (total_iters - warmup_total_iters - no_aug_iter)))
+        return lr
+
+    def step_lr(lr, decay_rate, step_size, iters):
+        if step_size < 1:
+            raise ValueError("step_size must above 1.")
+        n = iters // step_size
+        return lr * decay_rate ** n
+
+    if lr_decay_type == "cos":
+        warmup_total_iters = min(max(warmup_iters_ratio * total_iters, 1), 3)
+        warmup_lr_start = max(warmup_lr_ratio * lr, 1e-6)
+        no_aug_iter = min(max(no_aug_iter_ratio * total_iters, 1), 15)
+        return partial(yolox_warm_cos_lr, lr, min_lr, total_iters, warmup_total_iters, warmup_lr_start, no_aug_iter)
+    decay_rate = (min_lr / lr) ** (1 / (step_num - 1))
+    step_size = total_iters / step_num
+    return partial(step_lr, lr, decay_rate, step_size)
 
 
-def __getattr__(name):
-    if name in _REFERENCE_HELPERS:
-        fn = getattr(_reference_unet_training(), name)
-        globals()[name] = fn
-        return fn
-    raise AttributeError(f"module {__name__!r} has no attribute {name!r}")
+def set_optimizer_lr(optimizer, lr_scheduler_func, epoch):
+    lr = lr_scheduler_func(epoch)
+    for param_group in optimizer.param_groups:
+        param_group["lr"] = lr
