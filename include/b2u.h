@@ -224,9 +224,11 @@ int b2u_se_fc_bwd(const float* dscale, const float* pooled, const float* hidden,
                   const float* w2, float* dpooled, float* dw1, float* db1, float* dw2, float* db2, float* scratch, int N,
                   int C, int Cp, int R, float dp_scale, void* stream);
 
-/* ---- classifier head (nn.Conv2d(64, num_classes, 1), nets/unet.py:58,76) ------------------------------------ */
+/* ---- classifier head (nn.Conv2d(64, num_classes, 1), nets/unet.py:58,76), 1 <= ncls <= 255 ------------------ */
 int b2u_head_fwd(const void* x, const float* w, const float* b, float* logits_nchw, int N, int H, int W, int Cin,
                  int ncls, void* stream);
+/* workspace bytes of b2u_head_bwd for ncls classes; b2u_head_bwd_workspace() = the size for up to 32 classes */
+size_t b2u_head_bwd_workspace_cls(int ncls);
 size_t b2u_head_bwd_workspace(void);
 int b2u_head_bwd(const float* dlogits_nchw, const void* x, const float* w, void* dx, float* dw, float* db, void* ws,
                  size_t ws_bytes, int N, int H, int W, int Cin, int ncls, int relu_mask, void* stream);
@@ -234,23 +236,26 @@ int b2u_head_bwd(const float* dlogits_nchw, const void* x, const float* w, void*
 /* ---- losses and metrics ------------------------------------------------------------------------------------ */
 /* CE_Loss / Focal_Loss / Dice_loss (nets/unet_training.py:9-56) and f_score (utils/utils_metrics.py:12-31) in one
  * pass.  out (device, b2u_loss_out_len(C) floats): [0] CE, [1] Focal, [2] Dice loss, [3] f_score, then backward
- * coefficients.  target: int64 [N,H,W]; onehot (nullable): fp32 [N,H,W,C+1]. */
+ * coefficients.  target: int64 [N,H,W]; onehot (nullable): fp32 [N,H,W,C+1].  1 <= C <= 255. */
 size_t b2u_loss_workspace(int C);
 int b2u_loss_out_len(int C);
 int b2u_loss_fwd(const float* logits, const long long* target, const float* onehot, const float* cls_w, float* out,
                  double* stats, void* ws, size_t ws_bytes, int N, int C, int H, int W, float beta, float smooth,
                  float focal_alpha, float focal_gamma, float thr, void* stream);
 /* dlogits = gscale[0] dCE + gscale[1] dFocal + gscale[2] dDice (gscale: 3 floats on device).
- * out_mode 0: fp32 NCHW (autograd of the drop-in losses); 1: bf16 NHWC [N,H,W,64] = [hi(32) | lo(32)] two-term bf16
- * split of dlogits (classes >= C zero), the dz operand of b2u_conv_dgrad / b2u_conv_wgrad (taps = 1) for the head's
- * backward on the tensor cores (both halves meet the same weights, see b2u_pack_head_dgrad). */
+ * out_mode 0: fp32 NCHW (autograd of the drop-in losses); 1: bf16 NHWC [N,H,W,64 G], G = ceil(C / 32) groups, group g =
+ * [hi(32) | lo(32)] two-term bf16 split of the dlogits of classes 32g .. 32g + 31 (classes >= C zero), the dz operand of
+ * b2u_conv_dgrad / b2u_conv_wgrad (taps = 1) for the head's backward on the tensor cores (both halves meet the same
+ * weights, see b2u_pack_head_dgrad). */
 int b2u_loss_bwd(const float* logits, const long long* target, const float* onehot, const float* cls_w, const float* fin,
                  const float* gscale, void* dlogits, int out_mode, int N, int C, int H, int W, float focal_alpha,
                  float focal_gamma, void* stream);
-/* final.weight [C][64] fp32 -> 64x64 bf16 dgrad operand wd[ci][co], co in [0,32) and [32,64) both = class co % 32 */
+/* final.weight [C][64] fp32 -> [64][64 G] bf16 dgrad operand wd[ci][co]: columns 64g + r, r in [0,32) and [32,64), both
+ * = class 32g + r % 32 (zero past C) */
 int b2u_pack_head_dgrad(const float* w, void* wd, int ncls, void* stream);
-/* the same 1x1 classifier forward on the tensor cores: wf = bf16 [64][64] from b2u_pack_head_fprop (rows [0,32) =
- * bf16(W), rows [32,64) = bf16(W - bf16(W)); the epilogue adds the halves), fp32 NCHW logits written directly */
+/* the same 1x1 classifier forward on the tensor cores: wf = bf16 [64 G][64] from b2u_pack_head_fprop (in group g, rows
+ * 64g + [0,32) = bf16(W), rows 64g + [32,64) = bf16(W - bf16(W)) of classes 32g..; the epilogue adds the halves), fp32
+ * NCHW logits written directly; bias: [ncls] */
 int b2u_pack_head_fprop(const float* w, void* wf, int ncls, void* stream);
 int b2u_head_fwd_tc(const void* x, const void* wf, const float* bias, float* logits, int N, int H, int W, int ncls,
                     void* stream);
@@ -260,7 +265,7 @@ int b2u_argmax_u8(const float* logits, unsigned char* mask, int N, int C, int H,
  * INTER_LINEAR) of the probabilities to oh x ow, argmax -> uint8 mask [N][oh][ow]; nothing but the mask leaves the GPU */
 int b2u_softmax_resize_argmax_u8(const float* logits, unsigned char* mask, int N, int C, int H, int W, int cy, int cx,
                                  int ch, int cw, int oh, int ow, void* stream);
-/* fast_hist (utils/utils_metrics.py:34-43): hist (n*n+1 uint64, accumulated) ; dtype 0=u8 1=i32 2=i64 */
+/* fast_hist (utils/utils_metrics.py:34-43): hist (n*n+1 uint64, accumulated) ; dtype 0=u8 1=i32 2=i64; 1 <= n <= 256 */
 int b2u_fast_hist(const void* a, const void* b, long long len, int n, int dtype, unsigned long long* hist, void* stream);
 /* compute_mIoU's loop over an evaluation set (utils/utils_metrics.py:74-95) in ONE launch: items = count x {const uint8* a;
  * const uint8* b; int64 len; int64 first_chunk} (32 B each) in DEVICE memory, every pointer 16-byte aligned; first_chunk = running
@@ -269,7 +274,7 @@ int b2u_fast_hist_batch(const void* items, int count, long long total_chunks, in
 long long b2u_fast_hist_chunks(long long len);
 /* get_miou.py:45-65 without the mask round trip: pred = argmax_c logits (fp32 NCHW; lowest index on ties, unet.py:246-250),
  * optionally stored as a uint8 mask [N][H][W], and (gt, pred) counted into hist (n*n+1 uint64, accumulated) in the same pass;
- * gt: uint8 [N][H][W] (values >= n ignored) or NULL (mask only); H*W %% 4 == 0 */
+ * gt: uint8 [N][H][W] (values >= n ignored, 1 <= n <= 256) or NULL (mask only); H*W %% 4 == 0 */
 int b2u_argmax_hist(const float* logits, const unsigned char* gt, unsigned char* pred, int N, int C, int H, int W, int n,
                     unsigned long long* hist, void* stream);
 

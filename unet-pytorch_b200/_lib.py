@@ -80,6 +80,7 @@ SIGNATURES = {
     "b2u_se_fc_bwd": (I, [P, P, P, P, P, P, P, P, P, P, P, P, I, I, I, I, F, P]),
     "b2u_head_fwd": (I, [P, P, P, P, I, I, I, I, I, P]),
     "b2u_head_bwd_workspace": (SZ, []),
+    "b2u_head_bwd_workspace_cls": (SZ, [I]),
     "b2u_head_bwd": (I, [P, P, P, P, P, P, P, SZ, I, I, I, I, I, I, P]),
     "b2u_loss_workspace": (SZ, [I]),
     "b2u_loss_out_len": (I, [I]),

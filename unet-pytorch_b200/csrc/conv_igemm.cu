@@ -530,7 +530,11 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constan
       float* sB = sBias + bpar * 256;
       float* sS = sStat + bpar * 256;      // the statistics scratch doubles as the scale buffer (training vs eval: never both)
       for (int c = threadIdx.x - 64; c < BN; c += 128) {
-        sB[c] = (p.bias && (!(p.flags & 4) || c < p.head_cls)) ? __ldg(p.bias + n0 + c) : 0.f;
+        // head: column n0 + c is row (n0 + c) % 64 of group (n0 + c) / 64, and the bias [head_cls] is indexed by class
+        const int hcol = n0 + c, hcls = (hcol >> 6) * 32 + (hcol & 31);
+        sB[c] = !p.bias ? 0.f
+                : !(p.flags & 4) ? __ldg(p.bias + n0 + c)
+                : ((hcol & 63) < 32 && hcls < p.head_cls) ? __ldg(p.bias + hcls) : 0.f;
         if (p.scale) sS[c] = __ldg(p.scale + n0 + c);
       }
       named_bar_sync(2, 128);
@@ -557,16 +561,19 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constan
           if (lane == 0) mbar_arrive(t_empty(as));
         }
         if (p.flags & 4) {
-          // classifier head (nets/unet.py:58,76): the 64 accumulator columns are [hi(32) | lo(32)] of the two-term bf16
-          // split of the fp32 weights, so logits[c] = acc[c] + acc[32 + c] + bias[c] carries them to ~2^-17; written
-          // straight to the fp32 NCHW tensor the losses read (a warp covers two 64-byte runs per class)
+          // classifier head (nets/unet.py:58,76): each block of 64 accumulator columns is one group [hi(32) | lo(32)] of
+          // the two-term bf16 split of the fp32 weights of classes 32g .. 32g + 31, so logits[c] = acc[c] + acc[32 + c] +
+          // bias[c] carries them to ~2^-17; written straight to the fp32 NCHW tensor the losses read (a warp covers two
+          // 64-byte runs per class).  Groups past the last class (zero-filled rows of a ragged N tile) are skipped.
           const int gh = h0 + mt * kHb + ph;
-          if (gh < p.H && gw < p.W) {
+          const int cls0 = ((n0 + j * 64) >> 6) * 32;
+          if (gh < p.H && gw < p.W && cls0 < p.head_cls) {
             const size_t plane = static_cast<size_t>(p.H) * p.W;
-            float* o = p.head_out + static_cast<size_t>(img) * p.head_cls * plane + static_cast<size_t>(gh) * p.W + gw;
+            float* o = p.head_out + (static_cast<size_t>(img) * p.head_cls + cls0) * plane + static_cast<size_t>(gh) * p.W + gw;
+            const int ncls = p.head_cls - cls0;
 #pragma unroll
             for (int c = 0; c < 32; ++c)
-              if (c < p.head_cls) o[c * plane] = __uint_as_float(v[c]) + __uint_as_float(v[32 + c]) + sB[c];
+              if (c < ncls) o[c * plane] = __uint_as_float(v[c]) + __uint_as_float(v[32 + c]) + sB[j * 64 + c];
           }
           continue;
         }
@@ -785,7 +792,7 @@ static int launch_cfg(const ConvLaunch& a, cudaStream_t st) {
   p.tiles_w = (a.W + kWb - 1) / kWb;
   p.tiles_h = (a.H + kHb * MT - 1) / (kHb * MT);
   p.num_m_tiles = a.N * p.tiles_h * p.tiles_w;
-  p.num_n_tiles = a.Cout / BN;
+  p.num_n_tiles = (a.Cout + BN - 1) / BN;     // ragged only in head mode (the weight rows past Cout load as zeros)
   p.split_c = split;
   p.flags = a.flags;
   p.stat_partial = a.stat_partial;
@@ -857,10 +864,14 @@ int launch_conv(const ConvLaunch& a, cudaStream_t st) {
     return set_error(B2U_ERR_SHAPE, "conv: split_c %d must be a multiple of 64 inside (0,Cout)", a.split_c);
   if (a.scale && (a.stat_partial || (a.flags & 6)))
     return set_error(B2U_ERR_ARG, "conv: a per-channel scale excludes the statistics, mask and head epilogues");
-  if ((a.flags & 4) && (a.Cout != 64 || a.head_out == nullptr || a.head_cls < 1 || a.head_cls > 32 || a.y1 != nullptr))
-    return set_error(B2U_ERR_SHAPE, "conv: head mode needs Cout == 64, 1..32 classes and an fp32 output");
+  if ((a.flags & 4) && (a.head_out == nullptr || a.head_cls < 1 || a.head_cls > 255 || a.Cout != 64 * ((a.head_cls + 31) / 32) ||
+                        a.y1 != nullptr || a.bn_override))
+    return set_error(B2U_ERR_SHAPE, "conv: head mode needs 1..255 classes, Cout == 64 * ceil(classes / 32) and an fp32 output");
   int bn = 0;
-  if (a.bn_override) {
+  if (a.flags & 4) {
+    // head: the widest N tile (one pass over the 64-channel input per 4 groups); a ragged last tile runs on zero rows
+    bn = a.Cout >= 256 ? 256 : a.Cout;
+  } else if (a.bn_override) {
     if (a.Cout % a.bn_override != 0) return set_error(B2U_ERR_SHAPE, "conv: bn_override does not divide Cout");
     bn = a.bn_override;
   } else if (a.Cout % 256 == 0) bn = 256;
@@ -1085,14 +1096,16 @@ int b2u_conv_dgrad_bits(const void* dz, int Cz, const void* wd, void* dx0, int C
 }
 
 // Classifier head on the tensor cores: logits[n][c][h][w] = sum_k x[n][h][w][k] W[c][k] + b[c], fp32 NCHW.
-// wf: bf16 [64][64] from b2u_pack_head_fprop (rows [0,32) = bf16(W), rows [32,64) = bf16(W - bf16(W))).
+// wf: bf16 [64 G][64] from b2u_pack_head_fprop, G = ceil(ncls / 32) groups (in group g, rows [64g, 64g + 32) = bf16(W) and
+// rows [64g + 32, 64g + 64) = bf16(W - bf16(W)) of classes 32g..); bias: [ncls].
 int b2u_head_fwd_tc(const void* x, const void* wf, const float* bias, float* logits, int N, int H, int W, int ncls,
                     void* stream) {
+  if (ncls < 1 || ncls > 255) return b2u::set_error(B2U_ERR_SHAPE, "head_fwd_tc: 1 <= classes <= 255 (got %d)", ncls);
   b2u::ConvLaunch a;
   a.x0 = x; a.C0 = 64;
   a.wpacked = wf; a.bias = bias;
   a.y0 = const_cast<void*>(x);          // never written: the head epilogue bypasses the NHWC store path
-  a.N = N; a.H = H; a.W = W; a.Cout = 64; a.taps = 1;
+  a.N = N; a.H = H; a.W = W; a.Cout = 64 * ((ncls + 31) / 32); a.taps = 1;
   a.flags = 4; a.head_out = logits; a.head_cls = ncls;
   return b2u::launch_conv(a, static_cast<cudaStream_t>(stream));
 }

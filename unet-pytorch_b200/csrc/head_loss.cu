@@ -20,7 +20,8 @@ namespace b2u {
     b2u::note_launch();                                                                                  \
   } while (0)
 
-constexpr int kMaxCls = 32;
+constexpr int kMaxCls = 32;        // the register-array kernels below; wider heads take the *_wide kernels
+constexpr int kMaxClsWide = 255;   // uint8 masks: the reference's ignore label (= num_classes) must still fit a byte
 #ifndef B2U_FP32_VALIDATION
 constexpr int kHeadK = 64;
 #endif
@@ -170,6 +171,162 @@ __global__ void head_wgrad_reduce_kernel(const float* __restrict__ partial, floa
   const int c = i / (kHeadK + 1), k = i % (kHeadK + 1);
   float acc = 0.f;
   for (int b = 0; b < blocks; ++b) acc += partial[static_cast<size_t>(b) * kMaxCls * (kHeadK + 1) + c * (kHeadK + 1) + k];
+  if (k < kHeadK) { if (dw) dw[c * kHeadK + k] = acc; }
+  else if (db) db[c] = acc;
+}
+
+// ---- more than 32 classes: the same three computations, the weights staged through shared memory 32 classes at a time
+__global__ void __launch_bounds__(128)
+head_fwd_wide_kernel(const uint4* __restrict__ x, const float* __restrict__ w, const float* __restrict__ b,
+                     float* __restrict__ logits, long long HW, long long P, int ncls) {
+  __shared__ float sw[kMaxCls * kHeadK];
+  __shared__ float sb[kMaxCls];
+  const long long p = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+  const bool live = p < P;
+  float xv[kHeadK];
+#pragma unroll
+  for (int q = 0; q < 8; ++q) {
+    const uint4 v = live ? __ldg(x + p * 8 + q) : make_uint4(0u, 0u, 0u, 0u);
+    xv[q * 8 + 0] = bf16_lo(v.x); xv[q * 8 + 1] = bf16_hi(v.x); xv[q * 8 + 2] = bf16_lo(v.y); xv[q * 8 + 3] = bf16_hi(v.y);
+    xv[q * 8 + 4] = bf16_lo(v.z); xv[q * 8 + 5] = bf16_hi(v.z); xv[q * 8 + 6] = bf16_lo(v.w); xv[q * 8 + 7] = bf16_hi(v.w);
+  }
+  const long long n = live ? p / HW : 0, hw = live ? p % HW : 0;
+  float* out = logits + n * ncls * HW + hw;
+  for (int c0 = 0; c0 < ncls; c0 += kMaxCls) {
+    const int cn = ncls - c0 < kMaxCls ? ncls - c0 : kMaxCls;
+    __syncthreads();
+    for (int i = threadIdx.x; i < cn * kHeadK; i += blockDim.x) sw[i] = w[c0 * kHeadK + i];
+    for (int i = threadIdx.x; i < cn; i += blockDim.x) sb[i] = b ? b[c0 + i] : 0.f;
+    __syncthreads();
+    if (!live) continue;
+    for (int c = 0; c < cn; ++c) {
+      float acc = sb[c];
+      const float4* wr = reinterpret_cast<const float4*>(sw + c * kHeadK);
+#pragma unroll
+      for (int k = 0; k < kHeadK / 4; ++k) {
+        const float4 ww = wr[k];
+        acc = fmaf(xv[4 * k + 0], ww.x, acc); acc = fmaf(xv[4 * k + 1], ww.y, acc);
+        acc = fmaf(xv[4 * k + 2], ww.z, acc); acc = fmaf(xv[4 * k + 3], ww.w, acc);
+      }
+      out[(c0 + c) * HW] = acc;
+    }
+  }
+}
+
+__global__ void __launch_bounds__(128)
+head_dgrad_wide_kernel(const float* __restrict__ dlogits, const uint4* __restrict__ x, const float* __restrict__ w,
+                       uint4* __restrict__ dx, long long HW, long long P, int ncls, int relu_mask) {
+  __shared__ float sw[kMaxCls * kHeadK];
+  const long long p = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+  const bool live = p < P;
+  const long long n = live ? p / HW : 0, hw = live ? p % HW : 0;
+  const float* g = dlogits + n * ncls * HW + hw;
+  float acc[kHeadK];
+#pragma unroll
+  for (int k = 0; k < kHeadK; ++k) acc[k] = 0.f;
+  for (int c0 = 0; c0 < ncls; c0 += kMaxCls) {
+    const int cn = ncls - c0 < kMaxCls ? ncls - c0 : kMaxCls;
+    __syncthreads();
+    for (int i = threadIdx.x; i < cn * kHeadK; i += blockDim.x) sw[i] = w[c0 * kHeadK + i];
+    __syncthreads();
+    if (!live) continue;
+    for (int c = 0; c < cn; ++c) {
+      const float gc = __ldg(g + (c0 + c) * HW);
+      const float4* wr = reinterpret_cast<const float4*>(sw + c * kHeadK);
+#pragma unroll
+      for (int k = 0; k < kHeadK / 4; ++k) {
+        const float4 ww = wr[k];
+        acc[4 * k + 0] = fmaf(gc, ww.x, acc[4 * k + 0]); acc[4 * k + 1] = fmaf(gc, ww.y, acc[4 * k + 1]);
+        acc[4 * k + 2] = fmaf(gc, ww.z, acc[4 * k + 2]); acc[4 * k + 3] = fmaf(gc, ww.w, acc[4 * k + 3]);
+      }
+    }
+  }
+  if (!live) return;
+#pragma unroll
+  for (int q = 0; q < 8; ++q) {
+    float o[8];
+    if (relu_mask) {
+      const uint4 v = __ldg(x + p * 8 + q);
+      const float m[8] = {bf16_lo(v.x), bf16_hi(v.x), bf16_lo(v.y), bf16_hi(v.y),
+                          bf16_lo(v.z), bf16_hi(v.z), bf16_lo(v.w), bf16_hi(v.w)};
+#pragma unroll
+      for (int e = 0; e < 8; ++e) o[e] = m[e] > 0.f ? acc[q * 8 + e] : 0.f;
+    } else {
+#pragma unroll
+      for (int e = 0; e < 8; ++e) o[e] = acc[q * 8 + e];
+    }
+    uint4 r;
+    r.x = pack_bf16x2(o[0], o[1]); r.y = pack_bf16x2(o[2], o[3]); r.z = pack_bf16x2(o[4], o[5]); r.w = pack_bf16x2(o[6], o[7]);
+    dx[p * 8 + q] = r;
+  }
+}
+
+// blockIdx.y selects the group of 32 classes; partial[(group * gridDim.x + block)][32][65] as in head_wgrad_kernel
+__global__ void __launch_bounds__(128)
+head_wgrad_wide_kernel(const float* __restrict__ dlogits, const __nv_bfloat16* __restrict__ x, float* __restrict__ partial,
+                       long long HW, long long P, int ncls) {
+  __shared__ float sg[kMaxCls][kHwTile];
+  __shared__ float sx[kHwTile][kHeadK + 4];
+  const int tid = threadIdx.x;
+  const int kg = tid & 15;
+  const int cg = tid >> 4;
+  const int c0 = blockIdx.y * kMaxCls;
+  float acc[4][4];
+  float bacc[4] = {0, 0, 0, 0};
+#pragma unroll
+  for (int i = 0; i < 4; ++i)
+#pragma unroll
+    for (int j = 0; j < 4; ++j) acc[i][j] = 0.f;
+  const long long ntiles = (P + kHwTile - 1) / kHwTile;
+  for (long long tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
+    const long long p0 = tile * kHwTile;
+    for (int i = tid; i < kMaxCls * kHwTile; i += 128) {
+      const int c = i / kHwTile, pp = i % kHwTile;
+      const long long p = p0 + pp;
+      float v = 0.f;
+      if (c0 + c < ncls && p < P) { const long long n = p / HW, hw = p % HW; v = __ldg(dlogits + (n * ncls + c0 + c) * HW + hw); }
+      sg[c][pp] = v;
+    }
+    for (int i = tid; i < kHwTile * kHeadK / 2; i += 128) {
+      const int pp = i / (kHeadK / 2), k2 = i % (kHeadK / 2);
+      const long long p = p0 + pp;
+      uint32_t v = 0;
+      if (p < P) v = __ldg(reinterpret_cast<const uint32_t*>(x) + p * (kHeadK / 2) + k2);
+      sx[pp][2 * k2] = bf16_lo(v); sx[pp][2 * k2 + 1] = bf16_hi(v);
+    }
+    __syncthreads();
+#pragma unroll 4
+    for (int pp = 0; pp < kHwTile; ++pp) {
+      const float4 xv = *reinterpret_cast<const float4*>(&sx[pp][kg * 4]);
+      float g[4];
+#pragma unroll
+      for (int i = 0; i < 4; ++i) g[i] = sg[cg * 4 + i][pp];
+#pragma unroll
+      for (int i = 0; i < 4; ++i) {
+        acc[i][0] = fmaf(g[i], xv.x, acc[i][0]); acc[i][1] = fmaf(g[i], xv.y, acc[i][1]);
+        acc[i][2] = fmaf(g[i], xv.z, acc[i][2]); acc[i][3] = fmaf(g[i], xv.w, acc[i][3]);
+        if (kg == 0) bacc[i] += g[i];
+      }
+    }
+    __syncthreads();
+  }
+  float* out = partial + (static_cast<size_t>(blockIdx.y) * gridDim.x + blockIdx.x) * kMaxCls * (kHeadK + 1);
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const int c = cg * 4 + i;
+#pragma unroll
+    for (int j = 0; j < 4; ++j) out[c * (kHeadK + 1) + kg * 4 + j] = acc[i][j];
+    if (kg == 0) out[c * (kHeadK + 1) + kHeadK] = bacc[i];
+  }
+}
+__global__ void head_wgrad_wide_reduce_kernel(const float* __restrict__ partial, float* __restrict__ dw, float* __restrict__ db,
+                                              int blocks, int ncls) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= ncls * (kHeadK + 1)) return;
+  const int c = i / (kHeadK + 1), k = i % (kHeadK + 1);
+  const float* src = partial + static_cast<size_t>(c / kMaxCls) * blocks * kMaxCls * (kHeadK + 1) + (c % kMaxCls) * (kHeadK + 1) + k;
+  float acc = 0.f;
+  for (int b = 0; b < blocks; ++b) acc += src[static_cast<size_t>(b) * kMaxCls * (kHeadK + 1)];
   if (k < kHeadK) { if (dw) dw[c * kHeadK + k] = acc; }
   else if (db) db[c] = acc;
 }
@@ -538,27 +695,232 @@ loss_bwd_kernel(const float* __restrict__ logits, const long long* __restrict__ 
   }
 }
 
+// ------------------------------------------------------------------------------------------
+// losses, more than 32 classes: no per-class register arrays.  A pixel's logits are read twice (a block's 256 pixels
+// span C KB, served from L2): an online pass gives the max and the sum of exponentials, a second pass forms p_c.
+// ------------------------------------------------------------------------------------------
+// online softmax over one pixel's classes: on return m = max_c z_c and s = sum_c exp(z_c - m)
+__device__ __forceinline__ void online_max_sum(float v, float& m, float& s) {
+  if (v > m) { s = s * __expf(m - v) + 1.f; m = v; }
+  else s += __expf(v - m);
+}
+
+// v[i] on every lane -> lane l returns the sum over the warp of v[l] (reduce-scatter: 31 shuffles for 32 values, fixed
+// order, so the sums are deterministic)
+__device__ __forceinline__ float warp_transpose_sum32(float (&v)[32], int lane) {
+#pragma unroll
+  for (int s = 16; s >= 1; s >>= 1) {
+    const bool up = (lane & s) != 0;
+#pragma unroll
+    for (int i = 0; i < s; ++i) {
+      const float send = up ? v[i] : v[i + s];
+      const float keep = up ? v[i + s] : v[i];
+      v[i] = keep + __shfl_xor_sync(0xffffffffu, send, s);
+    }
+  }
+  return v[0];
+}
+
+// Same statistics layout as loss_stats_kernel.  A warp holds 32 pixels (one per lane); for each group of 32 classes the
+// per-class sums over those pixels are transposed so lane l owns class 32g + l, and the lane adds them to its warp's
+// shared-memory table (only that lane writes that entry: no atomics, fixed order).  Tables are folded in fp64 per block.
+template <bool ONEHOT>
+__global__ void __launch_bounds__(kLossThreads)
+loss_stats_wide_kernel(const float* __restrict__ logits, const long long* __restrict__ target, const float* __restrict__ onehot,
+                       const float* __restrict__ cls_w, double* __restrict__ partial, long long HW, long long P, int C,
+                       float focal_alpha, float focal_gamma, float thr) {
+  constexpr int kWarps = kLossThreads / 32;
+  __shared__ float swt[kMaxClsWide];
+  __shared__ float tab[kWarps][5 * kMaxClsWide];     // [warp][q * C + c], q = tp, P, T, tpf, Pf
+  __shared__ double sred[4][kWarps];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  for (int i = threadIdx.x; i < C; i += blockDim.x) swt[i] = cls_w ? cls_w[i] : 1.f;
+  for (int i = threadIdx.x; i < kWarps * 5 * kMaxClsWide; i += blockDim.x) (&tab[0][0])[i] = 0.f;
+  __syncthreads();
+  float a_ce = 0.f, a_w = 0.f, a_focal = 0.f, a_cnt = 0.f;
+  float* mytab = tab[warp];
+  for (long long p0 = static_cast<long long>(blockIdx.x) * blockDim.x + warp * 32; p0 < P;
+       p0 += static_cast<long long>(gridDim.x) * blockDim.x) {
+    const long long p = p0 + lane;
+    const bool inb = p < P;
+    const long long pc_ = inb ? p : P - 1;
+    const long long n = pc_ / HW, hw = pc_ % HW;
+    const float* z = logits + n * C * HW + hw;
+    float m = -INFINITY, s = 0.f;
+    for (int c = 0; c < C; ++c) online_max_sum(__ldg(z + c * HW), m, s);
+    const float inv = 1.f / s;
+    const long long y64 = (target && inb) ? target[pc_] : -1;
+    const bool valid = y64 >= 0 && y64 < C;
+    const int y = valid ? static_cast<int>(y64) : -1;
+    if (valid) {
+      const float nll = m + logf(s) - __ldg(z + y * HW);
+      const float wy = swt[y];
+      a_ce += wy * nll; a_w += wy;
+      const float logpt = -wy * nll;
+      const float pt = expf(logpt);
+      a_focal += -powf(fmaxf(1.f - pt, 0.f), focal_gamma) * (focal_alpha * logpt);
+    }
+    if (inb) a_cnt += 1.f;
+    for (int c0 = 0; c0 < C; c0 += 32) {
+      float pc[32], t[32], v[32];
+#pragma unroll
+      for (int i = 0; i < 32; ++i) {
+        const int c = c0 + i;
+        pc[i] = (inb && c < C) ? __expf(__ldg(z + c * HW) - m) * inv : 0.f;
+        if (ONEHOT) t[i] = (inb && c < C) ? __ldg(onehot + pc_ * (C + 1) + c) : 0.f;
+        else t[i] = (y == c) ? 1.f : 0.f;
+      }
+      const int cl = c0 + lane;
+      float r;
+#pragma unroll
+      for (int i = 0; i < 32; ++i) v[i] = t[i] * pc[i];
+      r = warp_transpose_sum32(v, lane);
+      if (cl < C) mytab[cl] += r;
+#pragma unroll
+      for (int i = 0; i < 32; ++i) v[i] = pc[i];
+      r = warp_transpose_sum32(v, lane);
+      if (cl < C) mytab[C + cl] += r;
+#pragma unroll
+      for (int i = 0; i < 32; ++i) v[i] = t[i];
+      r = warp_transpose_sum32(v, lane);
+      if (cl < C) mytab[2 * C + cl] += r;
+#pragma unroll
+      for (int i = 0; i < 32; ++i) v[i] = pc[i] > thr ? t[i] : 0.f;
+      r = warp_transpose_sum32(v, lane);
+      if (cl < C) mytab[3 * C + cl] += r;
+#pragma unroll
+      for (int i = 0; i < 32; ++i) v[i] = (inb && c0 + i < C && pc[i] > thr) ? 1.f : 0.f;
+      r = warp_transpose_sum32(v, lane);
+      if (cl < C) mytab[4 * C + cl] += r;
+    }
+  }
+  auto red = [&](float val, int slot) {
+    double d = static_cast<double>(val);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) d += __shfl_xor_sync(0xffffffffu, d, o);
+    if (lane == 0) sred[slot][warp] = d;
+  };
+  red(a_ce, 0); red(a_w, 1); red(a_focal, 2); red(a_cnt, 3);
+  __syncthreads();
+  const int L = 5 * C + 4;
+  double* out = partial + static_cast<size_t>(blockIdx.x) * L;
+  for (int sI = threadIdx.x; sI < L; sI += blockDim.x) {
+    double d = 0.0;
+    for (int w2 = 0; w2 < kWarps; ++w2) d += sI < 4 ? sred[sI][w2] : static_cast<double>(tab[w2][sI - 4]);
+    out[sI] = d;
+  }
+}
+
+// loss_bwd_kernel for more than 32 classes.  The online pass also accumulates sum_c (A_c t_c + B_c) exp(z_c - m), the
+// Dice term's dot product, so the second pass can write dz_c directly.
+// NHWC64: bf16 [pixel][64 G], group g = [hi(32) | lo(32)] of classes 32g .. 32g + 31 (padded classes exactly zero).
+template <bool ONEHOT, bool NHWC64>
+__global__ void __launch_bounds__(kLossThreads)
+loss_bwd_wide_kernel(const float* __restrict__ logits, const long long* __restrict__ target, const float* __restrict__ onehot,
+                     const float* __restrict__ cls_w, const float* __restrict__ fin, const float* __restrict__ gscale,
+                     void* __restrict__ dlogits, long long HW, long long P, int C, float focal_alpha, float focal_gamma) {
+  __shared__ float swt[kMaxClsWide], sA[kMaxClsWide], sB[kMaxClsWide];
+  for (int i = threadIdx.x; i < C; i += blockDim.x) {
+    swt[i] = cls_w ? cls_w[i] : 1.f; sA[i] = fin[4 + i]; sB[i] = fin[4 + C + i];
+  }
+  __syncthreads();
+  const float g_ce = gscale[0] * fin[4 + 2 * C];
+  const float g_focal = gscale[1] * fin[4 + 2 * C + 1];
+  const float g_dice = gscale[2];
+  const long long p = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (p >= P) return;
+  const long long n = p / HW, hw = p % HW;
+  const float* z = logits + n * C * HW + hw;
+  const long long y64 = target ? target[p] : -1;
+  const bool valid = target && y64 >= 0 && y64 < C;
+  const int y = valid ? static_cast<int>(y64) : -1;
+  auto tgt = [&](int c) -> float {
+    if (ONEHOT) return __ldg(onehot + p * (C + 1) + c);
+    return c == y ? 1.f : 0.f;
+  };
+  float m = -INFINITY, s = 0.f, gs = 0.f;
+  if (g_dice != 0.f) {
+    for (int c = 0; c < C; ++c) {
+      const float v = __ldg(z + c * HW), gc = sA[c] * tgt(c) + sB[c];
+      if (v > m) { const float r = __expf(m - v); s = s * r + 1.f; gs = gs * r + gc; m = v; }
+      else { const float e = __expf(v - m); s += e; gs = fmaf(gc, e, gs); }
+    }
+  } else {
+    for (int c = 0; c < C; ++c) online_max_sum(__ldg(z + c * HW), m, s);
+  }
+  const float inv = 1.f / s;
+  const float gdot = gs * inv;
+  float k_py = 0.f;
+  if (valid) {
+    const float wy = swt[y];
+    k_py = g_ce * wy;
+    if (g_focal != 0.f) {
+      const float nll = m + logf(s) - __ldg(z + y * HW);
+      const float logpt = -wy * nll;
+      const float pt = expf(logpt);
+      const float om = fmaxf(1.f - pt, 0.f);
+      const float dF = focal_alpha * (focal_gamma * powf(om, focal_gamma - 1.f) * pt * logpt - powf(om, focal_gamma));
+      k_py += g_focal * dF * (-wy);
+    }
+  }
+  auto dz = [&](int c) -> float {
+    const float pc = __expf(__ldg(z + c * HW) - m) * inv;
+    float d = k_py * (pc - (c == y ? 1.f : 0.f));
+    if (g_dice != 0.f) d += g_dice * pc * (sA[c] * tgt(c) + sB[c] - gdot);
+    return d;
+  };
+  if (!NHWC64) {
+    float* dzp = static_cast<float*>(dlogits) + n * C * HW + hw;
+    for (int c = 0; c < C; ++c) dzp[c * HW] = dz(c);
+  } else {
+    const int G = (C + 31) / 32;
+    uint4* row = static_cast<uint4*>(dlogits) + p * 8 * G;
+    for (int g = 0; g < G; ++g) {
+      float d[32];
+#pragma unroll
+      for (int i = 0; i < 32; ++i) d[i] = 32 * g + i < C ? dz(32 * g + i) : 0.f;
+#pragma unroll
+      for (int q = 0; q < 4; ++q) {
+        uint4 h, l;
+        float lo[8];
+#pragma unroll
+        for (int e = 0; e < 8; ++e) lo[e] = d[q * 8 + e] - __bfloat162float(__float2bfloat16_rn(d[q * 8 + e]));
+        h.x = pack_bf16x2(d[q * 8 + 0], d[q * 8 + 1]); h.y = pack_bf16x2(d[q * 8 + 2], d[q * 8 + 3]);
+        h.z = pack_bf16x2(d[q * 8 + 4], d[q * 8 + 5]); h.w = pack_bf16x2(d[q * 8 + 6], d[q * 8 + 7]);
+        l.x = pack_bf16x2(lo[0], lo[1]); l.y = pack_bf16x2(lo[2], lo[3]); l.z = pack_bf16x2(lo[4], lo[5]); l.w = pack_bf16x2(lo[6], lo[7]);
+        row[8 * g + q] = h;
+        row[8 * g + 4 + q] = l;
+      }
+    }
+  }
+}
+
 #ifndef B2U_FP32_VALIDATION
-// final.weight [C][64] fp32 -> dgrad operand wd[ci][co] bf16, 64 x 64: columns [0,32) and [32,64) both hold W
-// (they multiply the hi and lo halves of the split dlogits), classes >= C are zero
+// The tensor-core head works on G = ceil(C / 32) groups of 64 columns; group g covers classes 32g .. 32g + 31 as
+// [hi(32) | lo(32)].
+// final.weight [C][64] fp32 -> dgrad operand wd[ci][co] bf16, 64 x 64G: columns [64g, 64g + 32) and [64g + 32, 64g + 64)
+// both hold the weights of classes 32g.. (they multiply the hi and lo halves of the split dlogits), classes >= C are zero
 __global__ void pack_head_dgrad_kernel(const float* __restrict__ w, __nv_bfloat16* __restrict__ wd, int C) {
+  const int cols = 64 * ((C + kMaxCls - 1) / kMaxCls);
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= 64 * 64) return;
-  const int ci = i / 64, co = (i % 64) % kMaxCls;
+  if (i >= 64 * cols) return;
+  const int ci = i / cols, col = i % cols, co = (col / 64) * kMaxCls + (col % 64) % kMaxCls;
   wd[i] = __float2bfloat16_rn(co < C ? w[co * 64 + ci] : 0.f);
 }
 
-// final.weight [C][64] fp32 -> fprop operand wf[co'][k] bf16, 64 x 64: rows [0,32) = bf16(W), rows [32,64) = the bf16
-// remainder W - bf16(W); the head epilogue adds the two halves (classes >= C are zero rows)
+// final.weight [C][64] fp32 -> fprop operand wf[co'][k] bf16, 64G x 64: in group g, rows [64g, 64g + 32) = bf16(W) and rows
+// [64g + 32, 64g + 64) = the bf16 remainder W - bf16(W) of classes 32g..; the head epilogue adds the two halves (classes
+// >= C are zero rows)
 __global__ void pack_head_fprop_kernel(const float* __restrict__ w, __nv_bfloat16* __restrict__ wf, int C) {
+  const int rows = 64 * ((C + kMaxCls - 1) / kMaxCls);
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= 64 * 64) return;
-  const int co = i / 64, k = i % 64, c = co % kMaxCls;
+  if (i >= rows * 64) return;
+  const int co = i / 64, k = i % 64, r = co % 64, c = (co / 64) * kMaxCls + r % kMaxCls;
   float v = 0.f;
   if (c < C) {
     const float full = w[c * 64 + k];
     const float hi = __bfloat162float(__float2bfloat16_rn(full));
-    v = co < kMaxCls ? hi : full - hi;
+    v = r < kMaxCls ? hi : full - hi;
   }
   wf[i] = __float2bfloat16_rn(v);
 }
@@ -621,6 +983,46 @@ softmax_resize_argmax_kernel(const float* __restrict__ logits, uint8_t* __restri
   mask[(static_cast<size_t>(n) * oh + y) * ow + x] = static_cast<uint8_t>(arg);
 }
 
+// softmax_resize_argmax_kernel for more than 32 classes, without per-class arrays: loop 1 gives each tap's max and sum
+// (the same max-then-sum order as the kernel above), loop 2 interpolates each class's probability and keeps a running
+// arg-max (strict >, so the lowest index wins ties)
+__global__ void __launch_bounds__(128)
+softmax_resize_argmax_wide_kernel(const float* __restrict__ logits, uint8_t* __restrict__ mask, int C, int H, int W, int cy,
+                                  int cx, int ch, int cw, int oh, int ow, float sy, float sx) {
+  const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y, n = blockIdx.z;
+  if (x >= ow) return;
+  float fy = (y + 0.5f) * sy - 0.5f, fx = (x + 0.5f) * sx - 0.5f;
+  int y0 = static_cast<int>(floorf(fy)), x0 = static_cast<int>(floorf(fx));
+  fy -= y0; fx -= x0;
+  if (y0 < 0) { y0 = 0; fy = 0.f; }
+  if (y0 >= ch - 1) { y0 = ch - 1; fy = 0.f; }
+  if (x0 < 0) { x0 = 0; fx = 0.f; }
+  if (x0 >= cw - 1) { x0 = cw - 1; fx = 0.f; }
+  const int y1 = y0 + 1 < ch ? y0 + 1 : ch - 1, x1 = x0 + 1 < cw ? x0 + 1 : cw - 1;
+  const size_t plane = static_cast<size_t>(H) * W;
+  const float* base = logits + static_cast<size_t>(n) * C * plane;
+  const size_t o[4] = {static_cast<size_t>(cy + y0) * W + cx + x0, static_cast<size_t>(cy + y0) * W + cx + x1,
+                       static_cast<size_t>(cy + y1) * W + cx + x0, static_cast<size_t>(cy + y1) * W + cx + x1};
+  const float wgt[4] = {(1.f - fy) * (1.f - fx), (1.f - fy) * fx, fy * (1.f - fx), fy * fx};
+  float m[4], k[4];
+#pragma unroll
+  for (int t = 0; t < 4; ++t) {
+    m[t] = -INFINITY;
+    for (int c = 0; c < C; ++c) m[t] = fmaxf(m[t], __ldg(base + c * plane + o[t]));
+    float sum = 0.f;
+    for (int c = 0; c < C; ++c) sum += __expf(__ldg(base + c * plane + o[t]) - m[t]);
+    k[t] = wgt[t] / sum;
+  }
+  float best = -INFINITY; int arg = 0;
+  for (int c = 0; c < C; ++c) {
+    float acc = 0.f;
+#pragma unroll
+    for (int t = 0; t < 4; ++t) acc = fmaf(k[t], __expf(__ldg(base + c * plane + o[t]) - m[t]), acc);
+    if (c == 0 || acc > best) { best = acc; arg = c; }
+  }
+  mask[(static_cast<size_t>(n) * oh + y) * ow + x] = static_cast<uint8_t>(arg);
+}
+
 }  // namespace b2u
 
 extern "C" {
@@ -629,35 +1031,54 @@ using namespace b2u;
 #ifndef B2U_FP32_VALIDATION
 int b2u_head_fwd(const void* x, const float* w, const float* b, float* logits, int N, int H, int W, int Cin, int ncls,
                  void* stream) {
-  if (Cin != kHeadK || ncls <= 0 || ncls > kMaxCls) return set_error(B2U_ERR_SHAPE, "head_fwd: needs Cin == 64 and 1 <= classes <= 32 (got %d, %d)", Cin, ncls);
+  if (Cin != kHeadK || ncls <= 0 || ncls > kMaxClsWide) return set_error(B2U_ERR_SHAPE, "head_fwd: needs Cin == 64 and 1 <= classes <= 255 (got %d, %d)", Cin, ncls);
   if (N <= 0 || H <= 0 || W <= 0) return set_error(B2U_ERR_SHAPE, "head_fwd: empty tensor");
   const long long HW = static_cast<long long>(H) * W, P = HW * N;
-  head_fwd_kernel<<<static_cast<unsigned>((P + 127) / 128), 128, 0, static_cast<cudaStream_t>(stream)>>>(
-      static_cast<const uint4*>(x), w, b, logits, HW, P, ncls);
+  const unsigned grid = static_cast<unsigned>((P + 127) / 128);
+  if (ncls <= kMaxCls)
+    head_fwd_kernel<<<grid, 128, 0, static_cast<cudaStream_t>(stream)>>>(static_cast<const uint4*>(x), w, b, logits, HW, P, ncls);
+  else
+    head_fwd_wide_kernel<<<grid, 128, 0, static_cast<cudaStream_t>(stream)>>>(static_cast<const uint4*>(x), w, b, logits, HW, P, ncls);
   B2U_CHECK_LAUNCH("head_fwd");
   return 0;
 }
 
-size_t b2u_head_bwd_workspace(void) { return static_cast<size_t>(4 * 148) * kMaxCls * (kHeadK + 1) * sizeof(float); }
+// workspace of b2u_head_bwd: one [32][65] fp32 partial per block and group of 32 classes
+size_t b2u_head_bwd_workspace_cls(int ncls) {
+  const int groups = ncls > kMaxCls ? (ncls + kMaxCls - 1) / kMaxCls : 1;
+  return static_cast<size_t>(4 * 148) * groups * kMaxCls * (kHeadK + 1) * sizeof(float);
+}
+size_t b2u_head_bwd_workspace(void) { return b2u_head_bwd_workspace_cls(kMaxCls); }   // enough for up to 32 classes
 
 // dx may be NULL (frozen everything below); dw/db may be NULL.
 int b2u_head_bwd(const float* dlogits, const void* x, const float* w, void* dx, float* dw, float* db, void* ws,
                  size_t ws_bytes, int N, int H, int W, int Cin, int ncls, int relu_mask, void* stream) {
-  if (Cin != kHeadK || ncls <= 0 || ncls > kMaxCls) return set_error(B2U_ERR_SHAPE, "head_bwd: needs Cin == 64 and 1 <= classes <= 32");
+  if (Cin != kHeadK || ncls <= 0 || ncls > kMaxClsWide) return set_error(B2U_ERR_SHAPE, "head_bwd: needs Cin == 64 and 1 <= classes <= 255");
   if (N <= 0 || H <= 0 || W <= 0) return set_error(B2U_ERR_SHAPE, "head_bwd: empty tensor");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const long long HW = static_cast<long long>(H) * W, P = HW * N;
+  const bool wide = ncls > kMaxCls;
   if (dx) {
-    head_dgrad_kernel<<<static_cast<unsigned>((P + 127) / 128), 128, 0, st>>>(dlogits, static_cast<const uint4*>(x), w,
-                                                                             static_cast<uint4*>(dx), HW, P, ncls, relu_mask);
+    const unsigned grid = static_cast<unsigned>((P + 127) / 128);
+    if (!wide)
+      head_dgrad_kernel<<<grid, 128, 0, st>>>(dlogits, static_cast<const uint4*>(x), w, static_cast<uint4*>(dx), HW, P, ncls, relu_mask);
+    else
+      head_dgrad_wide_kernel<<<grid, 128, 0, st>>>(dlogits, static_cast<const uint4*>(x), w, static_cast<uint4*>(dx), HW, P, ncls, relu_mask);
     B2U_CHECK_LAUNCH("head_dgrad");
   }
   if (dw || db) {
     const int blocks = 4 * 148;
-    if (!ws || ws_bytes < b2u_head_bwd_workspace()) return set_error(B2U_ERR_ARG, "head_bwd: workspace too small");
-    head_wgrad_kernel<<<blocks, 128, 0, st>>>(dlogits, static_cast<const __nv_bfloat16*>(x), static_cast<float*>(ws), HW, P, ncls);
-    B2U_CHECK_LAUNCH("head_wgrad");
-    head_wgrad_reduce_kernel<<<(ncls * (kHeadK + 1) + 127) / 128, 128, 0, st>>>(static_cast<const float*>(ws), dw, db, blocks, ncls);
+    if (!ws || ws_bytes < b2u_head_bwd_workspace_cls(ncls)) return set_error(B2U_ERR_ARG, "head_bwd: workspace too small");
+    if (!wide) {
+      head_wgrad_kernel<<<blocks, 128, 0, st>>>(dlogits, static_cast<const __nv_bfloat16*>(x), static_cast<float*>(ws), HW, P, ncls);
+      B2U_CHECK_LAUNCH("head_wgrad");
+      head_wgrad_reduce_kernel<<<(ncls * (kHeadK + 1) + 127) / 128, 128, 0, st>>>(static_cast<const float*>(ws), dw, db, blocks, ncls);
+    } else {
+      const dim3 grid(blocks, (ncls + kMaxCls - 1) / kMaxCls);
+      head_wgrad_wide_kernel<<<grid, 128, 0, st>>>(dlogits, static_cast<const __nv_bfloat16*>(x), static_cast<float*>(ws), HW, P, ncls);
+      B2U_CHECK_LAUNCH("head_wgrad");
+      head_wgrad_wide_reduce_kernel<<<(ncls * (kHeadK + 1) + 127) / 128, 128, 0, st>>>(static_cast<const float*>(ws), dw, db, blocks, ncls);
+    }
     B2U_CHECK_LAUNCH("head_wgrad_reduce");
   }
   return 0;
@@ -675,7 +1096,7 @@ int b2u_loss_out_len(int C) { return 4 + 2 * C + 2; }
 int b2u_loss_fwd(const float* logits, const long long* target, const float* onehot, const float* cls_w, float* out,
                  double* stats, void* ws, size_t ws_bytes, int N, int C, int H, int W, float beta, float smooth,
                  float focal_alpha, float focal_gamma, float thr, void* stream) {
-  if (C <= 0 || C > kMaxCls) return set_error(B2U_ERR_SHAPE, "loss: 1 <= classes <= 32 (got %d)", C);
+  if (C <= 0 || C > kMaxClsWide) return set_error(B2U_ERR_SHAPE, "loss: 1 <= classes <= 255 (got %d)", C);
   if (N <= 0 || H <= 0 || W <= 0) return set_error(B2U_ERR_SHAPE, "loss: empty tensor");
   if (!ws || ws_bytes < b2u_loss_workspace(C)) return set_error(B2U_ERR_ARG, "loss: workspace too small");
   if (!target && !onehot) return set_error(B2U_ERR_ARG, "loss: need a target map or a one-hot tensor");
@@ -685,7 +1106,26 @@ int b2u_loss_fwd(const float* logits, const long long* target, const float* oneh
   long long want = (P + kLossThreads - 1) / kLossThreads;
   const int blocks = static_cast<int>(want < kLossBlocks ? want : kLossBlocks);
   const size_t sm = static_cast<size_t>(L) * (kLossThreads / 32) * sizeof(double);
-  if (onehot) {
+  const size_t fin_sm = 5 * L * sizeof(double);
+  if (fin_sm > 48 * 1024) {        // from C = 245 on the finalize's staging passes the default dynamic shared-memory limit
+    static bool attr_done[64] = {false};
+    int dev = 0;
+    cudaGetDevice(&dev);
+    if (dev < 0 || dev >= 64 || !attr_done[dev]) {
+      const cudaError_t e = cudaFuncSetAttribute(loss_finalize_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                                 static_cast<int>(5 * (5 * kMaxClsWide + 4) * sizeof(double)));
+      if (e != cudaSuccess) return set_error(B2U_ERR_CUDA, "loss: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
+      if (dev >= 0 && dev < 64) attr_done[dev] = true;
+    }
+  }
+  if (C > kMaxCls) {
+    if (onehot)
+      loss_stats_wide_kernel<true><<<blocks, kLossThreads, 0, st>>>(logits, target, onehot, cls_w, static_cast<double*>(ws), HW, P, C,
+                                                                    focal_alpha, focal_gamma, thr);
+    else
+      loss_stats_wide_kernel<false><<<blocks, kLossThreads, 0, st>>>(logits, target, nullptr, cls_w, static_cast<double*>(ws), HW, P, C,
+                                                                     focal_alpha, focal_gamma, thr);
+  } else if (onehot) {
     loss_stats_kernel<true><<<blocks, kLossThreads, sm, st>>>(logits, target, onehot, cls_w, static_cast<double*>(ws), HW, P, C,
                                                               focal_alpha, focal_gamma, thr);
   } else {
@@ -697,21 +1137,40 @@ int b2u_loss_fwd(const float* logits, const long long* target, const float* oneh
 #undef B2U_STATS
   }
   B2U_CHECK_LAUNCH("loss_stats");
-  loss_finalize_kernel<<<1, 1024, 5 * L * sizeof(double), st>>>(static_cast<const double*>(ws), blocks, C, beta, smooth, out, stats);
+  loss_finalize_kernel<<<1, 1024, fin_sm, st>>>(static_cast<const double*>(ws), blocks, C, beta, smooth, out, stats);
   B2U_CHECK_LAUNCH("loss_finalize");
   return 0;
 }
 
 // fin: the `out` vector of b2u_loss_fwd; gscale: 3 floats on device = upstream gradients of (CE, Focal, Dice)
-// out_mode 0: dlogits fp32 NCHW [N,C,H,W]; 1: bf16 NHWC [N,H,W,64] zero padded (feeds b2u_conv_dgrad/wgrad, taps=1)
+// out_mode 0: dlogits fp32 NCHW [N,C,H,W]; 1: bf16 NHWC [N,H,W,64 G], G = ceil(C / 32), group g = [hi(32) | lo(32)] of
+// classes 32g.. with padded classes zero (feeds b2u_conv_dgrad/wgrad, taps=1)
 int b2u_loss_bwd(const float* logits, const long long* target, const float* onehot, const float* cls_w, const float* fin,
                  const float* gscale, void* dlogits, int out_mode, int N, int C, int H, int W, float focal_alpha,
                  float focal_gamma, void* stream) {
-  if (C <= 0 || C > kMaxCls) return set_error(B2U_ERR_SHAPE, "loss_bwd: 1 <= classes <= 32");
+  if (C <= 0 || C > kMaxClsWide) return set_error(B2U_ERR_SHAPE, "loss_bwd: 1 <= classes <= 255");
   if (N <= 0 || H <= 0 || W <= 0) return set_error(B2U_ERR_SHAPE, "loss_bwd: empty tensor");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const long long HW = static_cast<long long>(H) * W, P = HW * N;
   const unsigned blocks = static_cast<unsigned>((P + kLossThreads - 1) / kLossThreads);
+  if (C > kMaxCls) {
+#define B2U_LBWDW(OH_, NH_) loss_bwd_wide_kernel<OH_, NH_><<<blocks, kLossThreads, 0, st>>>( \
+      logits, target, onehot, cls_w, fin, gscale, dlogits, HW, P, C, focal_alpha, focal_gamma)
+    if (out_mode == 1) {
+#ifdef B2U_FP32_VALIDATION
+      return set_error(B2U_ERR_ARG, "loss_bwd: the bf16 [hi | lo] output is not part of the fp32 validation build");
+#else
+      if (onehot) B2U_LBWDW(true, true); else B2U_LBWDW(false, true);
+#endif
+    } else if (out_mode == 0) {
+      if (onehot) B2U_LBWDW(true, false); else B2U_LBWDW(false, false);
+    } else {
+      return set_error(B2U_ERR_ARG, "loss_bwd: out_mode must be 0 or 1");
+    }
+#undef B2U_LBWDW
+    B2U_CHECK_LAUNCH("loss_bwd");
+    return 0;
+  }
   float* out = static_cast<float*>(dlogits);
 #define B2U_LBWD(OH_, NH_, CM_) loss_bwd_kernel<OH_, NH_, CM_><<<blocks, kLossThreads, 0, st>>>( \
       logits, target, onehot, cls_w, fin, gscale, out, HW, P, C, focal_alpha, focal_gamma)
@@ -736,15 +1195,17 @@ int b2u_loss_bwd(const float* logits, const long long* target, const float* oneh
 
 #ifndef B2U_FP32_VALIDATION
 int b2u_pack_head_dgrad(const float* w, void* wd, int ncls, void* stream) {
-  if (ncls <= 0 || ncls > kMaxCls) return set_error(B2U_ERR_SHAPE, "pack_head_dgrad: 1 <= classes <= 32");
-  pack_head_dgrad_kernel<<<16, 256, 0, static_cast<cudaStream_t>(stream)>>>(w, static_cast<__nv_bfloat16*>(wd), ncls);
+  if (ncls <= 0 || ncls > kMaxClsWide) return set_error(B2U_ERR_SHAPE, "pack_head_dgrad: 1 <= classes <= 255");
+  const int groups = (ncls + kMaxCls - 1) / kMaxCls;
+  pack_head_dgrad_kernel<<<16 * groups, 256, 0, static_cast<cudaStream_t>(stream)>>>(w, static_cast<__nv_bfloat16*>(wd), ncls);
   B2U_CHECK_LAUNCH("pack_head_dgrad");
   return 0;
 }
 
 int b2u_pack_head_fprop(const float* w, void* wf, int ncls, void* stream) {
-  if (ncls <= 0 || ncls > kMaxCls) return set_error(B2U_ERR_SHAPE, "pack_head_fprop: 1 <= classes <= 32");
-  pack_head_fprop_kernel<<<16, 256, 0, static_cast<cudaStream_t>(stream)>>>(w, static_cast<__nv_bfloat16*>(wf), ncls);
+  if (ncls <= 0 || ncls > kMaxClsWide) return set_error(B2U_ERR_SHAPE, "pack_head_fprop: 1 <= classes <= 255");
+  const int groups = (ncls + kMaxCls - 1) / kMaxCls;
+  pack_head_fprop_kernel<<<16 * groups, 256, 0, static_cast<cudaStream_t>(stream)>>>(w, static_cast<__nv_bfloat16*>(wf), ncls);
   B2U_CHECK_LAUNCH("pack_head_fprop");
   return 0;
 }
@@ -761,7 +1222,7 @@ int b2u_argmax_u8(const float* logits, unsigned char* mask, int N, int C, int H,
 // logits [N][C][H][W] fp32; crop (cy, cx, ch, cw) inside H x W; mask [N][oh][ow] uint8 (class index, lowest on ties)
 int b2u_softmax_resize_argmax_u8(const float* logits, unsigned char* mask, int N, int C, int H, int W, int cy, int cx,
                                  int ch, int cw, int oh, int ow, void* stream) {
-  if (N <= 0 || C <= 0 || C > kMaxCls || H <= 0 || W <= 0 || oh <= 0 || ow <= 0 || N > 65535 || oh > 65535)
+  if (N <= 0 || C <= 0 || C > kMaxClsWide || H <= 0 || W <= 0 || oh <= 0 || ow <= 0 || N > 65535 || oh > 65535)
     return set_error(B2U_ERR_SHAPE, "softmax_resize_argmax: bad shape");
   if (cy < 0 || cx < 0 || ch <= 0 || cw <= 0 || cy + ch > H || cx + cw > W)
     return set_error(B2U_ERR_SHAPE, "softmax_resize_argmax: crop outside the logits");
@@ -769,7 +1230,8 @@ int b2u_softmax_resize_argmax_u8(const float* logits, unsigned char* mask, int N
   const dim3 grid((ow + 127) / 128, oh, N);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
 #define B2U_SRA(CM_) softmax_resize_argmax_kernel<CM_><<<grid, 128, 0, st>>>(logits, mask, C, H, W, cy, cx, ch, cw, oh, ow, sy, sx)
-  if (C <= 8) B2U_SRA(8); else if (C <= 16) B2U_SRA(16); else if (C <= 24) B2U_SRA(24); else B2U_SRA(32);
+  if (C <= 8) B2U_SRA(8); else if (C <= 16) B2U_SRA(16); else if (C <= 24) B2U_SRA(24); else if (C <= 32) B2U_SRA(32);
+  else softmax_resize_argmax_wide_kernel<<<grid, 128, 0, st>>>(logits, mask, C, H, W, cy, cx, ch, cw, oh, ow, sy, sx);
 #undef B2U_SRA
   B2U_CHECK_LAUNCH("softmax_resize_argmax");
   return 0;

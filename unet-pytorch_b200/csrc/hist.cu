@@ -525,6 +525,135 @@ argmax_hist_kernel(const float* __restrict__ logits, const unsigned char* __rest
   if (gt) hist_publish(sm, warps, rows, slots, ign, hist, &s_ign);
 }
 
+// ---------------------------------------------------------------------------------------------------------------
+// 64 < n <= 256 ("wide"): n*n + 1 bins no longer fit lane-private byte counters.  One shared-memory table per block;
+// lanes of a warp holding the same bin (real masks are piecewise constant) are combined with __match_any_sync so one
+// atomic covers them; the table is flushed to the 64-bit global histogram with integer atomics (exact, order-free).
+// Counters are 32-bit while n*n + 1 of them fit a block's 227 KB (n <= 241).  Beyond that (C16) two 16-bit counters
+// share a word and the table is flushed after every 63 pixels per thread (at most 64512 < 2^16 increments per counter).
+// ---------------------------------------------------------------------------------------------------------------
+constexpr int kWideThreads = 1024;
+constexpr size_t kWideSmemMax = 227 * 1024;
+
+__host__ __device__ inline bool hist_wide_c16(int n) { return static_cast<size_t>(n * n + 1) * 4 > kWideSmemMax; }
+__host__ __device__ inline int hist_wide_words(int n) { return hist_wide_c16(n) ? (n * n + 2) / 2 : n * n + 1; }
+
+template <bool C16>
+__device__ __forceinline__ void wide_flush(unsigned int* sh, int n, unsigned long long* __restrict__ hist) {
+  const int slots = n * n + 1, words = hist_wide_words(n);
+  for (int i = threadIdx.x; i < words; i += blockDim.x) {
+    const unsigned v = sh[i];
+    if (!v) continue;
+    sh[i] = 0u;
+    if (C16) {
+      if (v & 0xffffu) atomicAdd(&hist[2 * i], static_cast<unsigned long long>(v & 0xffffu));
+      if ((v >> 16) && 2 * i + 1 < slots) atomicAdd(&hist[2 * i + 1], static_cast<unsigned long long>(v >> 16));
+    } else {
+      atomicAdd(&hist[i], static_cast<unsigned long long>(v));
+    }
+  }
+}
+
+// counts pixels [p0, p1) of a block-uniform range; fetch(i, a, b) returns the pair of pixel i (fast_hist's semantics:
+// a outside [0, n) is ignored, n * a + b outside [0, n*n) goes to the overflow slot n*n)
+template <bool C16, typename Fetch>
+__device__ __forceinline__ void wide_count_range(long long p0, long long p1, int n, unsigned int* sh,
+                                                 unsigned long long* __restrict__ hist, Fetch fetch) {
+  const int lane = threadIdx.x & 31, nbins = n * n;
+  const long long step = C16 ? 63LL * blockDim.x : p1 - p0;
+  for (long long s0 = p0; s0 < p1; s0 += step) {
+    const long long s1 = s0 + step < p1 ? s0 + step : p1;
+    for (long long i0 = s0 + (threadIdx.x & ~31); i0 < s1; i0 += blockDim.x) {    // warp-uniform: full-warp match below
+      const long long i = i0 + lane;
+      int bin = -1;
+      if (i < s1) {
+        long long av, bv;
+        fetch(i, av, bv);
+        if (av >= 0 && av < n) {
+          const long long bb = static_cast<long long>(n) * av + bv;
+          bin = (bb >= 0 && bb < nbins) ? static_cast<int>(bb) : nbins;
+        }
+      }
+      const unsigned peers = __match_any_sync(0xffffffffu, bin);
+      if (bin >= 0 && lane == __ffs(peers) - 1) {
+        if (C16) atomicAdd(&sh[bin >> 1], static_cast<unsigned>(__popc(peers)) << ((bin & 1) * 16));
+        else atomicAdd(&sh[bin], static_cast<unsigned>(__popc(peers)));
+      }
+    }
+    if (C16) { __syncthreads(); wide_flush<true>(sh, n, hist); __syncthreads(); }
+  }
+}
+
+template <bool C16>
+__device__ __forceinline__ unsigned int* wide_table_init(int n) {
+  extern __shared__ __align__(16) unsigned int sh_wide[];
+  for (int i = threadIdx.x; i < hist_wide_words(n); i += blockDim.x) sh_wide[i] = 0u;
+  __syncthreads();
+  return sh_wide;
+}
+
+template <typename T, bool C16>
+__global__ void __launch_bounds__(kWideThreads)
+fast_hist_wide_kernel(const T* __restrict__ a, const T* __restrict__ b, long long len, long long unit, int n,
+                      unsigned long long* __restrict__ hist) {
+  unsigned int* sh = wide_table_init<C16>(n);
+  for (long long p0 = blockIdx.x * unit; p0 < len; p0 += gridDim.x * unit) {
+    const long long p1 = p0 + unit < len ? p0 + unit : len;
+    wide_count_range<C16>(p0, p1, n, sh, hist, [&](long long i, long long& av, long long& bv) {
+      av = static_cast<long long>(a[i]); bv = static_cast<long long>(b[i]);
+    });
+  }
+  __syncthreads();
+  wide_flush<C16>(sh, n, hist);
+}
+
+// batched form: work units are the item table's chunks (as in fast_hist_lanes_kernel); the last chunk of a pair also
+// takes its len % 16 tail pixels
+template <bool C16>
+__global__ void __launch_bounds__(kWideThreads)
+fast_hist_wide_batch_kernel(const HistItem* __restrict__ items, int count, long long total_chunks, int n,
+                            unsigned long long* __restrict__ hist) {
+  unsigned int* sh = wide_table_init<C16>(n);
+  for (long long u = blockIdx.x; u < total_chunks; u += gridDim.x) {
+    int lo = 0, hi = count - 1;
+    while (lo < hi) {
+      const int mid = (lo + hi + 1) >> 1;
+      if (__ldg(&items[mid].first_chunk) <= u) lo = mid; else hi = mid - 1;
+    }
+    const unsigned char *pa = items[lo].a, *pb = items[lo].b;
+    const long long len = items[lo].len, nvec = len / 16;
+    const long long v0 = (u - items[lo].first_chunk) * kHistChunkVec;
+    const long long p0 = 16 * v0, p1 = v0 + kHistChunkVec >= nvec ? len : 16 * (v0 + kHistChunkVec);
+    wide_count_range<C16>(p0, p1, n, sh, hist, [&](long long i, long long& av, long long& bv) {
+      av = __ldg(pa + i); bv = __ldg(pb + i);
+    });
+  }
+  __syncthreads();
+  wide_flush<C16>(sh, n, hist);
+}
+
+// argmax_hist_kernel for 64 < n: one thread per pixel, arg-max over the class planes (lowest index on ties)
+template <bool C16>
+__global__ void __launch_bounds__(kWideThreads)
+argmax_hist_wide_kernel(const float* __restrict__ logits, const unsigned char* __restrict__ gt, unsigned char* __restrict__ pred,
+                        int N, int C, long long HW, long long unit, int n, unsigned long long* __restrict__ hist) {
+  unsigned int* sh = wide_table_init<C16>(n);
+  const long long total = static_cast<long long>(N) * HW;
+  for (long long p0 = blockIdx.x * unit; p0 < total; p0 += gridDim.x * unit) {
+    const long long p1 = p0 + unit < total ? p0 + unit : total;
+    wide_count_range<C16>(p0, p1, n, sh, hist, [&](long long i, long long& av, long long& bv) {
+      const long long img = i / HW, hw = i - img * HW;
+      const float* z = logits + img * C * HW + hw;
+      float best = __ldg(z); int arg = 0;
+      for (int c = 1; c < C; ++c) { const float v = __ldg(z + c * HW); if (v > best) { best = v; arg = c; } }
+      if (pred) pred[i] = static_cast<unsigned char>(arg);
+      av = __ldg(gt + i); bv = arg;
+    });
+  }
+  __syncthreads();
+  wide_flush<C16>(sh, n, hist);
+}
+
 }  // namespace b2u
 
 extern "C" {
@@ -576,13 +705,75 @@ static int launch_hist_lanes(const HistItem* items, int count, long long total_c
   return 0;
 }
 
+// the wide kernels' dynamic shared memory: set once per device for every instantiation
+static int hist_wide_attr() {
+  static bool attr_done[64] = {false};
+  int dev = 0;
+  cudaGetDevice(&dev);
+  if (dev >= 0 && dev < 64 && attr_done[dev]) return 0;
+  const void* fns[] = {reinterpret_cast<const void*>(fast_hist_wide_kernel<unsigned char, false>),
+                       reinterpret_cast<const void*>(fast_hist_wide_kernel<unsigned char, true>),
+                       reinterpret_cast<const void*>(fast_hist_wide_kernel<int, false>),
+                       reinterpret_cast<const void*>(fast_hist_wide_kernel<int, true>),
+                       reinterpret_cast<const void*>(fast_hist_wide_kernel<long long, false>),
+                       reinterpret_cast<const void*>(fast_hist_wide_kernel<long long, true>),
+                       reinterpret_cast<const void*>(fast_hist_wide_batch_kernel<false>),
+                       reinterpret_cast<const void*>(fast_hist_wide_batch_kernel<true>),
+                       reinterpret_cast<const void*>(argmax_hist_wide_kernel<false>),
+                       reinterpret_cast<const void*>(argmax_hist_wide_kernel<true>)};
+  for (const void* fn : fns) {
+    const cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(kWideSmemMax));
+    if (e != cudaSuccess) return set_error(B2U_ERR_CUDA, "fast_hist (wide): cudaFuncSetAttribute: %s", cudaGetErrorString(e));
+  }
+  if (dev >= 0 && dev < 64) attr_done[dev] = true;
+  return 0;
+}
+static size_t hist_wide_smem(int n) { return static_cast<size_t>(hist_wide_words(n)) * sizeof(unsigned int); }
+// pixels per work unit: about one unit per SM (at least 64K pixels)
+static long long hist_wide_unit(long long len) {
+  long long u = (len + num_sms() - 1) / num_sms();
+  return u < 65536 ? 65536 : u;
+}
+static int hist_wide_grid(long long units) { return static_cast<int>(units < num_sms() ? (units < 1 ? 1 : units) : num_sms()); }
+
+static int fast_hist_wide(const void* a, const void* b, long long len, int n, int dtype, unsigned long long* hist, cudaStream_t st) {
+  if (int rc = hist_wide_attr()) return rc;
+  const long long unit = hist_wide_unit(len);
+  const int grid = hist_wide_grid((len + unit - 1) / unit);
+  const size_t sm = hist_wide_smem(n);
+  const bool c16 = hist_wide_c16(n);
+#define B2U_WIDE(T_) do { const T_* pa = static_cast<const T_*>(a); const T_* pb = static_cast<const T_*>(b);                       \
+    if (c16) fast_hist_wide_kernel<T_, true><<<grid, kWideThreads, sm, st>>>(pa, pb, len, unit, n, hist);                         \
+    else fast_hist_wide_kernel<T_, false><<<grid, kWideThreads, sm, st>>>(pa, pb, len, unit, n, hist); } while (0)
+  if (dtype == 0) B2U_WIDE(unsigned char);
+  else if (dtype == 1) B2U_WIDE(int);
+  else if (dtype == 2) B2U_WIDE(long long);
+  else return set_error(B2U_ERR_ARG, "fast_hist: dtype must be 0 (u8), 1 (i32) or 2 (i64)");
+#undef B2U_WIDE
+  cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) return set_error(B2U_ERR_CUDA, "fast_hist_wide launch: %s", cudaGetErrorString(e));
+  note_launch();
+  return 0;
+}
+
 // hist: n*n + 1 uint64 on device, ACCUMULATED into (caller zeroes it); hist[n*n] counts out-of-range bins.
 // dtype: 0 = uint8, 1 = int32, 2 = int64.  Blocks of 2^31 elements at most per call keep uint32 counters exact.
+// 1 <= n <= 256 (64 < n: the shared-table kernels above).
 int b2u_fast_hist(const void* a, const void* b, long long len, int n, int dtype, unsigned long long* hist, void* stream) {
-  if (n <= 0 || n > 64) return set_error(B2U_ERR_SHAPE, "fast_hist: 1 <= n <= 64 (got %d)", n);
+  if (n <= 0 || n > 256) return set_error(B2U_ERR_SHAPE, "fast_hist: 1 <= n <= 256 (got %d)", n);
   if (len < 0) return set_error(B2U_ERR_SHAPE, "fast_hist: negative length");
   if (len == 0) return 0;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (n > 64) {
+    const long long chunk = 1ll << 31;
+    const size_t esz = dtype == 0 ? 1 : (dtype == 1 ? 4 : 8);
+    for (long long off = 0; off < len; off += chunk) {
+      const long long l = len - off < chunk ? len - off : chunk;
+      if (int rc = fast_hist_wide(static_cast<const char*>(a) + off * esz, static_cast<const char*>(b) + off * esz, l, n, dtype, hist, st))
+        return rc;
+    }
+    return 0;
+  }
   const size_t sm = static_cast<size_t>(kHistWarps) * (n * n + 1) * sizeof(unsigned int);
   if (sm > 48 * 1024) {
     static bool big_done[64] = {false};
@@ -670,9 +861,21 @@ int b2u_fast_hist(const void* a, const void* b, long long len, int n, int dtype,
 // int64 first_chunk} (32 bytes each) in DEVICE memory, first_chunk = running sum of b2u_fast_hist_chunks(len) over the previous
 // items, total_chunks = the sum over all items; every pointer 16-byte aligned.  hist as in b2u_fast_hist.
 int b2u_fast_hist_batch(const void* items, int count, long long total_chunks, int n, unsigned long long* hist, void* stream) {
-  if (n <= 0 || n > 64) return set_error(B2U_ERR_SHAPE, "fast_hist_batch: 1 <= n <= 64 (got %d)", n);
+  if (n <= 0 || n > 256) return set_error(B2U_ERR_SHAPE, "fast_hist_batch: 1 <= n <= 256 (got %d)", n);
   if (count < 0 || (count > 0 && (!items || total_chunks < count))) return set_error(B2U_ERR_ARG, "fast_hist_batch: bad item table");
   if (count == 0) return 0;
+  if (n > 64) {
+    if (int rc = hist_wide_attr()) return rc;
+    const int grid = hist_wide_grid(total_chunks);
+    const HistItem* it = static_cast<const HistItem*>(items);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (hist_wide_c16(n)) fast_hist_wide_batch_kernel<true><<<grid, kWideThreads, hist_wide_smem(n), st>>>(it, count, total_chunks, n, hist);
+    else fast_hist_wide_batch_kernel<false><<<grid, kWideThreads, hist_wide_smem(n), st>>>(it, count, total_chunks, n, hist);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return set_error(B2U_ERR_CUDA, "fast_hist_wide_batch launch: %s", cudaGetErrorString(e));
+    note_launch();
+    return 0;
+  }
   if (n * n + 1 <= kVoteMaxBins) {         // few bins: register counters (see b2u_fast_hist)
     int grid = 8 * num_sms();
     if (total_chunks < grid) grid = static_cast<int>(total_chunks);
@@ -703,8 +906,21 @@ int b2u_argmax_hist(const float* logits, const unsigned char* gt, unsigned char*
   if (N <= 0 || C <= 0 || C > 255 || H <= 0 || W <= 0) return set_error(B2U_ERR_SHAPE, "argmax_hist: bad shape");
   const long long HW = static_cast<long long>(H) * W;
   if (HW % 4 != 0) return set_error(B2U_ERR_SHAPE, "argmax_hist: H*W must be a multiple of 4");
-  if (gt && (n <= 0 || n > 64 || !hist || hist_lanes_warps(n) < 1)) return set_error(B2U_ERR_ARG, "argmax_hist: bad n / hist");
+  if (gt && (n <= 0 || n > 256 || !hist || (n <= 64 && hist_lanes_warps(n) < 1)))
+    return set_error(B2U_ERR_ARG, "argmax_hist: bad n / hist");
   if (!gt && !pred) return set_error(B2U_ERR_ARG, "argmax_hist: nothing to produce");
+  if (gt && n > 64) {
+    if (int rc = hist_wide_attr()) return rc;
+    const long long total = static_cast<long long>(N) * HW, unit = hist_wide_unit(total);
+    const int grid = hist_wide_grid((total + unit - 1) / unit);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (hist_wide_c16(n)) argmax_hist_wide_kernel<true><<<grid, kWideThreads, hist_wide_smem(n), st>>>(logits, gt, pred, N, C, HW, unit, n, hist);
+    else argmax_hist_wide_kernel<false><<<grid, kWideThreads, hist_wide_smem(n), st>>>(logits, gt, pred, N, C, HW, unit, n, hist);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return set_error(B2U_ERR_CUDA, "argmax_hist_wide launch: %s", cudaGetErrorString(e));
+    note_launch();
+    return 0;
+  }
   const int nn = gt ? n : 1;
   const int warps = hist_lanes_warps(nn);
   const int slots = nn * nn + 1, rows = (slots + 3) / 4;

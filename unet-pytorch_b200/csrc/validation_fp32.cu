@@ -995,7 +995,7 @@ int b2u_upsample2x_bwd(const void* dup, const void* ylow, void* dlow, int N, int
 }
 
 int b2u_head_fwd(const void* x, const float* w, const float* b, float* logits, int N, int H, int W, int Cin, int ncls, void* stream) {
-  if (Cin != 64 || ncls <= 0 || ncls > 32) return set_error(B2U_ERR_SHAPE, "head_fwd: needs Cin == 64 and 1 <= classes <= 32 (got %d, %d)", Cin, ncls);
+  if (Cin != 64 || ncls <= 0 || ncls > 255) return set_error(B2U_ERR_SHAPE, "head_fwd: needs Cin == 64 and 1 <= classes <= 255 (got %d, %d)", Cin, ncls);
   if (N <= 0 || H <= 0 || W <= 0) return set_error(B2U_ERR_SHAPE, "head_fwd: empty tensor");
   const long long HW = static_cast<long long>(H) * W, P = HW * N;
   v32_head_fwd_kernel<<<blocks_for(P * ncls, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(static_cast<const float*>(x), w, b,
@@ -1004,9 +1004,10 @@ int b2u_head_fwd(const void* x, const float* w, const float* b, float* logits, i
   return 0;
 }
 size_t b2u_head_bwd_workspace(void) { return 16; }
+size_t b2u_head_bwd_workspace_cls(int /*ncls*/) { return 16; }
 int b2u_head_bwd(const float* dlogits, const void* x, const float* w, void* dx, float* dw, float* db, void* /*ws*/,
                  size_t /*ws_bytes*/, int N, int H, int W, int Cin, int ncls, int relu_mask, void* stream) {
-  if (Cin != 64 || ncls <= 0 || ncls > 32) return set_error(B2U_ERR_SHAPE, "head_bwd: needs Cin == 64 and 1 <= classes <= 32");
+  if (Cin != 64 || ncls <= 0 || ncls > 255) return set_error(B2U_ERR_SHAPE, "head_bwd: needs Cin == 64 and 1 <= classes <= 255");
   if (N <= 0 || H <= 0 || W <= 0) return set_error(B2U_ERR_SHAPE, "head_bwd: empty tensor");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const long long HW = static_cast<long long>(H) * W, P = HW * N;

@@ -121,8 +121,8 @@ class UNetEngine:
     def __init__(self, cfg, device=None):
         if cfg.in_channels * 9 > 64:
             raise ValueError("in_channels must be <= 7 (first-layer im2col is 64 columns wide)")
-        if not 1 <= cfg.num_classes <= 32:
-            raise ValueError("num_classes must be in [1, 32]")
+        if not 1 <= cfg.num_classes <= 255:
+            raise ValueError("num_classes must be in [1, 255]")
         self.cfg = cfg
         self.num_classes = cfg.num_classes
         self.in_channels = cfg.in_channels
@@ -442,7 +442,7 @@ class UNetEngine:
         if ops.act_dtype() == torch.float32:       # fp32 validation build: plain fp32 1x1 conv
             logits = ops.head_fwd(low, wh, params[self.head_name + ".bias"])
         else:
-            wf_head = ops.pack_head_fprop(wh, wf=self._buf("head:wf", (64, 64)))
+            wf_head = ops.pack_head_fprop(wh, wf=self._buf("head:wf", (64 * ops.head_groups(self.num_classes), 64)))
             logits = ops.head_fwd_tc(low, wf_head, params[self.head_name + ".bias"], self.num_classes)
         if save:
             self.saved = (A, feats, (N, H, W))
@@ -619,27 +619,29 @@ class UNetEngine:
         C = self.num_classes
         fw, fb = has(hn + ".weight"), has(hn + ".bias")
         g = self._buf("g:" + self.dec[-1][1].name, last.shape) if need_dx[hn] else None
-        if dlogits.dtype == torch.bfloat16 and dlogits.dim() == 4 and dlogits.shape[-1] == 64 and ops.act_dtype() == torch.bfloat16:
-            # [N,H,W,64] = [hi | lo] split dlogits from loss_bwd(nhwc64=True): the head's backward runs on the tensor
-            # cores as a 1x1 dgrad (+ReLU mask) and a 1x1 wgrad (+bias) over 2 x 32 padded classes
+        cz = 64 * ops.head_groups(C)
+        if dlogits.dtype == torch.bfloat16 and dlogits.dim() == 4 and dlogits.shape[-1] == cz and ops.act_dtype() == torch.bfloat16:
+            # [N,H,W,64 G] = per group of 32 classes, [hi | lo] split dlogits from loss_bwd(nhwc64=True): the head's backward
+            # runs on the tensor cores as a 1x1 dgrad (+ReLU mask) and a 1x1 wgrad (+bias) over G x 2 x 32 padded classes
             dl = dlogits.contiguous()
             if need_dx[hn]:
-                wd_head = ops.pack_head_dgrad(wh, wd=self._buf("head:wd", (64, 64)))
+                wd_head = ops.pack_head_dgrad(wh, wd=self._buf("head:wd", (64, cz)))
                 hbits = None if bn else A.get("bits:" + self.dec[-1][1].name)
                 if hbits is not None:
                     ops.conv_dgrad_bits(dl, wd_head, 64, hbits, taps=1, out0=g)
                 else:
                     ops.conv_dgrad(dl, wd_head, 64, taps=1, mask=None if bn else last, out0=g)
             if fw or fb:
-                dw64 = self._buf("head:dw", (64, 64, 1, 1), torch.float32)
-                db64 = self._buf("head:db", (64,), torch.float32)
-                need = ops.lib().b2u_conv_wgrad_workspace(dl.shape[0], dl.shape[1], dl.shape[2], 64, 64, 1)
+                dw64 = self._buf("head:dw", (cz, 64, 1, 1), torch.float32)
+                db64 = self._buf("head:db", (cz,), torch.float32)
+                need = ops.lib().b2u_conv_wgrad_workspace(dl.shape[0], dl.shape[1], dl.shape[2], 64, cz, 1)
                 with grad_stream():
                     ops.conv_wgrad(last, dl, taps=1, dw=dw64, db=db64, ws=self._workspace("wgrad", need))
-                    if fw:      # rows [0,32) came from the hi half of dlogits, rows [32,64) from the lo half
-                        torch.add(dw64[:C, :self.head_cin], dw64[32:32 + C, :self.head_cin], out=grads[hn + ".weight"])
+                    # in group g, rows 64g + [0,32) came from the hi half of dlogits, rows 64g + [32,64) from the lo half
+                    if fw:
+                        ops.fold_head_groups(dw64, C, self.head_cin, grads[hn + ".weight"])
                     if fb:
-                        torch.add(db64[:C], db64[32:32 + C], out=grads[hn + ".bias"])
+                        ops.fold_head_groups(db64, C, self.head_cin, grads[hn + ".bias"])
         else:
             dl = dlogits.contiguous()
             if dl.dtype != torch.float32:
@@ -650,7 +652,7 @@ class UNetEngine:
                 dwt = self._buf("head:dwf", (C, 64, 1, 1), torch.float32) if fw else None
                 dbt = grads[hn + ".bias"] if fb else None
             ops.head_bwd(dl, last, wh, need_dx=need_dx[hn], need_dw=fw or fb, relu_mask=not bn, dx=g, dw=dwt, db=dbt,
-                         ws=self._workspace("head", ops.lib().b2u_head_bwd_workspace()))
+                         ws=self._workspace("head", ops.lib().b2u_head_bwd_workspace_cls(C)))
             if fw and self.head_cin != 64:
                 grads[hn + ".weight"].copy_(dwt[:, :self.head_cin])
         with grad_stream():          # (orders the side stream after the head's launches, whichever stream ran them)

@@ -769,7 +769,8 @@ class GraphEngine:
                 if ops.act_dtype() == torch.float32:       # fp32 validation build: plain fp32 1x1 conv
                     logits = ops.head_fwd(xin.data, self._head_weight(params, ins), params[ins["bias"]])
                 else:
-                    wf_head = ops.pack_head_fprop(self._head_weight(params, ins), wf=self._buf("head:wf", (64, 64)))
+                    wf_head = ops.pack_head_fprop(self._head_weight(params, ins),
+                                                  wf=self._buf("head:wf", (64 * ops.head_groups(self.num_classes), 64)))
                     logits = ops.head_fwd_tc(xin.data, wf_head, params[ins["bias"]], self.num_classes)
         if save:
             self.saved = (T, (N, H, W), set(trainable))
@@ -814,18 +815,19 @@ class GraphEngine:
                 g = self._buf("g:" + ins["x"], xin.data.shape) if xin.needs_grad else None
                 if dlogits.dtype == torch.bfloat16 and ops.act_dtype() == torch.bfloat16:
                     dl = dlogits.contiguous()
+                    cz = 64 * ops.head_groups(C)       # [hi | lo] per group of 32 classes (ops.loss_bwd(nhwc64=True))
                     if g is not None:
-                        wd_head = ops.pack_head_dgrad(wh, wd=self._buf("head:wd", (64, 64)))
+                        wd_head = ops.pack_head_dgrad(wh, wd=self._buf("head:wd", (64, cz)))
                         ops.conv_dgrad(dl, wd_head, 64, taps=1, mask=xin.data if xin.fused_relu else None, out0=g)
                     if fw or fb:
-                        dw64 = self._buf("head:dw", (64, 64, 1, 1), torch.float32)
-                        db64 = self._buf("head:db", (64,), torch.float32)
-                        need = ops.lib().b2u_conv_wgrad_workspace(dl.shape[0], dl.shape[1], dl.shape[2], 64, 64, 1)
+                        dw64 = self._buf("head:dw", (cz, 64, 1, 1), torch.float32)
+                        db64 = self._buf("head:db", (cz,), torch.float32)
+                        need = ops.lib().b2u_conv_wgrad_workspace(dl.shape[0], dl.shape[1], dl.shape[2], 64, cz, 1)
                         ops.conv_wgrad(xin.data, dl, taps=1, dw=dw64, db=db64, ws=self._workspace("wgrad", need))
                         if fw:
-                            torch.add(dw64[:C, :cin], dw64[32:32 + C, :cin], out=grads[ins["w"]])
+                            ops.fold_head_groups(dw64, C, cin, grads[ins["w"]])
                         if fb:
-                            torch.add(db64[:C], db64[32:32 + C], out=grads[ins["bias"]])
+                            ops.fold_head_groups(db64, C, cin, grads[ins["bias"]])
                 else:
                     dl = dlogits.float().contiguous() if dlogits.dtype != torch.float32 else dlogits.contiguous()
                     dwt = None
@@ -833,7 +835,7 @@ class GraphEngine:
                         dwt = grads[ins["w"]] if cin == 64 else self._buf("head:dwf", (C, 64, 1, 1), torch.float32)
                     ops.head_bwd(dl, xin.data, wh, need_dx=g is not None, need_dw=fw or fb, relu_mask=xin.fused_relu, dx=g,
                                  dw=dwt, db=grads[ins["bias"]] if fb else None,
-                                 ws=self._workspace("head", ops.lib().b2u_head_bwd_workspace()))
+                                 ws=self._workspace("head", ops.lib().b2u_head_bwd_workspace_cls(C)))
                     if fw and cin != 64:
                         grads[ins["w"]].copy_(dwt[:, :cin])
                 if g is not None:
@@ -1087,16 +1089,16 @@ class GraphEngine:
 
 class ResNet50UnetEngine(GraphEngine):
     def __init__(self, num_classes, device=None):
-        if not 1 <= num_classes <= 32:
-            raise ValueError("num_classes must be in [1, 32]")
+        if not 1 <= num_classes <= 255:
+            raise ValueError("num_classes must be in [1, 255]")
         program, convs = resnet50_unet_program(num_classes)
         super().__init__(program, convs, num_classes, device=device)
 
 
 class UltraLightUnetEngine(GraphEngine):
     def __init__(self, num_classes, variant="ultralight_large", device=None):
-        if not 1 <= num_classes <= 32:
-            raise ValueError("num_classes must be in [1, 32]")
+        if not 1 <= num_classes <= 255:
+            raise ValueError("num_classes must be in [1, 255]")
         widths, mid_min, se_rule, p = ULU_VARIANTS[variant]
         program, convs = ultralight_unet_program(num_classes, widths, mid_min, se_rule, p)
         super().__init__(program, convs, num_classes, device=device)
@@ -1105,8 +1107,8 @@ class UltraLightUnetEngine(GraphEngine):
 
 class LightweightUnetEngine(GraphEngine):
     def __init__(self, num_classes, in_channels=3, device=None):
-        if not 1 <= num_classes <= 32:
-            raise ValueError("num_classes must be in [1, 32]")
+        if not 1 <= num_classes <= 255:
+            raise ValueError("num_classes must be in [1, 255]")
         if not 1 <= in_channels <= 64:
             raise ValueError("in_channels must be in [1, 64] (the image is zero-padded to one 64-channel block)")
         program, convs = lightweight_unet_program(num_classes, in_channels)
@@ -1118,8 +1120,8 @@ class ImprovedSegNetEngine(GraphEngine):
     """nets/RepVGG_Unet.py::ImprovedSegNet(use_repvgg=True); deploy=True runs the re-parameterised single-conv blocks."""
 
     def __init__(self, num_classes, deploy=False, device=None):
-        if not 1 <= num_classes <= 32:
-            raise ValueError("num_classes must be in [1, 32]")
+        if not 1 <= num_classes <= 255:
+            raise ValueError("num_classes must be in [1, 255]")
         program, convs = improved_segnet_program(num_classes, deploy=deploy)
         super().__init__(program, convs, num_classes, device=device)
         self.deploy = deploy

@@ -725,7 +725,7 @@ def head_bwd(dlogits, x, w, need_dx=True, need_dw=True, relu_mask=True, dx=None,
     _req(dlogits, torch.float32, "dlogits"); _req(x, ACT, "x"); _req(w, torch.float32, "w")
     N, H, W, Cin = x.shape
     ncls = w.shape[0]
-    need = lib().b2u_head_bwd_workspace()
+    need = lib().b2u_head_bwd_workspace_cls(ncls)
     if need_dw and (ws is None or ws.numel() * ws.element_size() < need):
         ws = _ws(need, x.device)
     if need_dx and dx is None:
@@ -760,13 +760,32 @@ def loss_fwd(logits, target=None, onehot=None, cls_w=None, beta=1.0, smooth=1e-5
 
 
 def loss_bwd(logits, fin, gscale, target=None, onehot=None, cls_w=None, alpha=0.5, gamma=2.0, out=None, nhwc64=False):
-    """dlogits as fp32 NCHW, or (nhwc64) as bf16 [N, H, W, 64] zero padded for the tensor-core head backward."""
+    """dlogits as fp32 NCHW, or (nhwc64) as bf16 [N, H, W, 64 G] zero padded for the tensor-core head backward
+    (G = head_groups(C) groups [hi(32) | lo(32)] of 32 classes)."""
     _req(logits, torch.float32, "logits"); _req(gscale, torch.float32, "gscale")
     N, C, H, W = logits.shape
     if out is None:
-        out = torch.empty((N, H, W, 64), dtype=ACT, device=logits.device) if nhwc64 else torch.empty_like(logits)
+        out = (torch.empty((N, H, W, 64 * head_groups(C)), dtype=ACT, device=logits.device) if nhwc64
+               else torch.empty_like(logits))
     check(lib().b2u_loss_bwd(ptr(logits), ptr(target), ptr(onehot), ptr(cls_w), ptr(fin), ptr(gscale), ptr(out),
                              1 if nhwc64 else 0, N, C, H, W, 0.0 if alpha is None else alpha, gamma, stream_ptr()))
+    return out
+
+
+def head_groups(ncls):
+    """Column groups of the tensor-core head: group g = [hi(32) | lo(32)] of classes 32g .. 32g + 31."""
+    return (ncls + 31) // 32
+
+
+def fold_head_groups(t, C, cin, out):
+    """out[c] = t[64g + r] + t[64g + 32 + r] for class c = 32g + r: the per-class sum of the hi and lo halves of a [64 G, ...]
+    gradient of the tensor-core head (cin: leading input channels kept along dim 1, when t has one)."""
+    for g in range(head_groups(C)):
+        c0, cn = 32 * g, min(32, C - 32 * g)
+        hi, lo = t[64 * g:64 * g + cn], t[64 * g + 32:64 * g + 32 + cn]
+        if t.dim() > 1:
+            hi, lo = hi[:, :cin], lo[:, :cin]
+        torch.add(hi, lo, out=out[c0:c0 + cn])
     return out
 
 
@@ -774,7 +793,7 @@ def pack_head_dgrad(w, wd=None):
     _req(w, torch.float32, "final.weight")
     ncls = w.shape[0]
     if wd is None:
-        wd = torch.empty((64, 64), dtype=ACT, device=w.device)
+        wd = torch.empty((64, 64 * head_groups(ncls)), dtype=ACT, device=w.device)
     check(lib().b2u_pack_head_dgrad(ptr(w), ptr(wd), ncls, stream_ptr()))
     return wd
 
@@ -783,7 +802,7 @@ def pack_head_fprop(w, wf=None):
     _req(w, torch.float32, "final.weight")
     ncls = w.shape[0]
     if wf is None:
-        wf = torch.empty((64, 64), dtype=ACT, device=w.device)
+        wf = torch.empty((64 * head_groups(ncls), 64), dtype=ACT, device=w.device)
     check(lib().b2u_pack_head_fprop(ptr(w), ptr(wf), ncls, stream_ptr()))
     return wf
 

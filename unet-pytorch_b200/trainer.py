@@ -318,7 +318,7 @@ class UnetTrainer:
         stride = getattr(self.engine, "logit_stride", 1)
         if stride == 1 and ops.act_dtype() == torch.bfloat16:
             dlogits = ops.loss_bwd(logits, fin, self._gscale, target=pngs, onehot=None, cls_w=self.cls_w, nhwc64=True,
-                                   out=self.engine._buf("g:logits64", (n, h, w, 64)))
+                                   out=self.engine._buf("g:logits64", (n, h, w, 64 * ops.head_groups(self.num_classes))))
         elif stride == 1:       # fp32 validation build: fp32 NCHW dlogits, plain fp32 head backward
             dlogits = ops.loss_bwd(logits, fin, self._gscale, target=pngs, onehot=None, cls_w=self.cls_w)
         else:       # gradient at label resolution (fp32), then the adjoint of the resize back to the logits' own size
