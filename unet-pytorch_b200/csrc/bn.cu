@@ -49,8 +49,12 @@ __device__ __forceinline__ void bn_affine(float g, float bt, float mean, float i
   *shift = static_cast<float>(static_cast<double>(bt) - static_cast<double>(mean) * sc);
 }
 
-// Column sums of two per-element quantities.  MODE 0: (z, z^2).  MODE 1: (g, g * xhat) with g = dy * mask, where the
-// mask is y > 0 (y given: residual blocks) or recomputed from z (y null).  partial layout: [block][2][C].
+// Column sums of two per-element quantities.  MODE 0: (z - K, (z - K)^2) with the per-channel pivot K = row 0 of z when
+// `pivot` is set (K = 0 otherwise).  MODE 1: (g, g * xhat) with g = dy * mask, where the mask is y > 0 (y given: residual
+// blocks) or recomputed from z (y null).  partial layout: [block][2][C].
+// The pivot keeps the one-pass variance accurate at training scale: with raw sums, var = E[z^2] - mean^2 loses the fp32
+// rounding of E[z^2] amplified by (mean / std)^2 (1.2e-2 relative at mean = 64 std over 4M pixels).  Shifted by a value of
+// the same channel, both sums are of the channel's spread; z - K of two bf16 values is exact in fp32.
 // blockDim.x = 256; thread -> (row lane, 8-channel chunk); kBnUnroll rows (independent 16-byte loads per operand) are
 // requested before any is consumed: ~64 KB in flight per SM.
 template <int MODE>
@@ -58,7 +62,7 @@ __global__ void __launch_bounds__(256, 2)
 bn_colsum_kernel(const uint4* __restrict__ a, const uint4* __restrict__ y, const uint4* __restrict__ z,
                  const float* __restrict__ gamma, const float* __restrict__ beta,
                  const float* __restrict__ mean, const float* __restrict__ invstd, float* __restrict__ partial,
-                 long long P, int C8, int relu) {
+                 long long P, int C8, int relu, int pivot) {
   constexpr int kBnUnroll = MODE == 0 ? 8 : 4;
   extern __shared__ float sred[];          // [256][16]
   const int tid = threadIdx.x;
@@ -79,7 +83,10 @@ bn_colsum_kernel(const uint4* __restrict__ a, const uint4* __restrict__ y, const
             bn_affine(gamma ? gamma[c * 8 + k] : 1.f, beta ? beta[c * 8 + k] : 0.f, mu[k], is[k], &sc[k], &sh[k]);
         }
       }
-      const uint4 zero = make_uint4(0u, 0u, 0u, 0u);
+      // rows past the end load the pivot itself: they add exactly 0 to both sums
+      const uint4 zero = MODE == 0 && pivot ? __ldg(a + c) : make_uint4(0u, 0u, 0u, 0u);
+      float kp[8];
+      bn_unpack8(zero, kp);
       for (long long p = static_cast<long long>(blockIdx.x) * rows + rr; p < P; p += kBnUnroll * stride) {
         uint4 va[kBnUnroll], vz[kBnUnroll], vy[kBnUnroll];
 #pragma unroll
@@ -98,7 +105,7 @@ bn_colsum_kernel(const uint4* __restrict__ a, const uint4* __restrict__ y, const
           bn_unpack8(va[u], f);
           if (MODE == 0) {
 #pragma unroll
-            for (int k = 0; k < 8; ++k) { s0[k] += f[k]; s1[k] = fmaf(f[k], f[k], s1[k]); }
+            for (int k = 0; k < 8; ++k) { const float d = f[k] - kp[k]; s0[k] += d; s1[k] = fmaf(d, d, s1[k]); }
           } else {
             float zz[8], yy[8];
             bn_unpack8(vz[u], zz);
@@ -148,8 +155,9 @@ bn_rows_reduce_kernel(const float* __restrict__ rows, float* __restrict__ out, i
   }
 }
 
-// forward finalize: statistics -> (scale, shift) for the apply pass, saved mean/invstd, running-stat update
-__global__ void bn_fwd_finalize_kernel(const float* __restrict__ partial, int blocks, int C, long long P,
+// forward finalize: statistics -> (scale, shift) for the apply pass, saved mean/invstd, running-stat update.
+// pivot_z (nullable): z itself when the sums are of z - K with K = row 0 of z (bn_colsum_kernel<0> with pivot set)
+__global__ void bn_fwd_finalize_kernel(const float* __restrict__ partial, const __nv_bfloat16* __restrict__ pivot_z, int blocks, int C, long long P,
                                        const float* __restrict__ gamma, const float* __restrict__ beta,
                                        float* __restrict__ running_mean, float* __restrict__ running_var,
                                        float* __restrict__ save_mean, float* __restrict__ save_invstd,
@@ -162,8 +170,9 @@ __global__ void bn_fwd_finalize_kernel(const float* __restrict__ partial, int bl
     s += partial[static_cast<size_t>(b) * 2 * C + c];
     ss += partial[static_cast<size_t>(b) * 2 * C + C + c];
   }
-  const double mean = s / static_cast<double>(P);
-  double var = ss / static_cast<double>(P) - mean * mean;
+  const double ms = s / static_cast<double>(P);      // mean of the shifted values
+  const double mean = (pivot_z ? static_cast<double>(__bfloat162float(pivot_z[c])) : 0.0) + ms;
+  double var = ss / static_cast<double>(P) - ms * ms;
   if (var < 0.0) var = 0.0;
   const double invstd = 1.0 / sqrt(var + static_cast<double>(eps));
   const float mean_f = static_cast<float>(mean), invstd_f = static_cast<float>(invstd);
@@ -339,9 +348,10 @@ int b2u_bn_fwd_train(const void* z, const void* residual, void* y, const float* 
   float* partial = static_cast<float*>(ws);
   float* coef = partial + static_cast<size_t>(kBnBlocks) * 2 * C;
   bn_colsum_kernel<0><<<kBnBlocks, 256, 256 * 16 * sizeof(float), st>>>(static_cast<const uint4*>(z), nullptr, nullptr, nullptr,
-                                                                        nullptr, nullptr, nullptr, partial, P, C / 8, 0);
+                                                                        nullptr, nullptr, nullptr, partial, P, C / 8, 0, 1);
   B2U_CHECK_LAUNCH("bn_colsum");
-  bn_fwd_finalize_kernel<<<(C + 127) / 128, 128, 0, st>>>(partial, kBnBlocks, C, P, gamma, beta, running_mean, running_var,
+  bn_fwd_finalize_kernel<<<(C + 127) / 128, 128, 0, st>>>(partial, static_cast<const __nv_bfloat16*>(z), kBnBlocks, C, P, gamma,
+                                                          beta, running_mean, running_var,
                                                           save_mean, save_invstd, coef, coef + C, eps, momentum, centered);
   B2U_CHECK_LAUNCH("bn_fwd_finalize");
   const long long G = (P + kBnApplyRows - 1) / kBnApplyRows;
@@ -367,7 +377,7 @@ int b2u_bn_fwd_train_stats(const void* z, const void* residual, void* y, const f
   float* coef = partial + static_cast<size_t>(kBnBlocks) * 2 * C;
   bn_rows_reduce_kernel<<<(2 * C + 31) / 32, 256, 0, st>>>(stat_partial, partial, stat_rows, 2 * C);
   B2U_CHECK_LAUNCH("bn_rows_reduce");
-  bn_fwd_finalize_kernel<<<(C + 127) / 128, 128, 0, st>>>(partial, 1, C, P, gamma, beta, running_mean, running_var,
+  bn_fwd_finalize_kernel<<<(C + 127) / 128, 128, 0, st>>>(partial, nullptr, 1, C, P, gamma, beta, running_mean, running_var,
                                                           save_mean, save_invstd, coef, coef + C, eps, momentum, centered);
   B2U_CHECK_LAUNCH("bn_fwd_finalize");
   const long long G = (P + kBnApplyRows - 1) / kBnApplyRows;
@@ -379,14 +389,16 @@ int b2u_bn_fwd_train_stats(const void* z, const void* residual, void* y, const f
 
 // ---- SyncBatchNorm building blocks (nn.SyncBatchNorm.convert_sync_batchnorm, train.py:335-336): the statistics pass and the
 // apply pass as separate calls, so the caller can all-reduce the 2C per-layer sums across ranks in between.
-// sums [2][C] fp32 = (sum z, sum z^2) over this rank's P rows
+// sums [2][C] fp32 = (sum z, sum z^2) over this rank's P rows.  Unlike b2u_bn_fwd_train these are raw, unshifted sums: the
+// ranks add them up, and a per-rank pivot would not compose.  They keep the one-pass variance's loss of precision when a
+// channel's mean is large against its spread (the centred mode of the producing conv avoids that once running_mean is set).
 int b2u_bn_sums(const void* z, float* sums, void* ws, size_t ws_bytes, long long P, int C, void* stream) {
   int rc = bn_check(P, C, ws, ws_bytes, "bn_sums");
   if (rc) return rc;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   float* partial = static_cast<float*>(ws);
   bn_colsum_kernel<0><<<kBnBlocks, 256, 256 * 16 * sizeof(float), st>>>(static_cast<const uint4*>(z), nullptr, nullptr, nullptr,
-                                                                        nullptr, nullptr, nullptr, partial, P, C / 8, 0);
+                                                                        nullptr, nullptr, nullptr, partial, P, C / 8, 0, 0);
   B2U_CHECK_LAUNCH("bn_colsum");
   bn_rows_reduce_kernel<<<(2 * C + 31) / 32, 256, 0, st>>>(partial, sums, kBnBlocks, 2 * C);
   B2U_CHECK_LAUNCH("bn_rows_reduce");
@@ -405,7 +417,7 @@ int b2u_bn_fwd_train_sums(const void* z, const void* residual, void* y, const fl
   if (!sums || P_stat < P) return set_error(B2U_ERR_ARG, "bn_fwd_train_sums: sums missing or P_stat < P");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   float* coef = static_cast<float*>(ws) + static_cast<size_t>(kBnBlocks) * 2 * C;
-  bn_fwd_finalize_kernel<<<(C + 127) / 128, 128, 0, st>>>(sums, 1, C, P_stat, gamma, beta, running_mean, running_var,
+  bn_fwd_finalize_kernel<<<(C + 127) / 128, 128, 0, st>>>(sums, nullptr, 1, C, P_stat, gamma, beta, running_mean, running_var,
                                                           save_mean, save_invstd, coef, coef + C, eps, momentum, centered);
   B2U_CHECK_LAUNCH("bn_fwd_finalize");
   const long long G = (P + kBnApplyRows - 1) / kBnApplyRows;
@@ -426,7 +438,7 @@ int b2u_bn_bwd_sums(const void* dy, const void* y, const void* z, const float* g
   float* partial = static_cast<float*>(ws);
   bn_colsum_kernel<1><<<kBnBlocks, 256, 256 * 16 * sizeof(float), st>>>(static_cast<const uint4*>(dy), static_cast<const uint4*>(y),
                                                                         static_cast<const uint4*>(z), gamma, beta, save_mean,
-                                                                        save_invstd, partial, P, C / 8, relu);
+                                                                        save_invstd, partial, P, C / 8, relu, 0);
   B2U_CHECK_LAUNCH("bn_bwd_colsum");
   bn_rows_reduce_kernel<<<(2 * C + 31) / 32, 256, 0, st>>>(partial, sums, kBnBlocks, 2 * C);
   B2U_CHECK_LAUNCH("bn_rows_reduce");
@@ -494,7 +506,7 @@ int b2u_bn_bwd(const void* dy, const void* y, const void* z, const float* gamma,
   float* coef = partial + static_cast<size_t>(kBnBlocks) * 2 * C;
   bn_colsum_kernel<1><<<kBnBlocks, 256, 256 * 16 * sizeof(float), st>>>(static_cast<const uint4*>(dy), static_cast<const uint4*>(y),
                                                                         static_cast<const uint4*>(z), gamma, beta, save_mean,
-                                                                        save_invstd, partial, P, C / 8, relu);
+                                                                        save_invstd, partial, P, C / 8, relu, 0);
   B2U_CHECK_LAUNCH("bn_bwd_colsum");
   bn_bwd_finalize_kernel<<<(C + 127) / 128, 128, 0, st>>>(partial, kBnBlocks, C, P, gamma, beta, save_mean, save_invstd, dgamma,
                                                           dbeta, coef);
