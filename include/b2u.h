@@ -59,6 +59,15 @@ int b2u_nchw_f32_to_nhwc_bf16_padded(const float* x, void* y, int N, int C, int 
  * utils/utils.py:64-66), uint8 label map -> int64 (dataloader.py:43); 4 B/pixel over PCIe instead of 20 */
 int b2u_u8hwc_to_nchw_f32(const unsigned char* x, float* y, int N, int H, int W, int C, float scale, void* stream);
 int b2u_u8_to_i64(const unsigned char* x, long long* y, long long n, void* stream);
+/* the predictor's letterbox (utils/utils.py:22-34 resize_image + preprocess_input + transpose, unet.py:116-120) for a batch
+ * of uint8 RGB images of different sizes, bit-exact with PIL's Image.resize(..., BICUBIC) on a (128,128,128) canvas and
+ * numpy's float32 / 255.0.  An item is 64 B: {const uint8* src ([ih][iw][3], device); int ih, iw, nh, nw, dy, dx; int kx,
+ * ky; int64 coef_x, coef_y, tmp}.  The caller sets src .. dx in a HOST table (nw, nh = int(iw * scale), int(ih * scale),
+ * dx, dy = (W - nw) / 2, (H - nh) / 2, as resize_image computes them); b2u_letterbox_workspace fills kx .. tmp and returns
+ * the workspace bytes (0 and an error message if an item does not fit the H x W canvas).  b2u_letterbox_bicubic then
+ * reads that table from DEVICE memory and writes fp32 NCHW [count][3][H][W]; ws must hold the bytes the plan returned. */
+size_t b2u_letterbox_workspace(void* host_items, int count, int H, int W);
+int b2u_letterbox_bicubic(const void* items, int count, float* out, int H, int W, void* ws, size_t ws_bytes, void* stream);
 
 /* ---- tensor-core convolutions (tcgen05 implicit GEMM) ------------------------------------------------------ */
 /* y = [relu](conv(cat(x0, x1), w) + bias).  Replaces nn.Conv2d(k=3,p=1 | k=1)+ReLU (nets/vgg.py:53-57,
@@ -265,6 +274,12 @@ int b2u_argmax_u8(const float* logits, unsigned char* mask, int N, int C, int H,
  * INTER_LINEAR) of the probabilities to oh x ow, argmax -> uint8 mask [N][oh][ow]; nothing but the mask leaves the GPU */
 int b2u_softmax_resize_argmax_u8(const float* logits, unsigned char* mask, int N, int C, int H, int W, int cy, int cx,
                                  int ch, int cw, int oh, int ow, void* stream);
+/* the same tail for a batch whose images have their own crop and original size: logits [count][C][H][W]; items = count x
+ * {int cy, cx, ch, cw, oh, ow; int64 mask_off} (32 B each) in DEVICE memory, every crop inside H x W; image i's mask
+ * [oh][ow] goes to masks + mask_off (16-byte aligned offsets let the masks go straight to b2u_fast_hist_batch);
+ * max_oh, max_ow: the largest oh, ow of the batch.  Each pixel's class equals b2u_softmax_resize_argmax_u8's. */
+int b2u_softmax_resize_argmax_u8_batch(const float* logits, const void* items, int count, int C, int H, int W,
+                                       unsigned char* masks, int max_oh, int max_ow, void* stream);
 /* fast_hist (utils/utils_metrics.py:34-43): hist (n*n+1 uint64, accumulated) ; dtype 0=u8 1=i32 2=i64; 1 <= n <= 256 */
 int b2u_fast_hist(const void* a, const void* b, long long len, int n, int dtype, unsigned long long* hist, void* stream);
 /* compute_mIoU's loop over an evaluation set (utils/utils_metrics.py:74-95) in ONE launch: items = count x {const uint8* a;

@@ -29,6 +29,8 @@ SIGNATURES = {
     "b2u_nchw_f32_to_nhwc_bf16_padded": (I, [P, P, I, I, I, I, I, P]),
     "b2u_u8hwc_to_nchw_f32": (I, [P, P, I, I, I, I, F, P]),
     "b2u_u8_to_i64": (I, [P, P, LL, P]),
+    "b2u_letterbox_workspace": (SZ, [P, I, I, I]),
+    "b2u_letterbox_bicubic": (I, [P, I, P, I, I, P, SZ, P]),
     "b2u_conv_fprop": (I, [P, I, P, I, P, P, P, I, I, I, I, I, I, I, P]),
     "b2u_bn_sums": (I, [P, P, P, SZ, LL, I, P]),
     "b2u_bn_fwd_train_sums": (I, [P, P, P, P, P, P, P, P, P, P, LL, P, SZ, LL, I, F, F, I, P]),
@@ -91,6 +93,7 @@ SIGNATURES = {
     "b2u_head_fwd_tc": (I, [P, P, P, P, I, I, I, I, P]),
     "b2u_argmax_u8": (I, [P, P, I, I, I, I, P]),
     "b2u_softmax_resize_argmax_u8": (I, [P, P, I, I, I, I, I, I, I, I, I, I, P]),
+    "b2u_softmax_resize_argmax_u8_batch": (I, [P, P, I, I, I, I, P, I, I, P]),
     "b2u_fast_hist": (I, [P, P, LL, I, I, P, P]),
     "b2u_fast_hist_batch": (I, [P, I, LL, I, P, P]),
     "b2u_fast_hist_chunks": (LL, [LL]),

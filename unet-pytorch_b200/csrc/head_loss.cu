@@ -942,12 +942,14 @@ __global__ void argmax_u8_kernel(const float* __restrict__ logits, uint8_t* __re
 // one thread per output pixel interpolates the softmax of its 4 source pixels and keeps the best class, so only a
 // uint8 mask ever leaves the GPU.  cv2's float INTER_LINEAR: f = (d + 0.5) * in/out - 0.5, s = floor(f), f -= s;
 // s < 0 -> (s, f) = (0, 0); s >= in - 1 -> (s, f) = (in - 1, 0) (second tap clamped).
-template <int CM>
-__global__ void __launch_bounds__(128)
-softmax_resize_argmax_kernel(const float* __restrict__ logits, uint8_t* __restrict__ mask, int C, int H, int W, int cy,
-                             int cx, int ch, int cw, int oh, int ow, float sy, float sx) {
-  const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y, n = blockIdx.z;
-  if (x >= ow) return;
+// The per-pixel bodies are shared by the single-crop kernels and the batched kernel (one crop and output size per image),
+// so both give the same class for the same pixel.
+struct SraTaps {
+  size_t o[4];       // offsets of the 4 source pixels inside a class plane
+  float wgt[4];      // their bilinear weights
+};
+
+__device__ __forceinline__ SraTaps sra_taps(int W, int cy, int cx, int ch, int cw, int x, int y, float sy, float sx) {
   float fy = (y + 0.5f) * sy - 0.5f, fx = (x + 0.5f) * sx - 0.5f;
   int y0 = static_cast<int>(floorf(fy)), x0 = static_cast<int>(floorf(fx));
   fy -= y0; fx -= x0;
@@ -956,11 +958,16 @@ softmax_resize_argmax_kernel(const float* __restrict__ logits, uint8_t* __restri
   if (x0 < 0) { x0 = 0; fx = 0.f; }
   if (x0 >= cw - 1) { x0 = cw - 1; fx = 0.f; }
   const int y1 = y0 + 1 < ch ? y0 + 1 : ch - 1, x1 = x0 + 1 < cw ? x0 + 1 : cw - 1;
-  const size_t plane = static_cast<size_t>(H) * W;
-  const float* base = logits + static_cast<size_t>(n) * C * plane;
-  const size_t o[4] = {static_cast<size_t>(cy + y0) * W + cx + x0, static_cast<size_t>(cy + y0) * W + cx + x1,
-                       static_cast<size_t>(cy + y1) * W + cx + x0, static_cast<size_t>(cy + y1) * W + cx + x1};
-  const float wgt[4] = {(1.f - fy) * (1.f - fx), (1.f - fy) * fx, fy * (1.f - fx), fy * fx};
+  SraTaps t;
+  t.o[0] = static_cast<size_t>(cy + y0) * W + cx + x0; t.o[1] = static_cast<size_t>(cy + y0) * W + cx + x1;
+  t.o[2] = static_cast<size_t>(cy + y1) * W + cx + x0; t.o[3] = static_cast<size_t>(cy + y1) * W + cx + x1;
+  t.wgt[0] = (1.f - fy) * (1.f - fx); t.wgt[1] = (1.f - fy) * fx; t.wgt[2] = fy * (1.f - fx); t.wgt[3] = fy * fx;
+  return t;
+}
+
+// class of one output pixel, C <= CM <= 32; base = the image's logits [C][H][W]
+template <int CM>
+__device__ __forceinline__ int sra_pixel(const float* __restrict__ base, size_t plane, int C, const SraTaps& tp) {
   float acc[CM];
 #pragma unroll
   for (int c = 0; c < CM; ++c) acc[c] = 0.f;
@@ -969,58 +976,96 @@ softmax_resize_argmax_kernel(const float* __restrict__ logits, uint8_t* __restri
     float v[CM];
     float m = -INFINITY;
 #pragma unroll
-    for (int c = 0; c < CM; ++c) if (c < C) { v[c] = __ldg(base + c * plane + o[t]); m = fmaxf(m, v[c]); }
+    for (int c = 0; c < CM; ++c) if (c < C) { v[c] = __ldg(base + c * plane + tp.o[t]); m = fmaxf(m, v[c]); }
     float sum = 0.f;
 #pragma unroll
     for (int c = 0; c < CM; ++c) if (c < C) { v[c] = __expf(v[c] - m); sum += v[c]; }   // arguments <= 0: ex2.approx, <= 2 ulp near the max class
-    const float k = wgt[t] / sum;
+    const float k = tp.wgt[t] / sum;
 #pragma unroll
     for (int c = 0; c < CM; ++c) if (c < C) acc[c] = fmaf(k, v[c], acc[c]);
   }
   float best = acc[0]; int arg = 0;
 #pragma unroll
   for (int c = 1; c < CM; ++c) if (c < C && acc[c] > best) { best = acc[c]; arg = c; }
-  mask[(static_cast<size_t>(n) * oh + y) * ow + x] = static_cast<uint8_t>(arg);
+  return arg;
 }
 
-// softmax_resize_argmax_kernel for more than 32 classes, without per-class arrays: loop 1 gives each tap's max and sum
-// (the same max-then-sum order as the kernel above), loop 2 interpolates each class's probability and keeps a running
-// arg-max (strict >, so the lowest index wins ties)
-__global__ void __launch_bounds__(128)
-softmax_resize_argmax_wide_kernel(const float* __restrict__ logits, uint8_t* __restrict__ mask, int C, int H, int W, int cy,
-                                  int cx, int ch, int cw, int oh, int ow, float sy, float sx) {
-  const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y, n = blockIdx.z;
-  if (x >= ow) return;
-  float fy = (y + 0.5f) * sy - 0.5f, fx = (x + 0.5f) * sx - 0.5f;
-  int y0 = static_cast<int>(floorf(fy)), x0 = static_cast<int>(floorf(fx));
-  fy -= y0; fx -= x0;
-  if (y0 < 0) { y0 = 0; fy = 0.f; }
-  if (y0 >= ch - 1) { y0 = ch - 1; fy = 0.f; }
-  if (x0 < 0) { x0 = 0; fx = 0.f; }
-  if (x0 >= cw - 1) { x0 = cw - 1; fx = 0.f; }
-  const int y1 = y0 + 1 < ch ? y0 + 1 : ch - 1, x1 = x0 + 1 < cw ? x0 + 1 : cw - 1;
-  const size_t plane = static_cast<size_t>(H) * W;
-  const float* base = logits + static_cast<size_t>(n) * C * plane;
-  const size_t o[4] = {static_cast<size_t>(cy + y0) * W + cx + x0, static_cast<size_t>(cy + y0) * W + cx + x1,
-                       static_cast<size_t>(cy + y1) * W + cx + x0, static_cast<size_t>(cy + y1) * W + cx + x1};
-  const float wgt[4] = {(1.f - fy) * (1.f - fx), (1.f - fy) * fx, fy * (1.f - fx), fy * fx};
+// the same for more than 32 classes, without per-class arrays: loop 1 gives each tap's max and sum (the same max-then-sum
+// order as sra_pixel), loop 2 interpolates each class's probability and keeps a running arg-max (strict >, so the lowest
+// index wins ties)
+__device__ __forceinline__ int sra_pixel_wide(const float* __restrict__ base, size_t plane, int C, const SraTaps& tp) {
   float m[4], k[4];
 #pragma unroll
   for (int t = 0; t < 4; ++t) {
     m[t] = -INFINITY;
-    for (int c = 0; c < C; ++c) m[t] = fmaxf(m[t], __ldg(base + c * plane + o[t]));
+    for (int c = 0; c < C; ++c) m[t] = fmaxf(m[t], __ldg(base + c * plane + tp.o[t]));
     float sum = 0.f;
-    for (int c = 0; c < C; ++c) sum += __expf(__ldg(base + c * plane + o[t]) - m[t]);
-    k[t] = wgt[t] / sum;
+    for (int c = 0; c < C; ++c) sum += __expf(__ldg(base + c * plane + tp.o[t]) - m[t]);
+    k[t] = tp.wgt[t] / sum;
   }
   float best = -INFINITY; int arg = 0;
   for (int c = 0; c < C; ++c) {
     float acc = 0.f;
 #pragma unroll
-    for (int t = 0; t < 4; ++t) acc = fmaf(k[t], __expf(__ldg(base + c * plane + o[t]) - m[t]), acc);
+    for (int t = 0; t < 4; ++t) acc = fmaf(k[t], __expf(__ldg(base + c * plane + tp.o[t]) - m[t]), acc);
     if (c == 0 || acc > best) { best = acc; arg = c; }
   }
-  mask[(static_cast<size_t>(n) * oh + y) * ow + x] = static_cast<uint8_t>(arg);
+  return arg;
+}
+
+// CM = 0: the wide body (the batched kernel's dispatch)
+template <int CM>
+__device__ __forceinline__ int sra_class(const float* __restrict__ base, size_t plane, int C, const SraTaps& tp) {
+  if constexpr (CM == 0) return sra_pixel_wide(base, plane, C, tp);
+  else return sra_pixel<CM>(base, plane, C, tp);
+}
+
+template <int CM>
+__global__ void __launch_bounds__(128)
+softmax_resize_argmax_kernel(const float* __restrict__ logits, uint8_t* __restrict__ mask, int C, int H, int W, int cy,
+                             int cx, int ch, int cw, int oh, int ow, float sy, float sx) {
+  const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y, n = blockIdx.z;
+  if (x >= ow) return;
+  const size_t plane = static_cast<size_t>(H) * W;
+  const SraTaps tp = sra_taps(W, cy, cx, ch, cw, x, y, sy, sx);
+  mask[(static_cast<size_t>(n) * oh + y) * ow + x] =
+      static_cast<uint8_t>(sra_pixel<CM>(logits + static_cast<size_t>(n) * C * plane, plane, C, tp));
+}
+
+__global__ void __launch_bounds__(128)
+softmax_resize_argmax_wide_kernel(const float* __restrict__ logits, uint8_t* __restrict__ mask, int C, int H, int W, int cy,
+                                  int cx, int ch, int cw, int oh, int ow, float sy, float sx) {
+  const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y, n = blockIdx.z;
+  if (x >= ow) return;
+  const size_t plane = static_cast<size_t>(H) * W;
+  const SraTaps tp = sra_taps(W, cy, cx, ch, cw, x, y, sy, sx);
+  mask[(static_cast<size_t>(n) * oh + y) * ow + x] =
+      static_cast<uint8_t>(sra_pixel_wide(logits + static_cast<size_t>(n) * C * plane, plane, C, tp));
+}
+
+// one image of a batched tail call (32 bytes, include/b2u.h)
+struct SraItem {
+  int cy, cx, ch, cw, oh, ow;
+  long long mask_off;   // byte offset of the image's [oh][ow] mask in the flat output
+};
+static_assert(sizeof(SraItem) == 32, "SraItem is part of the ABI");
+
+// blockIdx.z = image; rows and columns are strided over the grid, which is sized for the largest image of the batch
+template <int CM>
+__global__ void __launch_bounds__(128)
+softmax_resize_argmax_batch_kernel(const float* __restrict__ logits, const SraItem* __restrict__ items,
+                                   uint8_t* __restrict__ masks, int C, int H, int W) {
+  const SraItem it = items[blockIdx.z];
+  if (it.cy < 0 || it.cx < 0 || it.ch <= 0 || it.cw <= 0 || it.cy + it.ch > H || it.cx + it.cw > W) return;
+  const float sy = static_cast<float>(__ddiv_rn(static_cast<double>(it.ch), static_cast<double>(it.oh)));
+  const float sx = static_cast<float>(__ddiv_rn(static_cast<double>(it.cw), static_cast<double>(it.ow)));
+  const size_t plane = static_cast<size_t>(H) * W;
+  const float* base = logits + static_cast<size_t>(blockIdx.z) * C * plane;
+  uint8_t* mask = masks + it.mask_off;
+  for (int y = blockIdx.y; y < it.oh; y += gridDim.y)
+    for (int x = blockIdx.x * blockDim.x + threadIdx.x; x < it.ow; x += gridDim.x * blockDim.x)
+      mask[static_cast<size_t>(y) * it.ow + x] =
+          static_cast<uint8_t>(sra_class<CM>(base, plane, C, sra_taps(W, it.cy, it.cx, it.ch, it.cw, x, y, sy, sx)));
 }
 
 }  // namespace b2u
@@ -1234,6 +1279,25 @@ int b2u_softmax_resize_argmax_u8(const float* logits, unsigned char* mask, int N
   else softmax_resize_argmax_wide_kernel<<<grid, 128, 0, st>>>(logits, mask, C, H, W, cy, cx, ch, cw, oh, ow, sy, sx);
 #undef B2U_SRA
   B2U_CHECK_LAUNCH("softmax_resize_argmax");
+  return 0;
+}
+
+// logits [count][C][H][W] fp32; items: count x {int cy, cx, ch, cw, oh, ow; int64 mask_off} (32 B each) in DEVICE memory,
+// every crop inside H x W (an item whose crop is not is left unwritten); masks: flat uint8, image i's [oh][ow] mask at
+// mask_off; max_oh / max_ow: the largest oh / ow of the batch (grid size only)
+int b2u_softmax_resize_argmax_u8_batch(const float* logits, const void* items, int count, int C, int H, int W,
+                                       unsigned char* masks, int max_oh, int max_ow, void* stream) {
+  if (!logits || !items || !masks || count <= 0 || count > 65535 || C <= 0 || C > kMaxClsWide || H <= 0 || W <= 0 ||
+      max_oh <= 0 || max_ow <= 0)
+    return set_error(B2U_ERR_SHAPE, "softmax_resize_argmax_batch: bad shape");
+  const dim3 grid((max_ow + 127) / 128, max_oh < 65535 ? max_oh : 65535, count);
+  const SraItem* it = static_cast<const SraItem*>(items);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+#define B2U_SRAB(CM_) softmax_resize_argmax_batch_kernel<CM_><<<grid, 128, 0, st>>>(logits, it, masks, C, H, W)
+  if (C <= 8) B2U_SRAB(8); else if (C <= 16) B2U_SRAB(16); else if (C <= 24) B2U_SRAB(24); else if (C <= 32) B2U_SRAB(32);
+  else B2U_SRAB(0);
+#undef B2U_SRAB
+  B2U_CHECK_LAUNCH("softmax_resize_argmax_batch");
   return 0;
 }
 

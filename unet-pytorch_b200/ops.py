@@ -4,6 +4,9 @@ Activations are NHWC bf16 CUDA tensors ([N, H, W, C], contiguous); parameters an
 fp32 OIHW / NCHW layouts.  Every function launches on torch's current stream and allocates its outputs and
 workspaces with torch's caching allocator; none of them has a CPU or PyTorch fallback.
 """
+import ctypes
+import struct
+
 import torch
 
 from . import _lib
@@ -840,6 +843,66 @@ def softmax_resize_argmax_u8(logits, crop, out_size, out=None):
     return out
 
 
+def pad16(nbytes):
+    """Byte offsets of the batched predictor's ragged buffers are multiples of 16 (fast_hist_batch reads 16-byte vectors)."""
+    return (int(nbytes) + 15) & ~15
+
+
+LETTERBOX_ITEM = struct.Struct("<Q8i3q")     # include/b2u.h: src; ih, iw, nh, nw, dy, dx, kx, ky; coef_x, coef_y, tmp
+TAIL_ITEM = struct.Struct("<6iq")            # include/b2u.h: cy, cx, ch, cw, oh, ow; mask_off
+
+
+def letterbox_plan(items, H, W):
+    """Host half of the batched letterbox.  items: (src device address of a uint8 [ih, iw, 3] image, ih, iw, nh, nw, dy, dx)
+    per image, with resize_image's geometry.  Returns (item table as bytes, workspace bytes) for letterbox_bicubic."""
+    if not items:
+        raise ValueError("letterbox: empty batch")
+    blob = bytearray(b"".join(LETTERBOX_ITEM.pack(int(p), *map(int, g), 0, 0, 0, 0, 0) for p, *g in items))
+    buf = (ctypes.c_char * len(blob)).from_buffer(blob)
+    ws = lib().b2u_letterbox_workspace(ctypes.addressof(buf), len(items), H, W)
+    del buf
+    if ws == 0:
+        msg = lib().b2u_last_error()
+        raise ValueError(f"b2u: {msg.decode() if msg else 'letterbox_workspace failed'}")
+    return bytes(blob), ws
+
+
+def letterbox_bicubic(table, count, out, ws):
+    """PIL BICUBIC letterbox of `count` images into fp32 NCHW out[:count] ([>= count, 3, H, W]), bit-exact with
+    resize_image + np.float32 / 255; table: letterbox_plan's bytes in a uint8 CUDA tensor, ws: uint8 CUDA workspace."""
+    _req(table, torch.uint8, "table"); _req(out, torch.float32, "out"); _req(ws, torch.uint8, "ws")
+    if out.dim() != 4 or out.shape[0] < count or out.shape[1] != 3 or table.numel() < count * LETTERBOX_ITEM.size:
+        raise ValueError("letterbox: out must be [>= count, 3, H, W] and the table must hold count items")
+    check(lib().b2u_letterbox_bicubic(ptr(table), count, ptr(out), out.shape[2], out.shape[3], ptr(ws), ws.numel(),
+                                      stream_ptr()))
+    return out
+
+
+def tail_table(crops, sizes, H, W):
+    """Item table of softmax_resize_argmax_u8_batch: crop (y, x, h, w) inside H x W and output size (oh, ow) per image.
+    Returns (bytes, mask byte offsets (16-byte aligned), total mask bytes)."""
+    blob, offs, off = [], [], 0
+    for (cy, cx, ch, cw), (oh, ow) in zip(crops, sizes):
+        if cy < 0 or cx < 0 or ch <= 0 or cw <= 0 or cy + ch > H or cx + cw > W or oh <= 0 or ow <= 0:
+            raise ValueError(f"softmax_resize_argmax_batch: crop {(cy, cx, ch, cw)} / size {(oh, ow)} outside {H}x{W}")
+        blob.append(TAIL_ITEM.pack(cy, cx, ch, cw, oh, ow, off))
+        offs.append(off)
+        off = pad16(off + oh * ow)
+    return b"".join(blob), offs, off
+
+
+def softmax_resize_argmax_u8_batch(logits, table, count, masks, max_oh, max_ow):
+    """softmax_resize_argmax_u8 with one crop and output size per image: image i's mask goes to the flat uint8 `masks` at
+    the offset tail_table gave it; table: tail_table's bytes in a uint8 CUDA tensor."""
+    _req(logits, torch.float32, "logits"); _req(table, torch.uint8, "table"); _req(masks, torch.uint8, "masks")
+    N, C, H, W = logits.shape
+    if count > N or table.numel() < count * TAIL_ITEM.size:
+        raise ValueError("softmax_resize_argmax_batch: more items than logits or table entries")
+    check(lib().b2u_softmax_resize_argmax_u8_batch(ptr(logits), ptr(table), count, C, H, W, ptr(masks), max_oh, max_ow,
+                                                   stream_ptr()))
+    return masks
+
+
 _HIST_DTYPES = {torch.uint8: 0, torch.int32: 1, torch.int64: 2}
 
 
@@ -854,23 +917,30 @@ def fast_hist_accumulate(a, b, n, hist):
     return hist
 
 
+def hist_items(pairs):
+    """Item table of fast_hist_batch from (a address, b address, length) per uint8 mask pair, both 16-byte aligned.
+    Returns (table bytes, total chunks)."""
+    blob, chunks = [], 0
+    chunk_fn = lib().b2u_fast_hist_chunks
+    for a, b, n in pairs:
+        if a % 16 or b % 16:
+            raise ValueError("fast_hist_batch: masks must be 16-byte aligned")
+        blob.append(struct.pack("<QQqq", a, b, n, chunks))
+        chunks += chunk_fn(n)
+    return b"".join(blob), chunks
+
+
 class HistTable:
     """Device-resident pointer table of (a, b) uint8 CUDA mask pairs for fast_hist_batch (keeps the masks alive)."""
 
     def __init__(self, pairs, device):
-        import struct
-        blob, chunks = [], 0
-        chunk_fn = lib().b2u_fast_hist_chunks
         for a, b in pairs:
             _req(a, torch.uint8, "a"); _req(b, torch.uint8, "b")
             if a.numel() != b.numel():
                 raise ValueError("fast_hist_batch: a and b must have the same number of elements")
-            if a.data_ptr() % 16 or b.data_ptr() % 16:
-                raise ValueError("fast_hist_batch: masks must be 16-byte aligned")
-            blob.append(struct.pack("<QQqq", a.data_ptr(), b.data_ptr(), a.numel(), chunks))
-            chunks += chunk_fn(a.numel())
-        self.pairs, self.count, self.chunks = list(pairs), len(blob), chunks
-        self.table = torch.frombuffer(bytearray(b"".join(blob)), dtype=torch.uint8).to(device) if blob else None
+        blob, chunks = hist_items([(a.data_ptr(), b.data_ptr(), a.numel()) for a, b in pairs])
+        self.pairs, self.count, self.chunks = list(pairs), len(pairs), chunks
+        self.table = torch.frombuffer(bytearray(blob), dtype=torch.uint8).to(device) if blob else None
 
 
 def fast_hist_batch(pairs, n, hist):
@@ -879,6 +949,17 @@ def fast_hist_batch(pairs, n, hist):
     tab = pairs if isinstance(pairs, HistTable) else HistTable(pairs, hist.device)
     if tab.count:
         check(lib().b2u_fast_hist_batch(ptr(tab.table), tab.count, tab.chunks, n, ptr(hist), stream_ptr()))
+    return hist
+
+
+def fast_hist_batch_items(table, count, chunks, n, hist):
+    """fast_hist_batch over an item table already in device memory (hist_items' bytes in a uint8 CUDA tensor); the caller
+    keeps the masks alive until the launch has run."""
+    _req(table, torch.uint8, "table"); _req(hist, torch.int64, "hist")
+    if table.numel() < 32 * count:
+        raise ValueError("fast_hist_batch: the table holds fewer than count items")
+    if count:
+        check(lib().b2u_fast_hist_batch(ptr(table), count, chunks, n, ptr(hist), stream_ptr()))
     return hist
 
 

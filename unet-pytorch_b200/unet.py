@@ -1,13 +1,16 @@
 """Drop-in for the reference's predictor class `unet.py::Unet` (lines 19-357): same keyword configuration
 (`model_path`, `num_classes`, `backbone`, `input_shape`, `mix_type`, `cuda`), same `detect_image`, `get_FPS`,
-`get_miou_png` results -- with the per-frame tail moved onto the GPU (SURVEY.md 8(f) rank 1).
+`get_miou_png` results -- with the per-frame work moved onto the GPU (SURVEY.md 8(f) rank 1) and batched.
 
-Reference per frame: logits -> softmax -> .cpu().numpy() (H x W x C fp32, 22 MB at C = 21, 512^2) -> crop of the letterbox
-bars -> cv2.resize of the probabilities to the original size -> argmax (unet.py:131-148).  Here: logits stay on the device,
-one kernel (`b2u_softmax_resize_argmax_u8`) does softmax + crop + INTER_LINEAR resize + argmax, and a uint8 mask (1 byte
-per pixel) is the only thing copied back.  Host-side image handling (RGB conversion, BICUBIC letterbox with grey bars,
-colour blending) follows utils/utils.py:12-34 and unet.py:150-203 with PIL/numpy, as in the reference."""
+Reference per frame: PIL BICUBIC letterbox with grey bars -> / 255 -> batch-1 forward -> softmax -> .cpu().numpy()
+(H x W x C fp32, 22 MB at C = 21, 512^2) -> crop of the letterbox bars -> cv2.resize of the probabilities to the original
+size -> argmax (utils/utils.py:22-34, unet.py:116-148).  Here, per batch of images of any sizes: the raw uint8 RGB bytes
+go up in one pinned copy, `b2u_letterbox_bicubic` builds the network input (bit-exact with PIL's BICUBIC resize and
+numpy's / 255), one forward runs the whole batch, and `b2u_softmax_resize_argmax_u8_batch` (softmax + crop +
+INTER_LINEAR resize + argmax) writes every image's uint8 mask into one flat buffer, the only thing copied back.  RGB
+conversion and colour blending stay on the host with PIL/numpy, as in the reference (unet.py:150-203)."""
 import colorsys
+import itertools
 import time
 
 import numpy as np
@@ -48,6 +51,12 @@ def resize_image(image, size):                         # utils/utils.py:22-34: u
     return canvas, nw, nh
 
 
+def _chunks(iterable, n):
+    it = iter(iterable)
+    while chunk := list(itertools.islice(it, n)):
+        yield chunk
+
+
 class Unet(object):
     _defaults = {
         "model_path": "model_data/unet_vgg_voc.pth",
@@ -81,6 +90,7 @@ class Unet(object):
 
     # ------------------------------------------------------------------ shared pieces
     def _letterbox(self, image):
+        """The host letterbox of the reference (PIL BICUBIC + numpy); the batched path computes the same tensor on the GPU."""
         image = cvtColor(image)
         oh, ow = np.array(image).shape[:2]
         boxed, nw, nh = resize_image(image, (self.input_shape[1], self.input_shape[0]))
@@ -90,44 +100,132 @@ class Unet(object):
     def _crop(self, nw, nh):
         return (int((self.input_shape[0] - nh) // 2), int((self.input_shape[1] - nw) // 2), nh, nw)
 
+    def _prepare(self, image):
+        """Host part of one image: cvtColor (the RGB view is returned for detect_image), its uint8 [h, w, 3] bytes and
+        resize_image's geometry (ih, iw, nh, nw, dy, dx)."""
+        arr = np.asarray(image)
+        if not (arr.ndim == 3 and arr.shape[2] == 3):       # cvtColor's test, without converting the image twice
+            image = image.convert("RGB")
+            arr = np.asarray(image)
+        ih, iw = arr.shape[:2]
+        if ih == 0 or iw == 0:
+            raise ValueError(f"predictor: empty image ({iw}x{ih})")
+        h, w = self.input_shape
+        scale = min(w / iw, h / ih)
+        nw, nh = int(iw * scale), int(ih * scale)
+        if nw == 0 or nh == 0:
+            raise ValueError(f"predictor: a {iw}x{ih} image letterboxes to {nw}x{nh} pixels")
+        return image, np.ascontiguousarray(arr, dtype=np.uint8), (ih, iw, nh, nw, (h - nh) // 2, (w - nw) // 2)
+
+    def _buffer(self, name, nbytes, pinned=False):
+        """Staging buffers reused across batches, grown on demand (uint8)."""
+        buf = getattr(self, name, None)
+        if buf is None or buf.numel() < nbytes:
+            nbytes = max(int(nbytes * 1.25), 4096)
+            buf = torch.empty(nbytes, dtype=torch.uint8, pin_memory=True) if pinned else \
+                torch.empty(nbytes, dtype=torch.uint8, device=self.device)
+            setattr(self, name, buf)
+        return buf
+
+    def _run_batch(self, prepared, gts=None):
+        """One batch on the device: a single pinned host-to-device copy of [letterbox table | tail table | histogram table |
+        images | ground truths], the letterbox kernels into the reused input buffer, one forward, the batched tail.
+        Returns (flat uint8 mask buffer, per-image (offset, oh, ow), total mask bytes, histogram items) where the
+        histogram items (device table, count, chunks) pair each ground truth of the image's size with its mask (None
+        without gts).  Must run under torch.no_grad()."""
+        b = len(prepared)
+        H, W = self.input_shape
+        sizes = [(ih, iw) for _, _, (ih, iw, _, _, _, _) in prepared]
+        crops = [(dy, dx, nh, nw) for _, _, (_, _, nh, nw, dy, dx) in prepared]
+        tail, mask_offs, mask_bytes = ops.tail_table(crops, sizes, H, W)
+        masks = self._buffer("_masks", mask_bytes)
+        tail_at = ops.pad16(b * ops.LETTERBOX_ITEM.size)
+        hist_at = tail_at + ops.pad16(len(tail))
+        counted = [i for i, g in enumerate(gts or ()) if g.size == sizes[i][0] * sizes[i][1]]   # the others are skipped
+        off = hist_at + ops.pad16(32 * len(counted))
+        src_offs, gt_offs = [], []
+        for _, arr, _ in prepared:
+            src_offs.append(off)
+            off = ops.pad16(off + arr.nbytes)
+        for g in gts or ():
+            gt_offs.append(off)
+            off = ops.pad16(off + g.nbytes)
+        total = off
+        if getattr(self, "_staged", None) is not None:
+            self._staged.synchronize()                      # the previous batch's copy has left the pinned buffer
+        host, dev = self._buffer("_host_stage", total, pinned=True), self._buffer("_dev_stage", total)
+        base = dev.data_ptr()
+        lb, ws_bytes = ops.letterbox_plan([(base + o, *geo) for o, (_, _, geo) in zip(src_offs, prepared)], H, W)
+        hist_tab, chunks = ops.hist_items([(base + gt_offs[i], masks.data_ptr() + mask_offs[i], gts[i].size) for i in counted])
+        hn = host.numpy()
+        for at, blob in ((0, lb), (tail_at, tail), (hist_at, hist_tab)):
+            hn[at:at + len(blob)] = np.frombuffer(blob, np.uint8)
+        for o, (_, arr, _) in zip(src_offs, prepared):
+            hn[o:o + arr.nbytes] = arr.reshape(-1)
+        for o, g in zip(gt_offs, gts or ()):
+            hn[o:o + g.nbytes] = g.reshape(-1)
+        dev[:total].copy_(host[:total], non_blocking=True)
+        self._staged = torch.cuda.Event()
+        self._staged.record()
+        x = getattr(self, "_input", None)
+        if x is None or x.shape[0] < b:
+            x = self._input = torch.empty((b, 3, H, W), dtype=torch.float32, device=self.device)
+        ws = self._buffer("_lb_ws", ws_bytes)
+        ops.letterbox_bicubic(dev[:len(lb)], b, x, ws)
+        logits = self.net(x[:b])
+        ops.softmax_resize_argmax_u8_batch(logits, dev[tail_at:tail_at + len(tail)], b, masks,
+                                           max(h for h, _ in sizes), max(w for _, w in sizes))
+        hist_items = (dev[hist_at:hist_at + max(len(hist_tab), 16)], len(counted), chunks) if gts is not None else None
+        return masks, [(o, h, w) for o, (h, w) in zip(mask_offs, sizes)], mask_bytes, hist_items
+
+    def predict_masks(self, images, batch_size=16):
+        """uint8 class maps, one per image at the image's original size, each equal to predict_mask(image)[1]; the images
+        run through the device letterbox, the forward and the tail `batch_size` at a time."""
+        return [m for _, m in self._predict(images, batch_size)]
+
+    def _predict(self, images, batch_size):
+        if batch_size < 1:
+            raise ValueError("predict_masks: batch_size must be >= 1")
+        out = []
+        for chunk in _chunks(images, batch_size):
+            prepared = [self._prepare(im) for im in chunk]
+            with torch.no_grad():
+                masks, layout, nbytes, _ = self._run_batch(prepared)
+            host = self._buffer("_host_masks", nbytes, pinned=True)
+            host[:nbytes].copy_(masks[:nbytes], non_blocking=True)
+            torch.cuda.current_stream().synchronize()
+            hn = host.numpy()
+            out.extend((p[0], hn[o:o + h * w].reshape(h, w).copy()) for p, (o, h, w) in zip(prepared, layout))
+        return out
+
     def predict_mask(self, image):
         """uint8 class map at the original image size (the `pr` of unet.py:148 / 340)."""
-        image, data, nw, nh, oh, ow = self._letterbox(image)
-        with torch.no_grad():
-            logits = self.net(data.to(self.device, non_blocking=True))
-            mask = ops.softmax_resize_argmax_u8(logits, self._crop(nw, nh), (oh, ow))
-        return image, mask[0].cpu().numpy()
+        return self._predict([image], 1)[0]
 
     def predict_mask_device(self, image):
         """The same class map, left on the device (uint8 [H, W] CUDA tensor)."""
-        _, data, nw, nh, oh, ow = self._letterbox(image)
         with torch.no_grad():
-            logits = self.net(data.to(self.device, non_blocking=True))
-            return ops.softmax_resize_argmax_u8(logits, self._crop(nw, nh), (oh, ow))[0]
+            masks, [(o, h, w)], _, _ = self._run_batch([self._prepare(image)])
+        return masks[o:o + h * w].view(h, w).clone()
 
-    def get_miou(self, images, gts):
-        """get_miou.py:45-65 + utils_metrics.compute_mIoU (:58-126) without the PNG round trip: every prediction stays on
-        the GPU and is folded into one device-resident confusion matrix (`fast_hist`), read back once at the end.
-        images: iterable of PIL images; gts: iterable of label maps (PIL 'L'/'P' images or uint8 arrays, 255 = ignore).
+    def get_miou(self, images, gts, batch_size=16):
+        """get_miou.py:45-65 + utils_metrics.compute_mIoU (:58-126) without the PNG round trip: the images run in batches
+        of `batch_size` (device letterbox, forward, batched tail), and each batch's masks are folded with their ground
+        truths into one device-resident confusion matrix (`fast_hist_batch`), read back once at the end.
+        images: iterable of PIL images; gts: iterable of label maps (PIL 'L'/'P' images or uint8 arrays, 255 = ignore);
+        a pair whose sizes differ is skipped (utils_metrics.py:88-93).
         Returns (hist int64 [n, n], IoUs, PA_Recall, Precision) like compute_mIoU."""
         from .utils.utils_metrics import per_class_iu, per_class_PA_Recall, per_class_Precision
+        if batch_size < 1:
+            raise ValueError("get_miou: batch_size must be >= 1")
         n = self.num_classes
         hist = torch.zeros(n * n + 1, dtype=torch.int64, device=self.device)
-        pairs = []
-
-        def flush():
-            if pairs:
-                ops.fast_hist_batch(pairs, n, hist)       # one launch for the whole group of masks
-                pairs.clear()
-        for image, gt in zip(images, gts):
-            pred = self.predict_mask_device(image)
-            g = torch.from_numpy(np.ascontiguousarray(np.array(gt, dtype=np.uint8))).to(self.device, non_blocking=True)
-            if g.numel() != pred.numel():          # utils_metrics.py:88-93: mismatching pairs are skipped
-                continue
-            pairs.append((g.reshape(-1), pred.reshape(-1).contiguous()))
-            if len(pairs) == 256:
-                flush()
-        flush()
+        for chunk in _chunks(zip(images, gts), batch_size):
+            prepared = [self._prepare(im) for im, _ in chunk]
+            garr = [np.ascontiguousarray(np.array(gt, dtype=np.uint8)) for _, gt in chunk]
+            with torch.no_grad():
+                _, _, _, (table, count, chunks) = self._run_batch(prepared, garr)
+            ops.fast_hist_batch_items(table, count, chunks, n, hist)      # one launch per batch, no host synchronisation
         h = hist.cpu().numpy()
         if h[-1] != 0:
             raise ValueError("predictions outside [0, num_classes)")
