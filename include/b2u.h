@@ -280,6 +280,14 @@ int b2u_softmax_resize_argmax_u8(const float* logits, unsigned char* mask, int N
  * max_oh, max_ow: the largest oh, ow of the batch.  Each pixel's class equals b2u_softmax_resize_argmax_u8's. */
 int b2u_softmax_resize_argmax_u8_batch(const float* logits, const void* items, int count, int C, int H, int W,
                                        unsigned char* masks, int max_oh, int max_ow, void* stream);
+/* detect_image's rendering (unet.py:150-203) for a batch: items = count x {const uint8* src ([ih][iw][3] RGB); const uint8*
+ * mask ([ih][iw], from the batched tail); int64 out_off; int ih, iw} (32 B each) in DEVICE memory; palette: [C][3] uint8,
+ * device.  mix_type 0 writes Image.blend(src, palette[mask], 0.7) (Pillow's float32 arithmetic without FMA, truncated),
+ * 1 palette[mask], 2 src where mask != 0 else 0, each to out + out_off as [ih][iw][3]; -1 writes no image (out, palette may
+ * be NULL).  counts (nullable): [count][C] uint64, cleared by the call, then the per-image pixel count of each class.
+ * max_pixels: the largest ih * iw of the batch; 1 <= C <= 255.  One kernel launch per batch. */
+int b2u_render_batch(const void* items, int count, const unsigned char* palette, int C, int mix_type, unsigned char* out,
+                     unsigned long long* counts, long long max_pixels, void* stream);
 /* fast_hist (utils/utils_metrics.py:34-43): hist (n*n+1 uint64, accumulated) ; dtype 0=u8 1=i32 2=i64; 1 <= n <= 256 */
 int b2u_fast_hist(const void* a, const void* b, long long len, int n, int dtype, unsigned long long* hist, void* stream);
 /* compute_mIoU's loop over an evaluation set (utils/utils_metrics.py:74-95) in ONE launch: items = count x {const uint8* a;

@@ -105,7 +105,7 @@ def main():
     prepared = [pred._prepare(im) for im in images[:64]]
     dev_ms = {}
     with torch.no_grad():
-        masks, layout, nbytes, _ = pred._run_batch(prepared)        # leaves this batch's tables in the device staging buffer
+        masks, layout, nbytes, _, _ = pred._run_batch(prepared)        # leaves this batch's tables in the device staging buffer
         tail_at = ops.pad16(64 * ops.LETTERBOX_ITEM.size)
         x = pred._input[:64]
         logits = pred.net(x)

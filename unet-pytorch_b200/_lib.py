@@ -94,6 +94,7 @@ SIGNATURES = {
     "b2u_argmax_u8": (I, [P, P, I, I, I, I, P]),
     "b2u_softmax_resize_argmax_u8": (I, [P, P, I, I, I, I, I, I, I, I, I, I, P]),
     "b2u_softmax_resize_argmax_u8_batch": (I, [P, P, I, I, I, I, P, I, I, P]),
+    "b2u_render_batch": (I, [P, I, P, I, I, P, P, LL, P]),
     "b2u_fast_hist": (I, [P, P, LL, I, I, P, P]),
     "b2u_fast_hist_batch": (I, [P, I, LL, I, P, P]),
     "b2u_fast_hist_chunks": (LL, [LL]),

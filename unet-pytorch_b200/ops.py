@@ -903,6 +903,36 @@ def softmax_resize_argmax_u8_batch(logits, table, count, masks, max_oh, max_ow):
     return masks
 
 
+RENDER_ITEM = struct.Struct("<QQq2i")       # include/b2u.h: src, mask; out_off; ih, iw
+
+
+def render_table(items, start=0):
+    """Item table of render_batch from (src address, mask address, ih, iw) per image; each rendered [ih, iw, 3] image gets a
+    16-byte aligned offset from `start` on.  Returns (bytes, image offsets, end offset)."""
+    blob, offs, off = [], [], pad16(start)
+    for src, mask, ih, iw in items:
+        if ih <= 0 or iw <= 0 or not src or not mask:
+            raise ValueError(f"render_batch: bad item ({ih}x{iw})")
+        blob.append(RENDER_ITEM.pack(src, mask, off, ih, iw))
+        offs.append(off)
+        off = pad16(off + 3 * ih * iw)
+    return b"".join(blob), offs, off
+
+
+def render_batch(table, count, palette, C, mix_type, out, counts, max_pixels):
+    """detect_image's rendering of `count` images in one launch (mix_type 0: blend with 0.7, 1: palette, 2: keep the
+    non-background pixels, -1: counts only): table is render_table's bytes in a uint8 CUDA tensor, palette a uint8 CUDA
+    tensor of >= 3 C bytes, out the flat uint8 buffer the offsets point into, counts (optional) int64 [>= count * C]."""
+    _req(table, torch.uint8, "table"); _req(palette, torch.uint8, "palette"); _req(out, torch.uint8, "out")
+    _req(counts, torch.int64, "counts")
+    if table.numel() < count * RENDER_ITEM.size or (palette is not None and palette.numel() < 3 * C) or \
+            (counts is not None and counts.numel() < count * C):
+        raise ValueError("render_batch: the table, palette or counts hold fewer entries than count / C")
+    check(lib().b2u_render_batch(ptr(table), count, ptr(palette), C, mix_type, ptr(out), ptr(counts), max_pixels,
+                                 stream_ptr()))
+    return out
+
+
 _HIST_DTYPES = {torch.uint8: 0, torch.int32: 1, torch.int64: 2}
 
 
