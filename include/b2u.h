@@ -124,7 +124,8 @@ int b2u_conv_dgrad(const void* dz, int Cz, const void* wd, void* dx0, int C0, vo
                    int N, int H, int W, int taps, int bn_override, void* stream);
 /* wgrad: dw (OIHW fp32, overwritten) = sum over pixels of dz (x) cat(x0, x1); db (nullable, [Cout]) = sum over pixels
  * of dz, from the same pass.  first_cin > 0: x0 is the im2col tensor of b2u_im2col_first and dw is
- * [Cout][first_cin][3][3].  flags bit0: unmerged vertical taps (debug). */
+ * [Cout][first_cin][3][3].  flags bit1: never use the swapped-role Cout = 64 kernel (tests); any other bit set returns
+ * B2U_ERR_ARG. */
 size_t b2u_conv_wgrad_workspace(int N, int H, int W, int Cin_tot, int Cout, int taps);
 int b2u_conv_wgrad(const void* x0, int C0, const void* x1, int C1, const void* dz, int Cout, float* dw, float* db, void* ws,
                    size_t ws_bytes, int N, int H, int W, int taps, int first_cin, int flags, void* stream);

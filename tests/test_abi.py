@@ -39,6 +39,17 @@ def test_version_and_error_channel_without_gpu(b2u):
     assert lib.b2u_conv_wgrad_workspace(16, 512, 512, 64, 64, 9) > 0
 
 
+def test_conv_wgrad_rejects_undefined_flags(b2u):
+    """b2u_conv_wgrad defines flags bit 1 only (force the generic kernel); the product and the fp32 validation library both
+    reject any other bit before touching the GPU."""
+    fp32 = ctypes.CDLL(b2u._lib.LIB_PATH_FP32)
+    fp32.b2u_last_error.restype = ctypes.c_char_p
+    for lib in (b2u._lib.lib(), fp32):
+        for flags in (1, 3, 4):
+            rc = lib.b2u_conv_wgrad(None, 64, None, 0, None, 64, None, None, None, 0, 1, 8, 16, 9, 0, flags, None)
+            assert rc == 5 and b"flags" in lib.b2u_last_error(), (lib, flags)       # B2U_ERR_ARG
+
+
 def test_product_path_has_no_cpu_fallback(b2u):
     m = b2u.Unet(num_classes=2)
     with pytest.raises(RuntimeError):

@@ -154,7 +154,7 @@ def test_lightweight_state_dict_and_program_contract(b2u):
         b2u.LightweightUnet(num_classes=2, backbone="resnet50")
 
 
-def test_fused_upsample_planning(b2u, monkeypatch):
+def test_fused_upsample_planning(b2u):
     """Which "up" instructions the graph engines leave to the decoder conv (b2u_decoder_conv_fprop): only up-sampled tensors read
     exactly once, as the SECOND source of a stride-1 3x3 conv (unetUp, nets/unet.py:16-18) -- Unet-ResNet50's four decoder
     stages and LightweightUnet's (nets/LightWeightUnet.py concatenates [skip, up] too); the UltraLightweight family concatenates
@@ -162,20 +162,14 @@ def test_fused_upsample_planning(b2u, monkeypatch):
     from unet_pytorch_b200.graph import LightweightUnetEngine, ResNet50UnetEngine, UltraLightUnetEngine
     from unet_pytorch_b200.engine import VGGUnetEngine
     eng = ResNet50UnetEngine(21)
-    assert eng.fuse_upsample == 1
     assert eng._lazy_up == {"up4": 512, "up3": 256, "up2": 128, "up1": 64}          # name -> padded output channels of the reader
     assert "upc" not in eng._lazy_up                                                # up_conv reads it as its FIRST source
     assert LightweightUnetEngine(2)._lazy_up == {"up4": 192, "up3": 128, "up2": 64, "up1": 64}
     assert not UltraLightUnetEngine(2, variant="ultralight_large")._lazy_up
-    monkeypatch.setenv("B2U_FUSE_UPSAMPLE", "0")
-    assert ResNet50UnetEngine(21).fuse_upsample == 0 and VGGUnetEngine(21).fuse_upsample == 0
-    monkeypatch.setenv("B2U_FUSE_UPSAMPLE", "2")
-    assert VGGUnetEngine(21).fuse_upsample == 2
-    monkeypatch.delenv("B2U_FUSE_UPSAMPLE")
+    # the rule: fuse where the decoder conv has >= 128 output channels
     v = VGGUnetEngine(21)
-    assert v.fuse_upsample == 1 and v.relu_bits and v.bias_from_dgrad and v.wgrad_stream and not v.bias_in_wgrad_rest
-    # the default rule: fuse where the decoder conv has >= 128 output channels
-    assert [c1.cout_p >= 128 for c1, _ in v.dec] == [True, True, True, False]
+    assert [v.fuse_upsample(c1.cout_p) for c1, _ in v.dec] == [True, True, True, False]
+    assert [eng.fuse_upsample(c) for c in eng._lazy_up.values()] == [True, True, True, False]
 
 
 def test_conv_tile_count_helper(b2u):

@@ -281,7 +281,7 @@ def test_conv_wgrad_at_scale(b2u, cuda_device, N, H, W, Cin, Cout, taps):
     ref_db, A_db = dz.double().sum((0, 1, 2)), dz.double().abs().sum((0, 1, 2))
     tag = f"{N}x{H}x{W} {Cin}->{Cout} t{taps}"
     swapped_shape = Cout == 64 and taps == 9
-    runs = [(0, True), (1, True), (0, False)] + ([(2, False), (2, True)] if swapped_shape else [])      # (flags, want_db)
+    runs = [(0, True), (0, False)] + ([(2, False), (2, True)] if swapped_shape else [])      # (flags, want_db)
     for flags, want_db in runs:
         swapped = swapped_shape and not flags & 2
         splits, units = wgrad_plan(N, H, W, Cin, Cout, taps, sms, swapped)

@@ -82,10 +82,9 @@ def test_conv_fprop_dgrad_wgrad(b2u, cuda_device, N, H, W, C0, C1, Cout, taps, r
         assert torch.equal(d0s.view(torch.int16), d0.view(torch.int16))
         assert rel(ops.bias_from_stats(st, rows, C0), nchw(d0).double().sum((0, 2, 3))) <= 1e-5
     ref_dw = torch.nn.grad.conv2d_weight(xr, w.shape, dzr, padding=k // 2)
-    for flags in (0, 1):          # merged N=192 vertical taps and the three-instruction variant
-        dw, db = ops.conv_wgrad(x0, dzb, taps=taps, x1=x1, flags=flags, want_db=True)
-        assert rel(dw, ref_dw) <= 1e-4
-        assert rel(db, dzr.sum((0, 2, 3))) <= 1e-4      # bias gradient fused into the wgrad kernel
+    dw, db = ops.conv_wgrad(x0, dzb, taps=taps, x1=x1, want_db=True)
+    assert rel(dw, ref_dw) <= 1e-4
+    assert rel(db, dzr.sum((0, 2, 3))) <= 1e-4      # bias gradient fused into the wgrad kernel
     # without db: Cout = 64 3x3 layers take the swapped-role kernel (x as the M operand, three shifted dz boxes as N);
     # flags bit 1 forces the generic kernel
     assert rel(ops.conv_wgrad(x0, dzb, taps=taps, x1=x1), ref_dw) <= 1e-4
@@ -641,7 +640,7 @@ def test_padded_channel_convs(b2u, cuda_device):
     run on the tensor-core kernels with zero-padded operands: pack_weights_multi pads, the conv sees pad64 channels."""
     import struct
     from unet_pytorch_b200 import ops
-    from unet_pytorch_b200.graph import pad64
+    from unet_pytorch_b200._engine_base import pad64
     dev = cuda_device
     g = torch.Generator().manual_seed(5)
     for (cout, c0, c1, taps) in ((22, 3, 0, 1), (44, 22, 0, 1), (176, 352, 176, 1), (88, 44, 0, 9), (352, 704, 352, 1)):

@@ -210,32 +210,35 @@ def test_eval_forward_is_deterministic_and_repeatable(b2u, cuda_device):
 
 
 @pytest.mark.parametrize("model,C", [("unet_vgg", 21), ("traditional", 4), ("unet_resnet50", 21)])
-def test_fused_upsample_equals_separate_pass(b2u, cuda_device, model, C):
+def test_fused_upsample_equals_separate_pass(b2u, cuda_device, monkeypatch, model, C):
     """nets/unet.py:16-18 in one kernel: the decoder conv that interpolates its low-resolution source itself
-    (engine.fuse_upsample: 1 = the stages where it pays, the default; 2 = every stage) gives BIT-identical logits, loss and
-    gradients to the build that runs b2u_upsample2x_fwd as a separate pass (0); a fused stage needs no upsample launch, and in
-    inference it allocates no up-sampled tensor."""
+    (EngineBase.fuse_upsample: 1 = the stages where it pays, the default; patched to 2 = every stage) gives BIT-identical
+    logits, loss and gradients to the separate b2u_upsample2x_fwd pass (patched to 0 = no stage); a fused stage needs no
+    upsample launch, and in inference it allocates no up-sampled tensor."""
+    from unet_pytorch_b200._engine_base import EngineBase
     dev = cuda_device
     imgs, pngs = O.make_inputs(2, C, 96, 64, seed=5)
     runs = {}
-    for fuse in (2, 1, 0):
-        tr = b2u.UnetTrainer(model=model, num_classes=C, device=dev, lr=0.0) if model != "unet_vgg" else \
-            b2u.UnetTrainer(num_classes=C, device=dev, lr=0.0, state_dict=O.make_params(C, seed=11))
-        tr.engine.fuse_upsample = fuse
-        # inference first, on the initial state (a training step of the BatchNorm nets moves the running statistics by the
-        # summation order of the per-tile sums, which differs between the two kernels' tilings)
-        logits = tr.engine.forward(imgs.to(dev), tr.tensors, save=False, training=False).clone()
-        b2u.ops.lib().b2u_reset_launch_count()
-        out = tr.train_step(imgs.to(dev), pngs.to(dev)).cpu()
-        torch.cuda.synchronize()
-        launches = b2u.ops.lib().b2u_launch_count()
-        runs[fuse] = (out, {k: v.clone() for k, v in tr.grads.items()}, logits, launches)
-        if fuse == 2:
-            tr.engine.release()
-            tr.engine.forward(imgs.to(dev), tr.tensors, save=False, training=False)
-            lazy = getattr(tr.engine, "_lazy_up", None)       # GraphEngine: the up-sampled tensors read by decoder convs
-            ups = [k for k in tr.engine._bufs if (k in lazy if lazy is not None else re.fullmatch(r"up\d+", k))]
-            assert not ups, "inference must not materialise the up-sampled tensors"
+    for fuse, rule in ((2, lambda self, cout_p: True), (1, None), (0, lambda self, cout_p: False)):
+        with monkeypatch.context() as m:
+            if rule is not None:
+                m.setattr(EngineBase, "fuse_upsample", rule)
+            tr = b2u.UnetTrainer(model=model, num_classes=C, device=dev, lr=0.0) if model != "unet_vgg" else \
+                b2u.UnetTrainer(num_classes=C, device=dev, lr=0.0, state_dict=O.make_params(C, seed=11))
+            # inference first, on the initial state (a training step of the BatchNorm nets moves the running statistics by the
+            # summation order of the per-tile sums, which differs between the two kernels' tilings)
+            logits = tr.engine.forward(imgs.to(dev), tr.tensors, save=False, training=False).clone()
+            b2u.ops.lib().b2u_reset_launch_count()
+            out = tr.train_step(imgs.to(dev), pngs.to(dev)).cpu()
+            torch.cuda.synchronize()
+            launches = b2u.ops.lib().b2u_launch_count()
+            runs[fuse] = (out, {k: v.clone() for k, v in tr.grads.items()}, logits, launches)
+            if fuse == 2:
+                tr.engine.release()
+                tr.engine.forward(imgs.to(dev), tr.tensors, save=False, training=False)
+                lazy = getattr(tr.engine, "_lazy_up", None)       # GraphEngine: the up-sampled tensors read by decoder convs
+                ups = [k for k in tr.engine._bufs if (k in lazy if lazy is not None else re.fullmatch(r"up\d+", k))]
+                assert not ups, "inference must not materialise the up-sampled tensors"
     for fuse in (2, 1):
         assert torch.equal(runs[fuse][2], runs[0][2])            # inference logits: bit-identical for every family
         if model == "traditional":
@@ -253,20 +256,25 @@ def test_fused_upsample_equals_separate_pass(b2u, cuda_device, model, C):
     assert runs[0][3] - runs[1][3] == wide
 
 
-def test_relu_bit_masks_and_dgrad_bias_sums_change_nothing(b2u, cuda_device):
-    """Three round-2 traffic savers of the plain conv + ReLU nets -- ReLU backward from bit masks (engine.relu_bits), bias
-    gradients from the producing data gradient's column sums (engine.bias_from_dgrad), weight gradients on a second stream
-    (engine.wgrad_stream) -- against the straightforward order: the loss and the data path are bit-identical, bias gradients agree
-    to fp32 summation order."""
+def test_relu_bit_masks_and_dgrad_bias_sums_change_nothing(b2u, cuda_device, monkeypatch):
+    """Three round-2 traffic savers of the plain conv + ReLU nets -- ReLU backward from bit masks (UNetEngine.relu_bit_masks),
+    bias gradients from the producing data gradient's column sums (UNetEngine.bias_from_dgrad), weight gradients on a second
+    stream (single-stream while ops.timing_active()) -- against the straightforward order: the loss and the data path are
+    bit-identical, bias gradients agree to fp32 summation order."""
+    from unet_pytorch_b200.engine import UNetEngine
     dev, C = cuda_device, 21
     imgs, pngs = O.make_inputs(2, C, 96, 64, seed=8)
     runs = []
     for on in (True, False):
-        tr = b2u.UnetTrainer(num_classes=C, device=dev, lr=0.0, state_dict=O.make_params(C, seed=11))
-        tr.engine.relu_bits = tr.engine.bias_from_dgrad = tr.engine.wgrad_stream = on
-        out = tr.train_step(imgs.to(dev), pngs.to(dev)).cpu()
-        torch.cuda.synchronize()
-        runs.append((out, {k: v.clone() for k, v in tr.grads.items()}))
+        with monkeypatch.context() as m:
+            if not on:
+                m.setattr(UNetEngine, "relu_bit_masks", lambda self, save: False)
+                m.setattr(UNetEngine, "bias_from_dgrad", lambda self, c: False)
+                m.setattr(b2u.ops, "timing_active", lambda: True)
+            tr = b2u.UnetTrainer(num_classes=C, device=dev, lr=0.0, state_dict=O.make_params(C, seed=11))
+            out = tr.train_step(imgs.to(dev), pngs.to(dev)).cpu()
+            torch.cuda.synchronize()
+            runs.append((out, {k: v.clone() for k, v in tr.grads.items()}))
     assert torch.equal(runs[0][0], runs[1][0])
     for k, g in runs[1][1].items():
         if k.endswith(".weight"):

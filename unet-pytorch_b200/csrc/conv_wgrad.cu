@@ -31,7 +31,6 @@ struct WgradParams {
   int C0, C1, Cout;
   int tiles_w, tiles_h, kblocks;   // kblocks = N * tiles_h * tiles_w
   int num_mblk, num_cblk, splits, units;
-  int merged;                      // 1: N=192 merged vertical taps; 0: three N=64 instructions
   float* partial;                  // [splits][Cout][taps][C0+C1]
   float* bias_partial;             // [splits][Cout] or null: db = column sums of dz (warp 6 sums the staged dz tiles)
 };
@@ -60,7 +59,6 @@ conv_wgrad_kernel(const __grid_constant__ CUtensorMap tmX0, const __grid_constan
                   const __grid_constant__ CUtensorMap tmDZ, const WgradParams p) {
   using Cfg = WgCfg<TAPS, STAGES>;
   constexpr int S_TAPS = TAPS == 9 ? 3 : 1;
-  constexpr int R_TAPS = TAPS == 9 ? 3 : 1;
 
   extern __shared__ uint8_t smem_raw[];
   const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
@@ -140,13 +138,11 @@ conv_wgrad_kernel(const __grid_constant__ CUtensorMap tmX0, const __grid_constan
   } else if (warp == 1) {
     if (lane == 0) {
       // A = dz (M x K, MN-major), B = x (N x K, MN-major)
-      constexpr uint32_t idesc_merged = umma_idesc_bf16(128, Cfg::kAccN, 1, 1);
-      constexpr uint32_t idesc_single = umma_idesc_bf16(128, 64, 1, 1);
+      constexpr uint32_t idesc = umma_idesc_bf16(128, Cfg::kAccN, 1, 1);
       const uint32_t lbo_a = two_halves ? Cfg::kDzHalf : 0u;   // Cout == 64: rows 64..127 alias rows 0..63
       // descriptor templates: per MMA only the 14-bit start-address field moves (+128 = one 16-pixel image row)
       const uint64_t a_desc0 = umma_smem_desc(smem_base, lbo_a, 1024, 2u);
       const uint64_t b_desc0 = umma_smem_desc(smem_base + Cfg::kDzBytes, 2048, 1024, 2u);
-      const bool merged = TAPS == 1 || p.merged;
       int st = 0, as = 0; uint32_t ph = 0, pacc = 0;
       for (int unit = blockIdx.x; unit < p.units; unit += gridDim.x) {
         int split, mblk, cblk, s, k0, k1;
@@ -161,19 +157,9 @@ conv_wgrad_kernel(const __grid_constant__ CUtensorMap tmX0, const __grid_constan
           tc_fence_after();
           const uint64_t a_st = a_desc0 + static_cast<uint64_t>((st * Cfg::kStage) >> 4);
           const uint64_t b_st = b_desc0 + static_cast<uint64_t>((st * Cfg::kStage) >> 4);
-          if (merged) {
 #pragma unroll
-            for (int j = 0; j < kHb; ++j)
-              tc_mma_bf16(d_tmem, a_st + j * 128, b_st + j * 128, idesc_merged, j == 0 ? acc : 1u);
-          } else {
-#pragma unroll
-            for (int j = 0; j < kHb; ++j) {
-              const uint32_t accj = j == 0 ? acc : 1u;
-#pragma unroll
-              for (int r = 0; r < R_TAPS; ++r)
-                tc_mma_bf16(d_tmem + r * 64, a_st + j * 128, b_st + (j + r) * 128, idesc_single, accj);
-            }
-          }
+          for (int j = 0; j < kHb; ++j)
+            tc_mma_bf16(d_tmem, a_st + j * 128, b_st + j * 128, idesc, j == 0 ? acc : 1u);
           acc = 1;
           tc_commit(empty(st));
           if (++st == STAGES) { st = 0; ph ^= 1u; }
@@ -600,7 +586,7 @@ static WgradPlan plan_wgrad(int N, int H, int W, int Cin_tot, int Cout, int taps
 
 template <int TAPS, int STAGES>
 static int launch_wgrad_cfg(const void* x0, int C0, const void* x1, int C1, const void* dz, int Cout, float* partial,
-                            float* bias_partial, const WgradPlan& pl, int N, int H, int W, int merged, cudaStream_t st) {
+                            float* bias_partial, const WgradPlan& pl, int N, int H, int W, cudaStream_t st) {
   using Cfg = WgCfg<TAPS, STAGES>;
   auto kern = conv_wgrad_kernel<TAPS, STAGES>;
   static bool attr_done[64] = {false};
@@ -626,7 +612,6 @@ static int launch_wgrad_cfg(const void* x0, int C0, const void* x1, int C1, cons
   p.N = N; p.H = H; p.W = W; p.C0 = C0; p.C1 = C1; p.Cout = Cout;
   p.tiles_w = (W + kWb - 1) / kWb; p.tiles_h = (H + kHb - 1) / kHb; p.kblocks = pl.kblocks;
   p.num_mblk = pl.num_mblk; p.num_cblk = pl.num_cblk; p.splits = pl.splits; p.units = pl.units;
-  p.merged = merged;
   p.partial = partial;
   p.bias_partial = bias_partial;
   const int grid = pl.units < num_sms() ? pl.units : num_sms();
@@ -702,14 +687,14 @@ size_t b2u_conv_wgrad_workspace(int N, int H, int W, int Cin_tot, int Cout, int 
 // computed in the same pass as column sums of dz.
 // first_cin > 0: x0 is the first layer's im2col tensor [N,H,W,64] (taps must be 1, C0 == 64, C1 == 0);
 //                dw then is [Cout][first_cin][3][3].
-// flags bit0: use three N=64 instructions per image row instead of the merged N=192 one; bit1: never use the
-// swapped-role Cout = 64 kernel.
+// flags bit1: never use the swapped-role Cout = 64 kernel; every other bit is rejected.
 int b2u_conv_wgrad(const void* x0, int C0, const void* x1, int C1, const void* dz, int Cout, float* dw, float* db, void* ws,
                    size_t ws_bytes, int N, int H, int W, int taps, int first_cin, int flags, void* stream) {
   using namespace b2u;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (!x1) C1 = 0;
   const int ctot = C0 + C1;
+  if (flags & ~2) return set_error(B2U_ERR_ARG, "wgrad: unknown flags 0x%x (only bit 1 is defined)", flags);
   if (N <= 0 || H <= 0 || W <= 0) return set_error(B2U_ERR_SHAPE, "wgrad: empty tensor");
   if (taps != 9 && taps != 1) return set_error(B2U_ERR_SHAPE, "wgrad: taps must be 9 or 1");
   if (C0 % 64 != 0 || C1 % 64 != 0 || ctot <= 0)
@@ -742,11 +727,10 @@ int b2u_conv_wgrad(const void* x0, int C0, const void* x1, int C1, const void* d
   if (ws == nullptr || ws_bytes < pl.ws_bytes)
     return set_error(B2U_ERR_ARG, "wgrad: workspace %zu bytes < required %zu", ws_bytes, pl.ws_bytes);
   int rc;
-  const int merged = (flags & 1) ? 0 : 1;
   float* wpart = static_cast<float*>(ws);
   float* bpart = db ? wpart + static_cast<size_t>(pl.splits) * Cout * taps * ctot : nullptr;
-  if (taps == 9) rc = launch_wgrad_cfg<9, 4>(x0, C0, x1, C1, dz, Cout, wpart, bpart, pl, N, H, W, merged, st);
-  else           rc = launch_wgrad_cfg<1, 4>(x0, C0, x1, C1, dz, Cout, wpart, bpart, pl, N, H, W, merged, st);
+  if (taps == 9) rc = launch_wgrad_cfg<9, 4>(x0, C0, x1, C1, dz, Cout, wpart, bpart, pl, N, H, W, st);
+  else           rc = launch_wgrad_cfg<1, 4>(x0, C0, x1, C1, dz, Cout, wpart, bpart, pl, N, H, W, st);
   if (rc) return rc;
   if (db) {
     wgrad_bias_reduce_kernel<<<(Cout + 127) / 128, 128, 0, st>>>(bpart, db, pl.splits, Cout);
@@ -779,7 +763,7 @@ int b2u_conv_wgrad_im2col(const void* x0, int Kpad, const void* dz, int Cout, fl
   if (Cout % 64 != 0) return set_error(B2U_ERR_SHAPE, "wgrad_im2col: Cout %d must be a multiple of 64", Cout);
   const WgradPlan pl = plan_wgrad(N, H, W, Kpad, Cout, 1);
   if (ws == nullptr || ws_bytes < pl.ws_bytes) return set_error(B2U_ERR_ARG, "wgrad_im2col: workspace too small");
-  int rc = launch_wgrad_cfg<1, 4>(x0, Kpad, nullptr, 0, dz, Cout, static_cast<float*>(ws), nullptr, pl, N, H, W, 1, st);
+  int rc = launch_wgrad_cfg<1, 4>(x0, Kpad, nullptr, 0, dz, Cout, static_cast<float*>(ws), nullptr, pl, N, H, W, st);
   if (rc) return rc;
   const int total = Cout * cin * taps;
   wgrad_reduce_kernel<<<(total + 63) / 64, 256, 0, st>>>(static_cast<const float*>(ws), dw, pl.splits, Cout, taps, Kpad, cin, 1);

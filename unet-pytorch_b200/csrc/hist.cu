@@ -665,11 +665,6 @@ static int hist_lanes_warps(int n) {       // warps per block that fit 200 KB of
   int w = static_cast<int>((200 * 1024) / per_warp);
   return w > 12 ? 12 : w;
 }
-static bool hist_legacy() {                 // B2U_HIST_LEGACY=1: the round-1 kernels (A/B measurements)
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("B2U_HIST_LEGACY"); v = (e && e[0] == '1') ? 1 : 0; }
-  return v == 1;
-}
 static int hist_set_attr(const void* fn) {
   cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, 204 * 1024);
   return e == cudaSuccess ? 0 : set_error(B2U_ERR_CUDA, "fast_hist: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
@@ -805,7 +800,7 @@ int b2u_fast_hist(const void* a, const void* b, long long len, int n, int dtype,
       };
       // few bins (n*n + 1 <= 32): successive pixels keep hitting the same counter, a shared-memory round trip each; the
       // register-counter kernel below is 3-4x faster there (measured: 2.1 vs 0.56 TB/s at n = 2)
-      if (aligned && n * n + 1 > kVoteMaxBins && hist_lanes_warps(n) >= 4 && !hist_legacy()) {
+      if (aligned && n * n + 1 > kVoteMaxBins && hist_lanes_warps(n) >= 4) {
         int rc = launch_hist_lanes(nullptr, 1, 0, pa, pb, l, n, hist, st);
         if (rc) return rc;
         continue;

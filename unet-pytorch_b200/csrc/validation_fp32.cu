@@ -922,7 +922,8 @@ int b2u_conv_dgrad(const void* dz, int Cz, const void* wd, void* dx0, int C0, vo
 size_t b2u_conv_wgrad_workspace(int, int, int, int, int, int) { return 16; }
 
 int b2u_conv_wgrad(const void* x0, int C0, const void* x1, int C1, const void* dz, int Cout, float* dw, float* db, void* /*ws*/,
-                   size_t /*ws_bytes*/, int N, int H, int W, int taps, int first_cin, int /*flags*/, void* stream) {
+                   size_t /*ws_bytes*/, int N, int H, int W, int taps, int first_cin, int flags, void* stream) {
+  if (flags & ~2) return set_error(B2U_ERR_ARG, "wgrad: unknown flags 0x%x (only bit 1 is defined)", flags);
   if (N <= 0 || H <= 0 || W <= 0) return set_error(B2U_ERR_SHAPE, "wgrad: empty tensor");
   if (taps != 9 && taps != 1) return set_error(B2U_ERR_SHAPE, "wgrad: taps must be 9 or 1");
   const int c1 = x1 ? C1 : 0;

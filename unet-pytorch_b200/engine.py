@@ -19,13 +19,11 @@ Gradients are written straight into caller-provided fp32 OIHW tensors (normally 
 trainer can start that bucket's all-reduce while the remaining dgrad/wgrad kernels still run.
 """
 import contextlib
-import functools
-import os
-import struct
 
 import torch
 
 from . import ops
+from ._engine_base import EngineBase, pad64
 
 # (features index, Cin, Cout) and 'M' for nn.MaxPool2d(2,2): cfgs['D'] of nets/vgg.py:62-64 without the last pool
 VGG16_CFG = [(0, 3, 64), (2, 64, 64), "M", (5, 64, 128), (7, 128, 128), "M", (10, 128, 256), (12, 256, 256),
@@ -34,10 +32,6 @@ VGG16_CFG = [(0, 3, 64), (2, 64, 64), "M", (5, 64, 128), (7, 128, 128), "M", (10
 # (module name, C_skip, C_up, C_out): in_filters [192, 384, 768, 1024], out_filters [64, 128, 256, 512] (nets/unet.py:28-45)
 DECODER_CFG = [("up_concat4", 512, 512, 512), ("up_concat3", 256, 512, 256), ("up_concat2", 128, 256, 128),
                ("up_concat1", 64, 128, 64)]
-
-
-def pad64(c):
-    return (c + 63) // 64 * 64
 
 
 def vgg_unet_param_shapes(num_classes, in_channels=3):
@@ -117,100 +111,38 @@ def traditional_unet_config(num_classes, in_channels=3):
     return UNetConfig(enc, dec, ("outc", 32), num_classes, in_channels)
 
 
-class UNetEngine:
+class UNetEngine(EngineBase):
     def __init__(self, cfg, device=None):
         if cfg.in_channels * 9 > 64:
             raise ValueError("in_channels must be <= 7 (first-layer im2col is 64 columns wide)")
         if not 1 <= cfg.num_classes <= 255:
             raise ValueError("num_classes must be in [1, 255]")
+        super().__init__(device)
         self.cfg = cfg
         self.num_classes = cfg.num_classes
         self.in_channels = cfg.in_channels
-        self.device = device
         self.enc, self.dec, self.bn = cfg.enc, cfg.dec, cfg.bn
         self.head_name, self.head_cin = cfg.head
         self.convs = [c for b in self.enc for c in b] + [c for pair in self.dec for c in pair]
-        self.eps, self.momentum = 1e-5, 0.1                 # nn.BatchNorm2d defaults (the reference never changes them)
-        # The wgrad kernel can produce db in the same pass (an N=16 MMA against a ones tile); measured on B200 it costs
-        # more than the separate HBM-bound column-sum kernel (work units with the extra MMAs become the stragglers of
-        # the static schedule: +40 % wgrad time vs +1.2 ms for bias_grad), so it is off by default.
-        # BatchNorm statistics from the conv epilogue (one pass over z less); only where the reduction is long enough for the
-        # extra epilogue work to hide behind the main loop (scripts/ab_fuse_bnstats.py)
-        self.fuse_bn_stats = True
-        self.center_pre_bn = os.environ.get("B2U_CENTER_PRE_BN", "1") == "1"      # pre-BatchNorm tensors stored centred on the running mean
-        self.sync_bn_group = None        # torch.distributed group: BatchNorm statistics over all ranks (SyncBatchNorm)
-        self.bn_stats_min_k = 1024
-        self.bn_stats_min_cout = 256
-        # db from the wgrad kernel's bias warps (3x3 layers) instead of a separate pass over dz: an A/B on one box
-        # (scripts/ab_fuse_bias.py: 23.2-23.9 vs 23.4-23.5 ms/step) shows no gain, so the separate pass stays the default
-        self.fuse_bias_grad = False
-        # bilinear 2x up-sampling + concat folded into the decoder conv's operand load (b2u_decoder_conv_fprop).  Measured at
-        # the four unetUp shapes of the headline step (scripts/ab_fused_upsample.py, profiles/r2_fused_upsample.json): with
-        # N tiles of 128 / 256 output channels the fused conv beats upsample + conv (0.42 / 0.65 / 0.70 ms against 0.42 / 0.67 /
-        # 0.77); with the N = 64 tile (64+128 -> 64 at 512 x 512) the five interpolation warps cannot keep up with a main loop
-        # that short (1.32 against 1.07 ms), so that stage keeps the separate pass.  B2U_FUSE_UPSAMPLE: 0 = never,
-        # 1 = where it pays (default), 2 = every decoder stage (tests compare all three bit for bit).
-        self.fuse_upsample = int(os.environ.get("B2U_FUSE_UPSAMPLE", "1"))
-        # Bias gradients of the wide layers (Cout >= 128; the Cout = 64 ones get theirs from the swapped-role wgrad kernel) from
-        # the data-gradient launch that PRODUCES their dz: its epilogue leaves per-tile column sums of the masked gradient it
-        # stores (b2u_conv_dgrad_stats, the BatchNorm-statistics machinery) and b2u_bias_from_stats folds them, instead of
-        # b2u_bias_grad re-reading dz from HBM (1.2 GB per headline step).  Those dgrads have K >= 1152, long enough to hide the
-        # extra epilogue work.  Layers whose dz comes from the pool / upsample adjoints keep the separate pass.
-        self.bias_from_dgrad = os.environ.get("B2U_BIAS_FROM_DGRAD", "1") == "1"
-        self.bias_in_wgrad_rest = os.environ.get("B2U_BIAS_WGRAD_REST", "0") == "1"
-        # ReLU backward from bit masks (plain conv + ReLU nets, training forward): every conv epilogue also writes (y > 0) as one
-        # bit per channel ([N,H,W,C/64] 64-bit words, 1/16 of the bytes of y) and the masked data gradients / the head backward
-        # read those 8 bytes per pixel and block instead of 128 bytes of y -- 2.8 GB less HBM traffic per headline step, and the
-        # HBM-bound 64-channel data gradients at 512 x 512 then tile like unmasked launches (four stacked M tiles, no cp.async
-        # mask stream).  Same-call A/B: 22.13 / 22.15 ms per step without, 21.77 / 21.73 with, results bit-identical
-        # (test_relu_bit_masks*).  B2U_RELU_BITS=0 restores the bf16 masks (the pool / upsample adjoints always read y).
-        self.relu_bits = os.environ.get("B2U_RELU_BITS", "1") == "1"
-        # Weight/bias gradients on a second stream (plain conv+ReLU nets): wgrad_L depends only on dz_L and the saved
-        # activation, not on the dgrad chain, so its launches are queued on a side stream behind an event and the
-        # HBM-bound glue of the main chain (pool / upsample adjoints, column-sum folds) shares the SMs with tensor-core-bound
-        # kernels of the other stream instead of running alone.  Same-box A/B (bench.py --kernels-only, 12 steps, twice each,
-        # round 2 final build): 21.79 / 21.67 ms per step with it, 22.05 / 21.87 without (-1 %; round 1 measured -0.9 %).
-        # Per-launch CUDA-event times are not a kernel's own duration while two streams overlap, so the roofline pass of
-        # bench.py (ops.KernelTimer) runs single-stream: backward() checks ops.timing_active().  B2U_WGRAD_STREAM=0 turns it off.
-        self.wgrad_stream = os.environ.get("B2U_WGRAD_STREAM", "1") == "1"
         self._side = None
-        self._pack_key = self._pack_versions = self._pack_table = None
-        self._pack_total = 0
-        self._bufs = {}
-        self.saved = None
-        self._ws = {}
 
-    # ------------------------------------------------------------------ buffers
-    def _buf(self, key, shape, dtype=None, zero=False):
-        dtype = ops.act_dtype() if dtype is None else dtype      # bf16; fp32 under the fp32 validation build
-        t = self._bufs.get(key)
-        if t is None or tuple(t.shape) != tuple(shape) or t.dtype != dtype:
-            t = (torch.zeros if zero else torch.empty)(shape, dtype=dtype, device=self.device)
-            self._bufs[key] = t
-        return t
+    # ------------------------------------------------------------------ policies of the plain conv + ReLU nets
+    def relu_bit_masks(self, save):
+        """ReLU backward from bit masks (training forward, bf16): every conv epilogue also writes (y > 0) as one bit per
+        channel ([N,H,W,C/64] 64-bit words, 1/16 of the bytes of y) and the masked data gradients / the head backward read
+        those 8 bytes per pixel and block instead of 128 bytes of y -- 2.8 GB less HBM traffic per headline step, and the
+        HBM-bound 64-channel data gradients at 512 x 512 then tile like unmasked launches (four stacked M tiles, no cp.async
+        mask stream).  Same-call A/B: 22.13 / 22.15 ms per step without, 21.77 / 21.73 with, results bit-identical
+        (test_relu_bit_masks*).  The pool / upsample adjoints always read y."""
+        return save and ops.act_dtype() == torch.bfloat16
 
-    def _workspace(self, key, nbytes):
-        t = self._ws.get(key)
-        if t is None or t.numel() < nbytes:
-            t = torch.empty(max(int(nbytes), 16), dtype=torch.uint8, device=self.device)
-            self._ws[key] = t
-        return t
-
-    def release(self):
-        self._bufs.clear()
-        self._ws.clear()
-        self.saved = None
-
-    def _padded_vec(self, key, vec, n, fill=0.0):
-        """fp32 per-channel vector padded to n entries (persistent buffer, real part refreshed from `vec`)."""
-        if vec.numel() == n:
-            return vec
-        t = self._bufs.get(key)
-        if t is None or t.numel() != n:
-            t = torch.full((n,), fill, dtype=torch.float32, device=self.device)
-            self._bufs[key] = t
-        t[:vec.numel()].copy_(vec)
-        return t
+    def bias_from_dgrad(self, c):
+        """Bias gradient of a wide plain layer (one whose db does not come from the wgrad kernel, see fused_db) from the
+        data-gradient launch that PRODUCES its dz: that epilogue leaves per-tile column sums of the masked gradient it stores
+        (b2u_conv_dgrad_stats, the BatchNorm-statistics machinery) and b2u_bias_from_stats folds them, instead of
+        b2u_bias_grad re-reading dz from HBM (1.2 GB per headline step).  Those dgrads have K >= 1152, long enough to hide the
+        extra epilogue work.  Layers whose dz comes from the pool / upsample adjoints keep the separate pass."""
+        return not self.bn and ops.act_dtype() == torch.bfloat16 and not c.padded and not c.first and not self.fused_db(c.cout_p)
 
     # ------------------------------------------------------------------ weights
     def pack(self, params, need_dgrad=True):
@@ -218,33 +150,26 @@ class UNetEngine:
         driven by a device-resident table of (weight, operand) pointers that is rebuilt only if a pointer moved."""
         key = tuple(params[c.name + ".weight"].data_ptr() for c in self.convs) + (need_dgrad,)
         versions = tuple(params[c.name + ".weight"]._version for c in self.convs)
-        if self._pack_key == key and self._pack_versions == versions and self._pack_versions is not None:
+        if self._pack_key == key and self._pack_versions == versions:
             return
         dev = params[self.convs[0].name + ".weight"].device
         if self._pack_key != key:
-            blob, start = b"", 0
+            layers = []
             for c in self.convs:
-                w = params[c.name + ".weight"]
                 ctot_p = c.c0_p + c.c1_p
                 if c.first:
                     if c.wf is None:
                         c.wf = torch.zeros((c.cout_p, 64), dtype=ops.act_dtype(), device=dev)
-                    count = (c.cout + 31) // 32                      # work blocks of this layer
                 else:
                     if c.wf is None:
                         c.wf = torch.zeros((c.cout_p, 9 * ctot_p), dtype=ops.act_dtype(), device=dev)
                     if need_dgrad and c.wd is None:
                         c.wd = torch.zeros((ctot_p, 9 * c.cout_p), dtype=ops.act_dtype(), device=dev)
-                    count = ((c.cout + 31) // 32) * ((c.cin + 31) // 32)
-                wd_ptr = c.wd.data_ptr() if (need_dgrad and not c.first) else 0
-                blob += struct.pack("<QQQqiiiiiiii", w.data_ptr(), c.wf.data_ptr(), wd_ptr, start, c.cout, c.cin,
-                                    1 if c.first else 9, 1 if c.first else 0, c.c0, c.c0_p, ctot_p, c.cout_p)
-                start += count
-            self._pack_table = torch.frombuffer(bytearray(blob), dtype=torch.uint8).to(dev)
-            self._pack_total = start
+                layers.append((params[c.name + ".weight"], c.wf, c.wd if need_dgrad else None, c.cout, c.cin,
+                               1 if c.first else 9, c.first, c.c0, c.c0_p, ctot_p, c.cout_p))
+            self._set_pack_table(layers, dev)
             self._pack_key = key
-        ops.check(ops.lib().b2u_pack_weights_multi(self._pack_table.data_ptr(), len(self.convs), self._pack_total,
-                                                   ops.stream_ptr()))
+        self._launch_pack()
         self._pack_versions = versions
 
     def param_shapes(self):
@@ -284,16 +209,12 @@ class UNetEngine:
             out += [c.name + ".weight", c.name + ".bias"]
         return out
 
-    def invalidate_packed_weights(self):
-        """Call after writing parameters behind torch's back (raw-pointer optimizer kernels)."""
-        self._pack_versions = None
-
     # ------------------------------------------------------------------ one conv (+BN) + ReLU layer, forward
     def _layer_fwd(self, c, x0, params, A, training, x1=None, save=True, low=None, up_out=None):
         """low (instead of x1): the second source is upsample2x(low), interpolated inside the conv kernel
         (ops.decoder_conv_fprop); up_out then optionally receives the up-sampled tensor as a by-product."""
         n, h, w, _ = x0.shape
-        bias = self._padded_vec("b:" + c.name, params[c.name + ".bias"], c.cout_p)
+        bias = self._padded("b:" + c.name, params[c.name + ".bias"], (c.cout_p,))
         taps = 1 if c.first else 9
 
         def conv(bias_, relu, out, stats=None, scale=None):
@@ -305,7 +226,7 @@ class UNetEngine:
 
         if not c.bn:
             out = self._buf(c.name, (n, h, w, c.cout_p))
-            if save and self.relu_bits and ops.act_dtype() == torch.bfloat16:
+            if self.relu_bit_masks(save):
                 bits = self._buf("bits:" + c.name, (n, h, w, c.cout_p // 64), torch.int64)
                 ops.conv_fprop_relu_bits(x0, c.wf, bias, c.cout_p, bits, taps=taps, x1=x1, low=low, up_out=up_out, out=out)
                 A["bits:" + c.name] = bits
@@ -317,69 +238,23 @@ class UNetEngine:
             # pure inference: BatchNorm is an affine map with fixed statistics, folded into the conv epilogue
             # (y = relu(acc * s + b')): no z tensor, no BatchNorm pass.  An eval-mode forward that will be back-propagated
             # (model.eval() + loss.backward()) takes the unfused path below so the BatchNorm backward has z
-            gamma = self._padded_vec("g:" + c.bn, params[c.bn + ".weight"], c.cout_p, fill=1.0)
-            beta = self._padded_vec("bt:" + c.bn, params[c.bn + ".bias"], c.cout_p)
-            rmp = self._padded_vec("rm:" + c.bn, params[c.bn + ".running_mean"], c.cout_p)
-            rvp = self._padded_vec("rv:" + c.bn, params[c.bn + ".running_var"], c.cout_p, fill=1.0)
-            sc, bs = ops.bn_fold(gamma, beta, rmp, rvp, bias, self.eps, scale=self._buf("fs:" + c.bn, (c.cout_p,), torch.float32),
-                                 bias=self._buf("fb:" + c.bn, (c.cout_p,), torch.float32))
+            sc, bs = self._folded_bn(c.bn, params, bias, c.cout_p)
             out = self._buf(c.name, (n, h, w, c.cout_p))
             conv(bs, True, out, scale=sc)
             A[c.name] = out
             return out
         z = self._buf("z:" + c.name, (n, h, w, c.cout_p))
-        rm, rv = params[c.bn + ".running_mean"], params[c.bn + ".running_var"]
-        # Training: z is stored CENTRED on the running mean -- the shift rides in the conv bias (fp32, before the bf16
-        # rounding), BatchNorm is shift-invariant, and only the running-mean update adds it back.  A channel whose mean is large
-        # against its spread otherwise loses |mean|/std * 2^-9 of relative accuracy in bf16 (the dominant error site of the
-        # depthwise nets on warm weights, profiles/r2_precision_sites.txt); at initialisation the running mean is 0: no change.
-        centered = training and self.center_pre_bn and ops.act_dtype() == torch.bfloat16
+        centered = self.center_pre_bn(training)
         if centered:
-            rmp0 = self._padded_vec("rm:" + c.bn, rm, c.cout_p)
-            bias = torch.sub(bias, rmp0, out=self._buf("bc:" + c.name, (c.cout_p,), torch.float32))
-        # training: the conv epilogue also emits the BatchNorm statistics of z (per-tile sums), so BatchNorm skips its
-        # statistics pass over z
-        stats, rows = None, 0
+            rmp = self._padded("rm:" + c.bn, params[c.bn + ".running_mean"], (c.cout_p,))
+            bias = torch.sub(bias, rmp, out=self._buf("bc:" + c.name, (c.cout_p,), torch.float32))
+        stats = None
         kdim = taps * (x0.shape[3] + (x1.shape[3] if x1 is not None else 0) + (low.shape[3] if low is not None else 0))
-        if training and self.fuse_bn_stats and self.sync_bn_group is None and (kdim >= self.bn_stats_min_k or c.cout_p >= self.bn_stats_min_cout):
-            rows = ops.conv_stat_rows(n, h, w, c.cout_p, taps, bn=(1 << 18) if low is not None else 0)      # bit 18: the decoder conv's tiles
-            stats = self._workspace("bnstat", rows * 2 * c.cout_p * 4)[:rows * 2 * c.cout_p * 4].view(torch.float32)
-        conv(bias, False, z, stats=stats)
-        gamma = self._padded_vec("g:" + c.bn, params[c.bn + ".weight"], c.cout_p, fill=1.0)
-        beta = self._padded_vec("bt:" + c.bn, params[c.bn + ".bias"], c.cout_p)
+        if self.fuse_bn_stats(training, kdim, c.cout_p):
+            stats = self._bn_stats("bnstat", n, h, w, c.cout_p, taps, decoder=low is not None)
+        conv(bias, False, z, stats=stats[0] if stats else None)
         out = self._buf(c.name, (n, h, w, c.cout_p))
-        ws = self._workspace("bn", ops.lib().b2u_bn_workspace(c.cout_p))
-        if training and self.sync_bn_group is not None:
-            rmp = self._padded_vec("rm:" + c.bn, rm, c.cout_p)
-            rvp = self._padded_vec("rv:" + c.bn, rv, c.cout_p, fill=1.0)
-            _, mean, invstd = ops.bn_fwd_train_sync(z, gamma, beta, rmp, rvp, self.sync_bn_group, self.eps, self.momentum, True,
-                                                    out=out, ws=ws, centered=centered)
-            if c.cout_p != c.cout or rmp is not rm:
-                rm.copy_(rmp[:c.cout]); rv.copy_(rvp[:c.cout])
-            nbt = params.get(c.bn + ".num_batches_tracked")
-            if nbt is not None:
-                nbt.add_(1)
-            A["bn:" + c.name] = (z, mean, invstd, gamma, beta)
-        elif training:
-            if c.cout_p == c.cout:
-                _, mean, invstd = ops.bn_fwd_train(z, gamma, beta, rm, rv, self.eps, self.momentum, True, out=out, ws=ws,
-                                                   stats=stats, stat_rows=rows, centered=centered)
-            else:
-                rmp = self._padded_vec("rm:" + c.bn, rm, c.cout_p)
-                rvp = self._padded_vec("rv:" + c.bn, rv, c.cout_p, fill=1.0)
-                _, mean, invstd = ops.bn_fwd_train(z, gamma, beta, rmp, rvp, self.eps, self.momentum, True, out=out, ws=ws,
-                                                   stats=stats, stat_rows=rows, centered=centered)
-                rm.copy_(rmp[:c.cout])
-                rv.copy_(rvp[:c.cout])
-            nbt = params.get(c.bn + ".num_batches_tracked")
-            if nbt is not None:
-                nbt.add_(1)
-            A["bn:" + c.name] = (z, mean, invstd, gamma, beta)
-        else:
-            rmp = self._padded_vec("rm:" + c.bn, rm, c.cout_p)
-            rvp = self._padded_vec("rv:" + c.bn, rv, c.cout_p, fill=1.0)
-            ops.bn_fwd_eval(z, gamma, beta, rmp, rvp, self.eps, True, out=out, ws=ws)
-            A["bn:" + c.name] = (z, (rmp, rvp), None, gamma, beta)      # eval-mode backward: statistics are constants
+        A["bn:" + c.name] = (z,) + self._bn_fwd(c.bn, z, params, training, True, out, stats=stats, centered=centered)
         A[c.name] = out
         return out
 
@@ -424,7 +299,7 @@ class UNetEngine:
         for si, (c1, c2) in enumerate(self.dec):
             skip = feats[len(self.enc) - 2 - si]
             _, hl, wl, cl = low.shape
-            if self.fuse_upsample == 2 or (self.fuse_upsample == 1 and c1.cout_p >= 128):
+            if self.fuse_upsample(c1.cout_p):
                 # the decoder conv interpolates `low` inside its producer warps (nets/unet.py:16-18 in one kernel); the
                 # up-sampled tensor is written only when a backward pass will need it as the weight gradient's operand
                 # (the fp32 validation build always takes the buffer: it keeps the two steps apart)
@@ -450,11 +325,7 @@ class UNetEngine:
 
     def _head_weight(self, params):
         w = params[self.head_name + ".weight"].reshape(self.num_classes, self.head_cin)
-        if self.head_cin == 64:
-            return w
-        t = self._buf("head:w", (self.num_classes, 64), torch.float32, zero=True)
-        t[:, :self.head_cin].copy_(w)
-        return t
+        return self._padded("head:w", w, (self.num_classes, 64))
 
     # ------------------------------------------------------------------ backward
     def backward(self, dlogits, params, grads, trainable=None, on_grads_ready=None):
@@ -463,8 +334,15 @@ class UNetEngine:
         Returns nothing; the input image gets no gradient (the reference never asks for one)."""
         if self.saved is None:
             raise RuntimeError("backward() without a saved forward()")
+        # Weight/bias gradients on a second stream (plain conv+ReLU nets): wgrad_L depends only on dz_L and the saved
+        # activation, not on the dgrad chain, so its launches are queued on a side stream behind an event and the
+        # HBM-bound glue of the main chain (pool / upsample adjoints, column-sum folds) shares the SMs with tensor-core-bound
+        # kernels of the other stream instead of running alone.  Same-box A/B (bench.py --kernels-only, 12 steps, twice each,
+        # round 2 final build): 21.79 / 21.67 ms per step with it, 22.05 / 21.87 without (-1 %; round 1 measured -0.9 %).
+        # Per-launch CUDA-event times are not a kernel's own duration while two streams overlap, so the roofline pass of
+        # bench.py (ops.KernelTimer) runs single-stream.
         side = None
-        if self.wgrad_stream and not self.bn and dlogits.is_cuda and not ops.timing_active():
+        if not self.bn and dlogits.is_cuda and not ops.timing_active():
             if self._side is None or self._side.device != dlogits.device:
                 self._side = torch.cuda.Stream(device=dlogits.device)
             side = self._side
@@ -528,8 +406,7 @@ class UNetEngine:
             that would otherwise need a pass over dz.  The ReLU mask is `below`'s bit mask when the forward left one."""
             bits = A.get("bits:" + below.name) if mask is not None else None
             stats = None
-            if (self.bias_from_dgrad and not bn and ops.act_dtype() == torch.bfloat16 and want[below.name] and has(below.name + ".bias")
-                    and not below.padded and not below.first and below.cout_p >= 128 and not self.fuse_bias_grad):
+            if want[below.name] and has(below.name + ".bias") and self.bias_from_dgrad(below):
                 n_, h_, w_, _ = out0.shape
                 rows = ops.conv_dgrad_stat_rows(n_, h_, w_, C0, 9, masked=mask is not None and bits is None)
                 nbytes = rows * 2 * C0 * 4
@@ -545,17 +422,11 @@ class UNetEngine:
             masked).  Runs BN backward if any, wgrad, bias grad; returns dz (the conv's output gradient)."""
             dz = g
             if c.bn:
-                z, mean, invstd, gamma, beta = A["bn:" + c.name]
+                z, *saved = A["bn:" + c.name]
                 wn, bnn = c.bn + ".weight", c.bn + ".bias"
                 dgam = self._buf("dg:" + c.bn, (c.cout_p,), torch.float32)
                 dbet = self._buf("db:" + c.bn, (c.cout_p,), torch.float32)
-                if invstd is None:      # eval-mode forward: running statistics, mask from the saved output
-                    ops.bn_bwd_eval(g, A[c.name], z, gamma, beta, mean[0], mean[1], self.eps, relu=True, out=g, dgamma=dgam,
-                                    dbeta=dbet, ws=self._workspace("bn", ops.lib().b2u_bn_workspace(c.cout_p)))
-                else:
-                    bwd = ops.bn_bwd if self.sync_bn_group is None else functools.partial(ops.bn_bwd_sync, group=self.sync_bn_group)
-                    bwd(g, None, z, gamma, mean, invstd, relu=True, out=g, dgamma=dgam, dbeta=dbet, beta=beta,   # mask from z
-                        ws=self._workspace("bn", ops.lib().b2u_bn_workspace(c.cout_p)))
+                self._bn_bwd(g, A[c.name], z, saved, True, g, dgam, dbet)
                 if has(wn):
                     grads[wn].copy_(dgam[:c.cout])
                 if has(bnn):
@@ -570,11 +441,7 @@ class UNetEngine:
         def param_grads(c, x0, dz, x1):
             wn, bn_ = c.name + ".weight", c.name + ".bias"
             want_w, want_b = has(wn), has(bn_)
-            # Cout = 64: db is free in the swapped-role wgrad kernel.  bias_in_wgrad_rest: the wide layers whose dz comes from the
-            # pool / upsample adjoints (no producing dgrad to take column sums from) let the wgrad kernel's bias warps sum the dz
-            # tiles while they sit in shared memory, instead of a separate pass over dz
-            fuse_b = (want_w and want_b and not c.padded and not c.bn and not c.first
-                      and (self.fuse_bias_grad or c.cout_p == 64 or (self.bias_in_wgrad_rest and c.name not in db_stats)))
+            fuse_b = want_w and want_b and not c.padded and not c.bn and not c.first and self.fused_db(c.cout_p)
             taps = 1 if c.first else 9
             if want_w:
                 ctot_p = 64 if c.first else c.c0_p + c.c1_p

@@ -26,17 +26,10 @@ ReLU handling: a tensor produced by a conv with fused ReLU is marked `fused_relu
 applies the mask (y > 0) on the way (dgrad epilogue / upsample adjoint / head dgrad), so its gradient is always wrt
 the pre-activation.  BatchNorm outputs are plain: the bn instruction's own backward applies its ReLU mask.
 """
-import functools
-import os
-import struct
-
 import torch
 
 from . import ops
-
-
-def pad64(c):
-    return (c + 63) // 64 * 64
+from ._engine_base import EngineBase, pad64
 
 
 class _T:
@@ -288,15 +281,11 @@ ULU_VARIANTS = {
 }
 
 
-class GraphEngine:
+class GraphEngine(EngineBase):
     def __init__(self, program, convs, num_classes, device=None, first_trainable_prefix=None):
-        self.program, self.convs, self.num_classes, self.device = program, convs, num_classes, device
-        self.eps, self.momentum = 1e-5, 0.1
-        self._bufs, self._ws = {}, {}
+        super().__init__(device)
+        self.program, self.convs, self.num_classes = program, convs, num_classes
         self._packed = {}            # weight name -> (wf, wd)
-        self._pack_key = self._pack_versions = self._pack_table = None
-        self._pack_total = 0
-        self.saved = None
         self.has_stem = any(i["op"] == "stem" for i in program)
         self.in_channels = next((i["c"] for i in program if i["op"] == "input"), 3)      # the stem (ResNet) takes RGB
         self.pk = {i["w"]: i for i in program if i["op"] == "conv" and i.get("pk")}     # pixel-packed 1x1 convs
@@ -306,21 +295,6 @@ class GraphEngine:
         inputs = {i["out"]: i["c"] for i in program if i["op"] == "input"}
         self.image_convs = {i["w"]: inputs[i["x"]] for i in program if i["op"] == "conv" and i["x"] in inputs and 2 * inputs[i["x"]] <= 64}
         self.dropout_override = None
-        # db from the wgrad kernel's bias warps instead of a separate pass over dz: measured on one box (scripts/ab_fuse_bias.py)
-        # it does not change the step time (the extra smem reads slow the bias-owning work units), so it stays off
-        self.fuse_bias_grad = False
-        # BatchNorm statistics from the producing conv's epilogue (one pass over z less).  The extra epilogue work only hides
-        # behind the main loop when the reduction is long enough: measured (scripts/ab_fuse_bnstats.py) it gains 0.8 ms on
-        # Unet-ResNet50 but loses 0.7-1.3 ms on the full-resolution, short-K layers of the other BatchNorm nets
-        self.fuse_bn_stats = True
-        self.sync_bn_group = None       # torch.distributed group: BatchNorm statistics over all ranks (SyncBatchNorm)
-        # Training: a conv output read only by a BatchNorm is stored CENTRED on that BatchNorm's running mean (the shift rides
-        # in the conv bias, in fp32, before the bf16 rounding; BatchNorm is shift-invariant; the running-mean update adds it
-        # back).  Without it a channel with |mean| >> std loses |mean|/std * 2^-9 of relative accuracy in bf16 -- the dominant
-        # error site of the depthwise nets on warm weights (profiles/r2_precision_sites.txt).
-        self.center_pre_bn = os.environ.get("B2U_CENTER_PRE_BN", "1") == "1"
-        self.bn_stats_min_k = 1024
-        self.bn_stats_min_cout = 256
         readers = {}
         for i in program:
             for key in ("x", "x1", "z", "res", "a", "b"):
@@ -330,11 +304,9 @@ class GraphEngine:
         # eval-mode folding: conv output -> the BatchNorm (without residual) that is its only reader
         self._fold_bn = {i["z"]: i for i in program if i["op"] == "bn" and i["z"] in self._pre_bn and not i["res"]}
         self._bn_reader = {i["z"]: i for i in program if i["op"] == "bn" and i["z"] in self._pre_bn}      # conv output -> its BatchNorm
-        # "up" outputs read exactly once, as the SECOND source of a stride-1 3x3 conv (unetUp, nets/unet.py:16-18): that conv
-        # interpolates the low-resolution tensor in its producer warps (b2u_decoder_conv_fprop) and the "up" instruction
-        # launches nothing.  B2U_FUSE_UPSAMPLE: 0 = never, 1 = where it pays (N tiles of >= 128 output channels, see engine.py),
-        # 2 = every such conv.
-        self.fuse_upsample = int(os.environ.get("B2U_FUSE_UPSAMPLE", "1"))
+        # "up" outputs read exactly once, as the SECOND source of a stride-1 3x3 conv (unetUp, nets/unet.py:16-18) -> padded
+        # output channels of that conv: where fuse_upsample() says so, the conv interpolates the low-resolution tensor in its
+        # producer warps (b2u_decoder_conv_fprop) and the "up" instruction launches nothing
         ups = {i["out"] for i in program if i["op"] == "up"}
         self._lazy_up = {i["x1"]: pad64(i["cout"]) for i in program if i["op"] == "conv" and i.get("x1") in ups
                          and len(readers.get(i["x1"], [])) == 1 and i["taps"] == 9 and i["stride"] == 1 and not i.get("pk")}
@@ -395,47 +367,10 @@ class GraphEngine:
         return out
 
     # ------------------------------------------------------------------ buffers
-    def _buf(self, key, shape, dtype=None):
-        dtype = ops.act_dtype() if dtype is None else dtype      # bf16; fp32 under the fp32 validation build
-        t = self._bufs.get(key)
-        if t is None or tuple(t.shape) != tuple(shape) or t.dtype != dtype:
-            t = torch.empty(shape, dtype=dtype, device=self.device)
-            self._bufs[key] = t
-        return t
-
-    def _workspace(self, key, nbytes):
-        t = self._ws.get(key)
-        if t is None or t.numel() < nbytes:
-            t = torch.empty(max(int(nbytes), 16), dtype=torch.uint8, device=self.device)
-            self._ws[key] = t
-        return t
-
-    def _padded(self, key, t, shape, fill=0.0):
-        """fp32 parameter padded with `fill` to `shape` (persistent buffer; the real part is refreshed every call)."""
-        if tuple(t.shape) == tuple(shape):
-            return t
-        b = self._bufs.get(key)
-        if b is None or tuple(b.shape) != tuple(shape):
-            b = torch.full(shape, fill, dtype=torch.float32, device=self.device)
-            self._bufs[key] = b
-        b[tuple(slice(0, d) for d in t.shape)].copy_(t)
-        return b
-
-    def _folded_bn(self, bn_ins, params, conv_bias, cp):
-        """(scale, bias) of `conv -> eval BatchNorm` as one affine map, padded to cp channels."""
-        bnn = bn_ins["bn"]
-        gamma = self._padded("g:" + bnn, params[bnn + ".weight"], (cp,), 1.0)
-        beta = self._padded("bt:" + bnn, params[bnn + ".bias"], (cp,))
-        rmp = self._padded("rm:" + bnn, params[bnn + ".running_mean"], (cp,))
-        rvp = self._padded("rv:" + bnn, params[bnn + ".running_var"], (cp,), 1.0)
-        cb = self._padded("b:" + bnn, conv_bias, (cp,)) if conv_bias is not None else None
-        return ops.bn_fold(gamma, beta, rmp, rvp, cb, self.eps, scale=self._buf("fs:" + bnn, (cp,), torch.float32),
-                           bias=self._buf("fb:" + bnn, (cp,), torch.float32))
-
     def _center_shift(self, ins, params, training, width):
         """Padded running mean of the BatchNorm that is the only reader of this conv's output (training, bf16 path), or None."""
         bn_ins = self._bn_reader.get(ins["out"])
-        if bn_ins is None or not training or not self.center_pre_bn or ops.act_dtype() != torch.bfloat16:
+        if bn_ins is None or not self.center_pre_bn(training):
             return None
         return self._padded("rm:" + bn_ins["bn"], params[bn_ins["bn"] + ".running_mean"], (width,))
 
@@ -448,9 +383,6 @@ class GraphEngine:
         b[:, :t.numel()].copy_(t.reshape(1, -1).expand(f, -1))
         return b.view(-1)
 
-    def release(self):
-        self._bufs.clear(); self._ws.clear(); self.saved = None
-
     # ------------------------------------------------------------------ weights
     def pack(self, params, need_dgrad=True):
         names = list(self.convs.keys())
@@ -462,7 +394,7 @@ class GraphEngine:
             return
         dev = params[names[0]].device
         if self._pack_key != key:
-            blob, start = b"", 0
+            layers = []
             for n in names:
                 cout, c0, c1, taps = self.convs[n]
                 c0p, c1p, coutp = pad64(c0), (pad64(c1) if c1 else 0), pad64(cout)
@@ -492,11 +424,9 @@ class GraphEngine:
                 if need_dgrad and wd is None:
                     wd = torch.zeros((c0p + c1p, taps * coutp), dtype=ops.act_dtype(), device=dev)
                 self._packed[n] = (wf, wd)
-                blob += struct.pack("<QQQqiiiiiiii", src.data_ptr(), wf.data_ptr(), wd.data_ptr() if need_dgrad else 0,
-                                    start, cout, c0 + c1, taps, 0, c0, c0p, c0p + c1p, coutp)
-                start += ((cout + 31) // 32) * ((c0 + c1 + 31) // 32)
-            self._pack_table = torch.frombuffer(bytearray(blob), dtype=torch.uint8).to(dev)
-            self._pack_total, self._pack_key = start, key
+                layers.append((src, wf, wd if need_dgrad else None, cout, c0 + c1, taps, False, c0, c0p, c0p + c1p, coutp))
+            self._set_pack_table(layers, dev)
+            self._pack_key = key
         for n, ci in self.image_convs.items():   # refresh [w | w]
             if n not in self.pk:
                 w2, w = self._bufs["w2:" + n], params[n]
@@ -517,13 +447,10 @@ class GraphEngine:
                 mid, co, cop = ins["cin"], ins["cout"], pad64(ins["cout"])
                 for k in range(f):
                     w2[k * cop:k * cop + co, k * midp:k * midp + mid].copy_(w)
-        ops.check(ops.lib().b2u_pack_weights_multi(self._pack_table.data_ptr(), len(names), self._pack_total, ops.stream_ptr()))
+        self._launch_pack()
         if self.has_stem:
             self._stem_wf = ops.pack_weights_im2col(params["resnet.conv1.weight"], 192, wf=getattr(self, "_stem_wf", None))
         self._pack_versions = versions
-
-    def invalidate_packed_weights(self):
-        self._pack_versions = None
 
     # ------------------------------------------------------------------ forward
     def forward(self, x, params, save=True, training=None, trainable=None):
@@ -573,7 +500,7 @@ class GraphEngine:
                         bias = torch.sub(bias, self._tiled("c2:" + ins["w"], shift, z.shape[3], f), out=self._buf("bc:" + ins["w"], (bias.numel(),), torch.float32))
                     fold = self._fold_bn.get(ins["out"]) if (not training and not save) else None
                     if fold is not None:        # eval: BatchNorm (+ReLU) folded into the epilogue, vectors tiled like the bias
-                        sc, bs = self._folded_bn(fold, params, params[ins["bias"]], z.shape[3])
+                        sc, bs = self._folded_bn(fold["bn"], params, params[ins["bias"]], z.shape[3])
                         sc = self._tiled("fs2:" + ins["w"], sc, z.shape[3], f)
                         bs = self._tiled("fb2:" + ins["w"], bs, z.shape[3], f)
                         ops.conv_fprop_scaled(xin.data.view(n, h, w // f, -1), wf, sc, bs, z.shape[3] * f, taps=1, relu=fold["relu"],
@@ -611,7 +538,7 @@ class GraphEngine:
                 fold = self._fold_bn.get(ins["out"]) if (not training and not save) else None
                 if fold is not None:
                     # eval mode: y = [relu](acc * s + b') straight from the conv epilogue; the BatchNorm instruction passes it on
-                    sc, bs = self._folded_bn(fold, params, params[ins["bias"]] if ins["bias"] else None, coutp)
+                    sc, bs = self._folded_bn(fold["bn"], params, params[ins["bias"]] if ins["bias"] else None, coutp)
                     if ins["stride"] == 1 and low is not None:
                         z = self._buf(ins["out"], (n, h, w, coutp))
                         ops.decoder_conv_fprop(xin.data, low, wf, bs, coutp, relu=fold["relu"], out=z, up_out=up_out, scale=sc)
@@ -635,12 +562,10 @@ class GraphEngine:
                 if ins["stride"] == 1:
                     z = self._buf(ins["out"], (n, h, w, coutp))
                     kdim = ins["taps"] * (xin.data.shape[3] + (low.shape[3] if low is not None else x1.data.shape[3] if x1 else 0))
-                    if (training and self.fuse_bn_stats and self.sync_bn_group is None and ins["out"] in self._pre_bn
-                            and (kdim >= self.bn_stats_min_k or coutp >= self.bn_stats_min_cout)):
+                    if ins["out"] in self._pre_bn and self.fuse_bn_stats(training, kdim, coutp):
                         # the BatchNorm that reads this output takes its statistics from this conv's epilogue (no pass over
                         # z); one buffer per conv output: another conv may run before that BatchNorm (downsample branches)
-                        rows = ops.conv_stat_rows(n, h, w, coutp, ins["taps"], bn=(1 << 18) if low is not None else 0)
-                        stats = (self._workspace("bnstat:" + ins["out"], rows * 2 * coutp * 4)[:rows * 2 * coutp * 4].view(torch.float32), rows)
+                        stats = self._bn_stats("bnstat:" + ins["out"], n, h, w, coutp, ins["taps"], decoder=low is not None)
                     if low is not None:
                         ops.decoder_conv_fprop(xin.data, low, wf, bias, coutp, relu=ins["relu"], out=z, up_out=up_out,
                                                stats=stats[0] if stats else None)
@@ -668,36 +593,13 @@ class GraphEngine:
                     T[ins["out"]] = _T(zt.data)
                     continue
                 res = T[ins["res"]] if ins["res"] else None
-                bnn, c = ins["bn"], ins["c"]
-                cp = zt.data.shape[3]
+                bnn = ins["bn"]
                 y = self._buf(ins["out"], zt.data.shape)
-                ws = self._workspace("bn", ops.lib().b2u_bn_workspace(cp))
-                gamma = self._padded("g:" + bnn, params[bnn + ".weight"], (cp,), 1.0)
-                beta = self._padded("bt:" + bnn, params[bnn + ".bias"], (cp,))
-                rm, rv = params[bnn + ".running_mean"], params[bnn + ".running_var"]
-                rmp, rvp = self._padded("rm:" + bnn, rm, (cp,)), self._padded("rv:" + bnn, rv, (cp,), 1.0)
-                if training:
-                    if self.sync_bn_group is not None:
-                        _, mean, invstd = ops.bn_fwd_train_sync(zt.data, gamma, beta, rmp, rvp, self.sync_bn_group, self.eps,
-                                                                self.momentum, ins["relu"], out=y, ws=ws,
-                                                                residual=res.data if res else None, centered=zt.centered)
-                    else:
-                        _, mean, invstd = ops.bn_fwd_train(zt.data, gamma, beta, rmp, rvp, self.eps, self.momentum, ins["relu"],
-                                                           out=y, ws=ws, residual=res.data if res else None,
-                                                           stats=zt.stats[0] if zt.stats else None, stat_rows=zt.stats[1] if zt.stats else 0,
-                                                           centered=zt.centered)
-                    if cp != c:
-                        rm.copy_(rmp[:c]); rv.copy_(rvp[:c])
-                    nbt = params.get(bnn + ".num_batches_tracked")
-                    if nbt is not None:
-                        nbt.add_(1)
-                else:
-                    ops.bn_fwd_eval(zt.data, gamma, beta, rmp, rvp, self.eps, ins["relu"], out=y, ws=ws,
-                                    residual=res.data if res else None)
-                    mean, invstd = (rmp, rvp), None        # eval mode: the backward uses the running statistics (constants)
+                aux = self._bn_fwd(bnn, zt.data, params, training, ins["relu"], y, residual=res.data if res else None,
+                                   stats=zt.stats, centered=zt.centered)
                 ng = zt.needs_grad or (res is not None and res.needs_grad) or (bnn + ".weight") in trainable or (bnn + ".bias") in trainable
                 t = _T(y, needs_grad=ng)
-                t.aux = (mean, invstd, gamma, beta)
+                t.aux = aux
                 T[ins["out"]] = t
             elif op == "dw":
                 xin = T[ins["x"]]
@@ -757,7 +659,7 @@ class GraphEngine:
             elif op == "up":
                 xin = T[ins["x"]]
                 n, h, w, c = xin.data.shape
-                if ins["out"] in self._lazy_up and (self.fuse_upsample == 2 or (self.fuse_upsample == 1 and self._lazy_up[ins["out"]] >= 128)):
+                if ins["out"] in self._lazy_up and self.fuse_upsample(self._lazy_up[ins["out"]]):
                     t = _T(None, needs_grad=xin.needs_grad)          # the reading conv interpolates xin itself
                     t.low = xin.data
                     T[ins["out"]] = t
@@ -922,22 +824,13 @@ class GraphEngine:
                     continue
                 bnn, c = ins["bn"], ins["c"]
                 cp = zt.data.shape[3]
-                mean, invstd, gamma, beta = t.aux
                 need_res = res is not None and res.needs_grad
                 gout = self._buf("g:" + ins["out"] + ">res", t.data.shape) if need_res else None
                 dz = self._buf("g:" + ins["z"], zt.data.shape)
                 direct = cp == c
                 dgam = grads[bnn + ".weight"] if (direct and has(bnn + ".weight")) else self._buf("dg:" + bnn, (cp,), torch.float32)
                 dbet = grads[bnn + ".bias"] if (direct and has(bnn + ".bias")) else self._buf("db:" + bnn, (cp,), torch.float32)
-                # y is read only where a residual was added before the ReLU; otherwise the mask is recomputed from z
-                if invstd is None:          # eval-mode forward (model.eval() + backward): statistics are constants
-                    ops.bn_bwd_eval(t.grad, t.data, zt.data, gamma, beta, mean[0], mean[1], self.eps, relu=ins["relu"], out=dz,
-                                    dgamma=dgam, dbeta=dbet, ws=self._workspace("bn", ops.lib().b2u_bn_workspace(cp)), gout=gout)
-                else:
-                    bwd = ops.bn_bwd if self.sync_bn_group is None else functools.partial(ops.bn_bwd_sync, group=self.sync_bn_group)
-                    bwd(t.grad, t.data if res is not None else None, zt.data, gamma, mean, invstd, relu=ins["relu"], out=dz,
-                        dgamma=dgam, dbeta=dbet, beta=beta,
-                        ws=self._workspace("bn", ops.lib().b2u_bn_workspace(cp)), gout=gout)
+                self._bn_bwd(t.grad, t.data, zt.data, t.aux, ins["relu"], dz, dgam, dbet, residual=res is not None, gout=gout)
                 if not direct:
                     if has(bnn + ".weight"):
                         grads[bnn + ".weight"].copy_(dgam[:c])
@@ -1019,8 +912,7 @@ class GraphEngine:
                 xw = t.aux if (ins["stride"] == 2 and taps == 1) else xin.data          # wgrad's activation operand
                 c0p = xw.shape[3]
                 c1p = x1.data.shape[3] if x1 else 0
-                # 3x3 layers with a live bias: db comes out of the wgrad kernel (its bias warp sums the staged dz tiles)
-                fused_db = ((self.fuse_bias_grad or coutp == 64) and has(ins["w"]) and has(ins["bias"]) and taps == 9 and ins["out"] not in self._pre_bn
+                fused_db = (self.fused_db(coutp) and has(ins["w"]) and has(ins["bias"]) and taps == 9 and ins["out"] not in self._pre_bn
                             and coutp == cout and c0p == c0r and c1p == c1r)
                 if has(ins["w"]):
                     need = ops.lib().b2u_conv_wgrad_workspace(dz.shape[0], dz.shape[1], dz.shape[2], c0p + c1p, coutp, taps)
