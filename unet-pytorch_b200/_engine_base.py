@@ -4,8 +4,13 @@ the other families).
   buffers    activation buffers, kernel workspaces and padded parameter vectors, cached by key across steps
   weights    the device table of b2u_pack_weights_multi (one record per conv) and its launch
   policies   which fused kernel variant runs where -- each decided by a B200 measurement (DESIGN.md)
-  BatchNorm  forward (train / SyncBatchNorm / eval, padded running statistics) and the backward dispatch
+  BatchNorm  forward (train / SyncBatchNorm / eval, padded running statistics) and backward (dgamma / dbeta included)
+  convs      the choice among the forward conv launches, and a conv's weight and bias gradients
+  head       the 1x1 classifier, forward and backward
+
+Each engine decides WHICH of these a layer runs (its topology, its ReLU masks, its streams); the launches are written here once.
 """
+import contextlib
 import functools
 import struct
 
@@ -158,12 +163,17 @@ class EngineBase:
             nbt.add_(1)
         return mean, invstd, gamma, beta
 
-    def _bn_bwd(self, dy, y, z, saved, relu, out, dgamma, dbeta, residual=False, gout=None):
-        """Backward of _bn_fwd (saved = what it returned): dz into out, padded dgamma / dbeta; gout receives the ReLU-masked
-        dy (the residual branch's gradient).  y is read in eval mode and where a residual was added before the ReLU;
-        otherwise the mask is recomputed from z."""
+    def _bn_bwd(self, dy, y, z, saved, relu, out, grads, has, bn, c, residual=False, gout=None):
+        """Backward of _bn_fwd (saved = what it returned) for BatchNorm `bn` of c real channels: dz into out, dgamma / dbeta
+        into grads (through padded buffers when z's channels are padded); gout receives the ReLU-masked dy (the residual
+        branch's gradient).  y is read in eval mode and where a residual was added before the ReLU; otherwise the mask is
+        recomputed from z."""
         mean, invstd, gamma, beta = saved
-        ws = self._workspace("bn", ops.lib().b2u_bn_workspace(z.shape[3]))
+        cp = z.shape[3]
+        wn, bn_ = bn + ".weight", bn + ".bias"
+        dgamma = grads[wn] if cp == c and has(wn) else self._buf("dg:" + bn, (cp,), torch.float32)
+        dbeta = grads[bn_] if cp == c and has(bn_) else self._buf("db:" + bn, (cp,), torch.float32)
+        ws = self._workspace("bn", ops.lib().b2u_bn_workspace(cp))
         if invstd is None:          # eval-mode forward (model.eval() + backward): the statistics are constants
             ops.bn_bwd_eval(dy, y, z, gamma, beta, mean[0], mean[1], self.eps, relu=relu, out=out, dgamma=dgamma, dbeta=dbeta,
                             ws=ws, gout=gout)
@@ -171,3 +181,115 @@ class EngineBase:
             bwd = ops.bn_bwd if self.sync_bn_group is None else functools.partial(ops.bn_bwd_sync, group=self.sync_bn_group)
             bwd(dy, y if residual else None, z, gamma, mean, invstd, relu=relu, out=out, dgamma=dgamma, dbeta=dbeta, beta=beta,
                 ws=ws, gout=gout)
+        if cp != c:
+            if has(wn):
+                grads[wn].copy_(dgamma[:c])
+            if has(bn_):
+                grads[bn_].copy_(dbeta[:c])
+
+    # ------------------------------------------------------------------ convolutions
+    def _conv_fwd(self, x0, wf, bias, cout_p, taps, relu, out, x1=None, low=None, up_out=None, scale=None, stats=None):
+        """One conv launch into out: over x0 (+ x1, virtual concat), or over x0 + upsample2x(low) interpolated inside the
+        kernel (up_out optionally receives the up-sampled tensor); scale: an eval-mode BatchNorm folded into the epilogue;
+        stats: (per-tile column sums, rows) of _bn_stats, which the epilogue fills."""
+        sums = stats[0] if stats else None
+        if low is not None:
+            return ops.decoder_conv_fprop(x0, low, wf, bias, cout_p, relu=relu, out=out, up_out=up_out, scale=scale, stats=sums)
+        if scale is not None:
+            return ops.conv_fprop_scaled(x0, wf, scale, bias, cout_p, taps=taps, relu=relu, x1=x1, out=out)
+        return ops.conv_fprop(x0, wf, bias, cout_p, taps=taps, relu=relu, x1=x1, out=out, stats=sums)
+
+    def _conv_param_grads(self, x0, dz, grads, has, w, b, cout, c0, c1=0, x1=None, taps=9, pre_bn=False, first_cin=0,
+                          lo_half=False, db_stats=None):
+        """Weight gradient grads[w] and bias gradient grads[b] of a stride-1 conv over x0 (+ x1) with output gradient dz (a
+        stride-2 conv passes its stride-1 form: zero-inserted dz, or the subsampled x0 of a 1x1).  c0 / c1: real input channels of the two sources (x0 / x1 hold them zero-padded); cout: real output channels.
+        first_cin: x0 is the im2col of a first_cin-channel image (UNetEngine's first layer); lo_half: x0's channels
+        [c0, 2 c0) are the lo half of the image split and add to the same weights; pre_bn: a BatchNorm reads the output;
+        db_stats: (column sums, rows) of dz that the dgrad producing it left behind (UNetEngine.bias_from_dgrad)."""
+        cout_p, c0_p, c1_p = dz.shape[3], x0.shape[3], (x1.shape[3] if x1 is not None else 0)
+        direct = cout_p == cout and (first_cin or (c0_p == c0 and c1_p == c1))
+        fuse_b = has(w) and has(b) and direct and taps == 9 and not pre_bn and self.fused_db(cout_p)
+        if has(w):
+            need = ops.lib().b2u_conv_wgrad_workspace(dz.shape[0], dz.shape[1], dz.shape[2], c0_p + c1_p, cout_p, taps)
+            ws = self._workspace("wgrad", need)
+            if direct:
+                ops.conv_wgrad(x0, dz, taps=taps, x1=x1, first_cin=first_cin, dw=grads[w], db=grads[b] if fuse_b else None,
+                               ws=ws)
+            else:       # padded operands: gradient of the padded weight, then keep the real rows / columns
+                k = 3 if taps == 9 else 1
+                tmp = self._buf("dw:" + w, (cout_p, first_cin, 3, 3) if first_cin else (cout_p, c0_p + c1_p, k, k),
+                                torch.float32)
+                ops.conv_wgrad(x0, dz, taps=taps, x1=x1, first_cin=first_cin, dw=tmp, ws=ws)
+                gw = grads[w]
+                if first_cin:
+                    gw.copy_(tmp[:cout])
+                else:
+                    gw[:, :c0].copy_(tmp[:cout, :c0])
+                    if lo_half:
+                        gw[:, :c0].add_(tmp[:cout, c0:2 * c0])
+                    if c1:
+                        gw[:, c0:].copy_(tmp[:cout, c0_p:c0_p + c1])
+        if has(b) and pre_bn:
+            # a bias in front of BatchNorm: dz = a (g - mean(g) - xhat mean(g xhat)) sums to zero over the batch exactly,
+            # so the gradient is 0 (the reference's autograd returns fp32 cancellation residue ~1e-8)
+            grads[b].zero_()
+        elif has(b) and not fuse_b and db_stats is not None:
+            ops.bias_from_stats(db_stats[0], db_stats[1], cout_p, db=grads[b])
+        elif has(b) and not fuse_b:
+            ws = self._workspace("bias", ops.lib().b2u_bias_grad_workspace(cout_p))
+            if cout_p == cout:
+                ops.bias_grad(dz, db=grads[b], ws=ws)
+            else:
+                tb = ops.bias_grad(dz, db=self._buf("dbias:" + w, (cout_p,), torch.float32), ws=ws)
+                grads[b].copy_(tb[:cout])
+
+    # ------------------------------------------------------------------ classifier head
+    def _head_weight(self, params, w, cin):
+        return self._padded("head:w", params[w].reshape(self.num_classes, cin), (self.num_classes, 64))
+
+    def _head_fwd(self, x, params, w, b, cin):
+        """1x1 classifier -> fp32 NCHW logits: on the tensor cores ([hi | lo] bf16 split of the fp32 weights); the fp32
+        validation build runs a plain fp32 1x1 conv."""
+        wh = self._head_weight(params, w, cin)
+        if ops.act_dtype() == torch.float32:
+            return ops.head_fwd(x, wh, params[b])
+        wf = ops.pack_head_fprop(wh, wf=self._buf("head:wf", (64 * ops.head_groups(self.num_classes), 64)))
+        return ops.head_fwd_tc(x, wf, params[b], self.num_classes)
+
+    def _head_bwd(self, dlogits, x, params, grads, has, w, b, cin, g, mask, bits=None, grad_stream=contextlib.nullcontext):
+        """Backward of _head_fwd: the gradient wrt x into g (None: not needed), ReLU-masked by mask (= x) or by bits (x's bit
+        mask) when given; grads[w] / grads[b] from weight-gradient launches run under grad_stream()."""
+        C = self.num_classes
+        wh = self._head_weight(params, w, cin)
+        fw, fb = has(w), has(b)
+        cz = 64 * ops.head_groups(C)
+        if dlogits.dtype == torch.bfloat16 and dlogits.dim() == 4 and dlogits.shape[-1] == cz and ops.act_dtype() == torch.bfloat16:
+            # [N,H,W,64 G] = per group of 32 classes, [hi | lo] split dlogits from loss_bwd(nhwc64=True): the head's backward
+            # runs on the tensor cores as a 1x1 dgrad (+ReLU mask) and a 1x1 wgrad (+bias) over G x 2 x 32 padded classes
+            dl = dlogits.contiguous()
+            if g is not None:
+                wd = ops.pack_head_dgrad(wh, wd=self._buf("head:wd", (64, cz)))
+                if bits is not None:
+                    ops.conv_dgrad_bits(dl, wd, 64, bits, taps=1, out0=g)
+                else:
+                    ops.conv_dgrad(dl, wd, 64, taps=1, mask=mask, out0=g)
+            if fw or fb:
+                dw64 = self._buf("head:dw", (cz, 64, 1, 1), torch.float32)
+                db64 = self._buf("head:db", (cz,), torch.float32)
+                need = ops.lib().b2u_conv_wgrad_workspace(dl.shape[0], dl.shape[1], dl.shape[2], 64, cz, 1)
+                with grad_stream():
+                    ops.conv_wgrad(x, dl, taps=1, dw=dw64, db=db64, ws=self._workspace("wgrad", need))
+                    # in group g, rows 64g + [0,32) came from the hi half of dlogits, rows 64g + [32,64) from the lo half
+                    if fw:
+                        ops.fold_head_groups(dw64, C, cin, grads[w])
+                    if fb:
+                        ops.fold_head_groups(db64, C, cin, grads[b])
+        else:
+            dl = dlogits.float().contiguous() if dlogits.dtype != torch.float32 else dlogits.contiguous()
+            dwt = None
+            if fw:
+                dwt = grads[w] if cin == 64 else self._buf("head:dwf", (C, 64, 1, 1), torch.float32)
+            ops.head_bwd(dl, x, wh, need_dx=g is not None, need_dw=fw or fb, relu_mask=mask is not None, dx=g, dw=dwt,
+                         db=grads[b] if fb else None, ws=self._workspace("head", ops.lib().b2u_head_bwd_workspace_cls(C)))
+            if fw and cin != 64:
+                grads[w].copy_(dwt[:, :cin])

@@ -11,6 +11,10 @@ libb200unet.so in the order of the reference's forward, then the hand-derived ba
             upsample adjoint -> per encoder block: wgrad, dgrad, pool bwd (+skip grad); ReLU masks are fused into the
             dgrad / pool / upsample kernels (plain nets) or applied by the BN backward kernel (BN nets)
 
+The per-layer launches (conv forward, conv parameter gradients, BatchNorm, head) are EngineBase's (_engine_base.py), shared
+with GraphEngine; this engine adds what only the plain conv + ReLU nets use: ReLU bit masks, bias gradients from the
+dgrad epilogue and the weight-gradient side stream.
+
 Channel counts that are not multiples of 64 (the 32-channel layers of TraditionalUnet) are zero-padded to 64 in the
 activation buffers and operands; padded channels stay exactly zero in both directions.
 
@@ -216,32 +220,19 @@ class UNetEngine(EngineBase):
         n, h, w, _ = x0.shape
         bias = self._padded("b:" + c.name, params[c.name + ".bias"], (c.cout_p,))
         taps = 1 if c.first else 9
-
-        def conv(bias_, relu, out, stats=None, scale=None):
-            if low is not None:
-                return ops.decoder_conv_fprop(x0, low, c.wf, bias_, c.cout_p, relu=relu, out=out, up_out=up_out, scale=scale, stats=stats)
-            if scale is not None:
-                return ops.conv_fprop_scaled(x0, c.wf, scale, bias_, c.cout_p, taps=taps, relu=relu, x1=x1, out=out)
-            return ops.conv_fprop(x0, c.wf, bias_, c.cout_p, taps=taps, relu=relu, x1=x1, out=out, stats=stats)
-
-        if not c.bn:
-            out = self._buf(c.name, (n, h, w, c.cout_p))
-            if self.relu_bit_masks(save):
-                bits = self._buf("bits:" + c.name, (n, h, w, c.cout_p // 64), torch.int64)
-                ops.conv_fprop_relu_bits(x0, c.wf, bias, c.cout_p, bits, taps=taps, x1=x1, low=low, up_out=up_out, out=out)
-                A["bits:" + c.name] = bits
-            else:
-                conv(bias, True, out)
-            A[c.name] = out
+        out = A[c.name] = self._buf(c.name, (n, h, w, c.cout_p))
+        if not c.bn and self.relu_bit_masks(save):
+            bits = A["bits:" + c.name] = self._buf("bits:" + c.name, (n, h, w, c.cout_p // 64), torch.int64)
+            ops.conv_fprop_relu_bits(x0, c.wf, bias, c.cout_p, bits, taps=taps, x1=x1, low=low, up_out=up_out, out=out)
             return out
-        if not training and not save:
+        if not c.bn or (not training and not save):
             # pure inference: BatchNorm is an affine map with fixed statistics, folded into the conv epilogue
             # (y = relu(acc * s + b')): no z tensor, no BatchNorm pass.  An eval-mode forward that will be back-propagated
             # (model.eval() + loss.backward()) takes the unfused path below so the BatchNorm backward has z
-            sc, bs = self._folded_bn(c.bn, params, bias, c.cout_p)
-            out = self._buf(c.name, (n, h, w, c.cout_p))
-            conv(bs, True, out, scale=sc)
-            A[c.name] = out
+            scale = None
+            if c.bn:
+                scale, bias = self._folded_bn(c.bn, params, bias, c.cout_p)
+            self._conv_fwd(x0, c.wf, bias, c.cout_p, taps, True, out, x1=x1, low=low, up_out=up_out, scale=scale)
             return out
         z = self._buf("z:" + c.name, (n, h, w, c.cout_p))
         centered = self.center_pre_bn(training)
@@ -252,10 +243,8 @@ class UNetEngine(EngineBase):
         kdim = taps * (x0.shape[3] + (x1.shape[3] if x1 is not None else 0) + (low.shape[3] if low is not None else 0))
         if self.fuse_bn_stats(training, kdim, c.cout_p):
             stats = self._bn_stats("bnstat", n, h, w, c.cout_p, taps, decoder=low is not None)
-        conv(bias, False, z, stats=stats[0] if stats else None)
-        out = self._buf(c.name, (n, h, w, c.cout_p))
+        self._conv_fwd(x0, c.wf, bias, c.cout_p, taps, False, z, x1=x1, low=low, up_out=up_out, stats=stats)
         A["bn:" + c.name] = (z,) + self._bn_fwd(c.bn, z, params, training, True, out, stats=stats, centered=centered)
-        A[c.name] = out
         return out
 
     # ------------------------------------------------------------------ forward
@@ -312,20 +301,10 @@ class UNetEngine(EngineBase):
                 o1 = self._layer_fwd(c1, skip, params, A, training, x1=up, save=save)
             A[f"up{si}"] = up
             low = self._layer_fwd(c2, o1, params, A, training, save=save)
-        wh = self._head_weight(params)
-        # 1x1 classifier on the tensor cores: [hi | lo] bf16 split of the fp32 weights, fp32 NCHW logits from the epilogue
-        if ops.act_dtype() == torch.float32:       # fp32 validation build: plain fp32 1x1 conv
-            logits = ops.head_fwd(low, wh, params[self.head_name + ".bias"])
-        else:
-            wf_head = ops.pack_head_fprop(wh, wf=self._buf("head:wf", (64 * ops.head_groups(self.num_classes), 64)))
-            logits = ops.head_fwd_tc(low, wf_head, params[self.head_name + ".bias"], self.num_classes)
+        logits = self._head_fwd(low, params, self.head_name + ".weight", self.head_name + ".bias", self.head_cin)
         if save:
             self.saved = (A, feats, (N, H, W))
         return logits
-
-    def _head_weight(self, params):
-        w = params[self.head_name + ".weight"].reshape(self.num_classes, self.head_cin)
-        return self._padded("head:w", w, (self.num_classes, 64))
 
     # ------------------------------------------------------------------ backward
     def backward(self, dlogits, params, grads, trainable=None, on_grads_ready=None):
@@ -420,108 +399,24 @@ class UNetEngine(EngineBase):
         def layer_bwd(c, x0, g, x1=None):
             """g: gradient wrt the layer's output (BN nets: wrt y, unmasked; plain nets: wrt the pre-activation, already
             masked).  Runs BN backward if any, wgrad, bias grad; returns dz (the conv's output gradient)."""
-            dz = g
             if c.bn:
                 z, *saved = A["bn:" + c.name]
-                wn, bnn = c.bn + ".weight", c.bn + ".bias"
-                dgam = self._buf("dg:" + c.bn, (c.cout_p,), torch.float32)
-                dbet = self._buf("db:" + c.bn, (c.cout_p,), torch.float32)
-                self._bn_bwd(g, A[c.name], z, saved, True, g, dgam, dbet)
-                if has(wn):
-                    grads[wn].copy_(dgam[:c.cout])
-                if has(bnn):
-                    grads[bnn].copy_(dbet[:c.cout])
-                ready(wn, bnn)
-            if not want[c.name]:
-                return dz
-            with grad_stream():
-                param_grads(c, x0, dz, x1)
-            return dz
-
-        def param_grads(c, x0, dz, x1):
-            wn, bn_ = c.name + ".weight", c.name + ".bias"
-            want_w, want_b = has(wn), has(bn_)
-            fuse_b = want_w and want_b and not c.padded and not c.bn and not c.first and self.fused_db(c.cout_p)
-            taps = 1 if c.first else 9
-            if want_w:
-                ctot_p = 64 if c.first else c.c0_p + c.c1_p
-                need = ops.lib().b2u_conv_wgrad_workspace(dz.shape[0], dz.shape[1], dz.shape[2], ctot_p, c.cout_p, taps)
-                ws = self._workspace("wgrad", need)
-                if not c.padded:
-                    ops.conv_wgrad(x0, dz, taps=taps, x1=x1, first_cin=c.cin if c.first else 0, dw=grads[wn],
-                                   db=grads[bn_] if fuse_b else None, ws=ws)
-                else:
-                    if c.first:
-                        tmp = self._buf("dw:" + c.name, (c.cout_p, c.cin, 3, 3), torch.float32)
-                        ops.conv_wgrad(x0, dz, taps=1, first_cin=c.cin, dw=tmp, ws=ws)
-                        grads[wn].copy_(tmp[:c.cout])
-                    else:
-                        tmp = self._buf("dw:" + c.name, (c.cout_p, ctot_p, 3, 3), torch.float32)
-                        ops.conv_wgrad(x0, dz, taps=9, x1=x1, dw=tmp, ws=ws)
-                        if c.c1:
-                            grads[wn][:, :c.c0].copy_(tmp[:c.cout, :c.c0])
-                            grads[wn][:, c.c0:].copy_(tmp[:c.cout, c.c0_p:c.c0_p + c.c1])
-                        else:
-                            grads[wn].copy_(tmp[:c.cout, :c.c0])
-            if want_b and c.bn:
-                # a bias in front of BatchNorm: dz = a (g - mean(g) - xhat mean(g xhat)) sums to zero over the batch
-                # exactly, so the gradient is 0 (the reference's autograd returns fp32 cancellation residue ~1e-8)
-                grads[bn_].zero_()
-            elif want_b and not fuse_b and c.name in db_stats:
-                st_, rows_ = db_stats.pop(c.name)
-                ops.bias_from_stats(st_, rows_, c.cout_p, db=grads[bn_])
-            elif want_b and not fuse_b:
-                if c.cout_p == c.cout:
-                    ops.bias_grad(dz, db=grads[bn_], ws=self._workspace("bias", ops.lib().b2u_bias_grad_workspace(c.cout_p)))
-                else:
-                    tmpb = self._buf("dbias:" + c.name, (c.cout_p,), torch.float32)
-                    ops.bias_grad(dz, db=tmpb, ws=self._workspace("bias", ops.lib().b2u_bias_grad_workspace(c.cout_p)))
-                    grads[bn_].copy_(tmpb[:c.cout])
-            ready(wn, bn_)
+                self._bn_bwd(g, A[c.name], z, saved, True, g, grads, has, c.bn, c.cout)
+                ready(c.bn + ".weight", c.bn + ".bias")
+            if want[c.name]:
+                with grad_stream():
+                    self._conv_param_grads(x0, g, grads, has, c.name + ".weight", c.name + ".bias", c.cout, c.c0, c.c1, x1=x1,
+                                           taps=1 if c.first else 9, pre_bn=bool(c.bn), first_cin=c.cin if c.first else 0,
+                                           db_stats=db_stats.pop(c.name, None))
+                    ready(c.name + ".weight", c.name + ".bias")
+            return g
 
         # ---- head
         hn = self.head_name
         last = A[self.dec[-1][1].name]
-        wh = self._head_weight(params)
-        C = self.num_classes
-        fw, fb = has(hn + ".weight"), has(hn + ".bias")
         g = self._buf("g:" + self.dec[-1][1].name, last.shape) if need_dx[hn] else None
-        cz = 64 * ops.head_groups(C)
-        if dlogits.dtype == torch.bfloat16 and dlogits.dim() == 4 and dlogits.shape[-1] == cz and ops.act_dtype() == torch.bfloat16:
-            # [N,H,W,64 G] = per group of 32 classes, [hi | lo] split dlogits from loss_bwd(nhwc64=True): the head's backward
-            # runs on the tensor cores as a 1x1 dgrad (+ReLU mask) and a 1x1 wgrad (+bias) over G x 2 x 32 padded classes
-            dl = dlogits.contiguous()
-            if need_dx[hn]:
-                wd_head = ops.pack_head_dgrad(wh, wd=self._buf("head:wd", (64, cz)))
-                hbits = None if bn else A.get("bits:" + self.dec[-1][1].name)
-                if hbits is not None:
-                    ops.conv_dgrad_bits(dl, wd_head, 64, hbits, taps=1, out0=g)
-                else:
-                    ops.conv_dgrad(dl, wd_head, 64, taps=1, mask=None if bn else last, out0=g)
-            if fw or fb:
-                dw64 = self._buf("head:dw", (cz, 64, 1, 1), torch.float32)
-                db64 = self._buf("head:db", (cz,), torch.float32)
-                need = ops.lib().b2u_conv_wgrad_workspace(dl.shape[0], dl.shape[1], dl.shape[2], 64, cz, 1)
-                with grad_stream():
-                    ops.conv_wgrad(last, dl, taps=1, dw=dw64, db=db64, ws=self._workspace("wgrad", need))
-                    # in group g, rows 64g + [0,32) came from the hi half of dlogits, rows 64g + [32,64) from the lo half
-                    if fw:
-                        ops.fold_head_groups(dw64, C, self.head_cin, grads[hn + ".weight"])
-                    if fb:
-                        ops.fold_head_groups(db64, C, self.head_cin, grads[hn + ".bias"])
-        else:
-            dl = dlogits.contiguous()
-            if dl.dtype != torch.float32:
-                dl = dl.float()
-            if self.head_cin == 64:
-                dwt, dbt = (grads[hn + ".weight"] if fw else None), (grads[hn + ".bias"] if fb else None)
-            else:
-                dwt = self._buf("head:dwf", (C, 64, 1, 1), torch.float32) if fw else None
-                dbt = grads[hn + ".bias"] if fb else None
-            ops.head_bwd(dl, last, wh, need_dx=need_dx[hn], need_dw=fw or fb, relu_mask=not bn, dx=g, dw=dwt, db=dbt,
-                         ws=self._workspace("head", ops.lib().b2u_head_bwd_workspace_cls(C)))
-            if fw and self.head_cin != 64:
-                grads[hn + ".weight"].copy_(dwt[:, :self.head_cin])
+        self._head_bwd(dlogits, last, params, grads, has, hn + ".weight", hn + ".bias", self.head_cin, g,
+                       None if bn else last, bits=None if bn else A.get("bits:" + self.dec[-1][1].name), grad_stream=grad_stream)
         with grad_stream():          # (orders the side stream after the head's launches, whichever stream ran them)
             ready(hn + ".weight", hn + ".bias")
         if g is None:

@@ -4,7 +4,7 @@
 A network is a list of instructions over named tensors (NHWC bf16, channels multiples of 64).  forward() interprets
 the list and keeps what backward needs; backward() walks it in reverse, accumulating gradients at tensors that have
 several consumers (residual identities, skip connections) with the add kernel.  Every instruction maps to kernels
-of libb200unet.so:
+of libb200unet.so (the conv, BatchNorm and head launches through EngineBase, _engine_base.py, shared with UNetEngine):
 
   stem      7x7 stride-2 conv as im2col rows (K = 147 -> 192) + 1x1 tensor-core GEMM           nets/resnet.py:109
   conv      1x1 / 3x3, stride 1 or 2 (3x3 s2 = stride-1 conv -> keep even pixels; 1x1 s2 = keep even pixels -> conv),
@@ -487,6 +487,11 @@ class GraphEngine(EngineBase):
                 x1 = T[ins["x1"]] if ins["x1"] else None
                 wf, _ = self._packed[ins["w"]]
                 n, h, w, _ = xin.data.shape
+                ng = xin.needs_grad or (x1 is not None and x1.needs_grad) or ins["w"] in trainable or (ins["bias"] in trainable)
+                # folding is for pure inference: an eval-mode forward that will be back-propagated (model.eval() +
+                # loss.backward()) keeps z and runs the BatchNorm instruction so its backward has what it needs
+                fold = self._fold_bn.get(ins["out"]) if (not training and not save) else None
+                scale, relu = None, ins["relu"]
                 if ins.get("pk"):           # pixel-packed 1x1 conv: every tensor is viewed with f pixels per row
                     f = ins["pix"]
                     if ins["pk"] == "to":
@@ -498,17 +503,13 @@ class GraphEngine(EngineBase):
                     shift = self._center_shift(ins, params, training, z.shape[3])
                     if shift is not None:
                         bias = torch.sub(bias, self._tiled("c2:" + ins["w"], shift, z.shape[3], f), out=self._buf("bc:" + ins["w"], (bias.numel(),), torch.float32))
-                    fold = self._fold_bn.get(ins["out"]) if (not training and not save) else None
                     if fold is not None:        # eval: BatchNorm (+ReLU) folded into the epilogue, vectors tiled like the bias
                         sc, bs = self._folded_bn(fold["bn"], params, params[ins["bias"]], z.shape[3])
-                        sc = self._tiled("fs2:" + ins["w"], sc, z.shape[3], f)
-                        bs = self._tiled("fb2:" + ins["w"], bs, z.shape[3], f)
-                        ops.conv_fprop_scaled(xin.data.view(n, h, w // f, -1), wf, sc, bs, z.shape[3] * f, taps=1, relu=fold["relu"],
-                                              x1=x1.data.view(n, h, w // f, -1) if x1 else None, out=z.view(n, h, w // f, -1))
-                    else:
-                        ops.conv_fprop(xin.data.view(n, h, w // f, -1), wf, bias, z.shape[3] * f, taps=1, relu=False,
-                                       x1=x1.data.view(n, h, w // f, -1) if x1 else None, out=z.view(n, h, w // f, -1))
-                    ng = xin.needs_grad or (x1 is not None and x1.needs_grad) or ins["w"] in trainable or (ins["bias"] in trainable)
+                        scale = self._tiled("fs2:" + ins["w"], sc, z.shape[3], f)
+                        bias = self._tiled("fb2:" + ins["w"], bs, z.shape[3], f)
+                        relu = fold["relu"]
+                    self._conv_fwd(xin.data.view(n, h, w // f, -1), wf, bias, z.shape[3] * f, 1, relu, z.view(n, h, w // f, -1),
+                                   x1=x1.data.view(n, h, w // f, -1) if x1 else None, scale=scale)
                     t = _T(z, needs_grad=ng)
                     t.folded = fold is not None
                     t.centered = shift is not None
@@ -531,34 +532,11 @@ class GraphEngine(EngineBase):
                 if shift is not None:
                     cb = self._buf("bc:" + ins["w"], (coutp,), torch.float32)
                     bias = torch.sub(bias, shift, out=cb) if bias is not None else torch.neg(shift, out=cb)
-                aux = None
-                stats = None
-                # folding is for pure inference: an eval-mode forward that will be back-propagated (model.eval() +
-                # loss.backward()) keeps z and runs the BatchNorm instruction so its backward has what it needs
-                fold = self._fold_bn.get(ins["out"]) if (not training and not save) else None
                 if fold is not None:
                     # eval mode: y = [relu](acc * s + b') straight from the conv epilogue; the BatchNorm instruction passes it on
-                    sc, bs = self._folded_bn(fold["bn"], params, params[ins["bias"]] if ins["bias"] else None, coutp)
-                    if ins["stride"] == 1 and low is not None:
-                        z = self._buf(ins["out"], (n, h, w, coutp))
-                        ops.decoder_conv_fprop(xin.data, low, wf, bs, coutp, relu=fold["relu"], out=z, up_out=up_out, scale=sc)
-                        x1.data = up_out
-                    elif ins["stride"] == 1:
-                        z = self._buf(ins["out"], (n, h, w, coutp))
-                        ops.conv_fprop_scaled(xin.data, wf, sc, bs, coutp, taps=ins["taps"], relu=fold["relu"],
-                                              x1=x1.data if x1 else None, out=z)
-                    elif ins["taps"] == 9:
-                        full = self._buf(ins["out"] + ":full", (n, h, w, coutp))
-                        ops.conv_fprop_scaled(xin.data, wf, sc, bs, coutp, taps=9, relu=fold["relu"], out=full)
-                        z = ops.subsample2(full, out=self._buf(ins["out"], (n, h // 2, w // 2, coutp)))
-                    else:
-                        xs = ops.subsample2(xin.data, out=self._buf(ins["out"] + ":xs", (n, h // 2, w // 2, xin.data.shape[3])))
-                        z = self._buf(ins["out"], (n, h // 2, w // 2, coutp))
-                        ops.conv_fprop_scaled(xs, wf, sc, bs, coutp, taps=1, relu=fold["relu"], out=z)
-                    t = _T(z)
-                    t.folded = True
-                    T[ins["out"]] = t
-                    continue
+                    scale, bias = self._folded_bn(fold["bn"], params, params[ins["bias"]] if ins["bias"] else None, coutp)
+                    relu = fold["relu"]
+                aux = stats = None
                 if ins["stride"] == 1:
                     z = self._buf(ins["out"], (n, h, w, coutp))
                     kdim = ins["taps"] * (xin.data.shape[3] + (low.shape[3] if low is not None else x1.data.shape[3] if x1 else 0))
@@ -566,25 +544,22 @@ class GraphEngine(EngineBase):
                         # the BatchNorm that reads this output takes its statistics from this conv's epilogue (no pass over
                         # z); one buffer per conv output: another conv may run before that BatchNorm (downsample branches)
                         stats = self._bn_stats("bnstat:" + ins["out"], n, h, w, coutp, ins["taps"], decoder=low is not None)
+                    self._conv_fwd(xin.data, wf, bias, coutp, ins["taps"], relu, z, x1=x1.data if x1 else None, low=low,
+                                   up_out=up_out, scale=scale, stats=stats)
                     if low is not None:
-                        ops.decoder_conv_fprop(xin.data, low, wf, bias, coutp, relu=ins["relu"], out=z, up_out=up_out,
-                                               stats=stats[0] if stats else None)
                         x1.data = up_out
-                    else:
-                        ops.conv_fprop(xin.data, wf, bias, coutp, taps=ins["taps"], relu=ins["relu"],
-                                       x1=x1.data if x1 else None, out=z, stats=stats[0] if stats else None)
                 elif ins["taps"] == 9:      # 3x3 stride 2 = stride-1 conv, keep even pixels
                     full = self._buf(ins["out"] + ":full", (n, h, w, coutp))
-                    ops.conv_fprop(xin.data, wf, bias, coutp, taps=9, relu=ins["relu"], out=full)
+                    self._conv_fwd(xin.data, wf, bias, coutp, 9, relu, full, scale=scale)
                     z = ops.subsample2(full, out=self._buf(ins["out"], (n, h // 2, w // 2, coutp)))
                 else:                        # 1x1 stride 2 = keep even pixels, then conv
                     aux = ops.subsample2(xin.data, out=self._buf(ins["out"] + ":xs", (n, h // 2, w // 2, xin.data.shape[3])))
                     z = self._buf(ins["out"], (n, h // 2, w // 2, coutp))
-                    ops.conv_fprop(aux, wf, bias, coutp, taps=1, relu=ins["relu"], out=z)
-                ng = xin.needs_grad or (x1 is not None and x1.needs_grad) or ins["w"] in trainable or (ins["bias"] in trainable)
+                    self._conv_fwd(aux, wf, bias, coutp, 1, relu, z, scale=scale)
                 t = _T(z, fused_relu=ins["relu"], needs_grad=ng)
                 t.aux = aux
                 t.stats = stats
+                t.folded = fold is not None
                 t.centered = shift is not None
                 T[ins["out"]] = t
             elif op == "bn":
@@ -667,21 +642,10 @@ class GraphEngine(EngineBase):
                 y = ops.upsample2x(xin.data, out=self._buf(ins["out"], (n, 2 * h, 2 * w, c)))
                 T[ins["out"]] = _T(y, needs_grad=xin.needs_grad)
             elif op == "head":
-                xin = T[ins["x"]]
-                if ops.act_dtype() == torch.float32:       # fp32 validation build: plain fp32 1x1 conv
-                    logits = ops.head_fwd(xin.data, self._head_weight(params, ins), params[ins["bias"]])
-                else:
-                    wf_head = ops.pack_head_fprop(self._head_weight(params, ins),
-                                                  wf=self._buf("head:wf", (64 * ops.head_groups(self.num_classes), 64)))
-                    logits = ops.head_fwd_tc(xin.data, wf_head, params[ins["bias"]], self.num_classes)
+                logits = self._head_fwd(T[ins["x"]].data, params, ins["w"], ins["bias"], ins.get("cin", 64))
         if save:
             self.saved = (T, (N, H, W), set(trainable))
         return logits
-
-    def _head_weight(self, params, ins):
-        cin = ins.get("cin", 64)
-        w = params[ins["w"]].reshape(self.num_classes, cin)
-        return w if cin == 64 else self._padded("head:w", w, (self.num_classes, 64))
 
     # ------------------------------------------------------------------ backward
     def _acc(self, t, g):
@@ -710,36 +674,9 @@ class GraphEngine(EngineBase):
             op = ins["op"]
             if op == "head":
                 xin = T[ins["x"]]
-                cin = ins.get("cin", 64)
-                wh = self._head_weight(params, ins)
-                C = self.num_classes
-                fw, fb = has(ins["w"]), has(ins["bias"])
                 g = self._buf("g:" + ins["x"], xin.data.shape) if xin.needs_grad else None
-                if dlogits.dtype == torch.bfloat16 and ops.act_dtype() == torch.bfloat16:
-                    dl = dlogits.contiguous()
-                    cz = 64 * ops.head_groups(C)       # [hi | lo] per group of 32 classes (ops.loss_bwd(nhwc64=True))
-                    if g is not None:
-                        wd_head = ops.pack_head_dgrad(wh, wd=self._buf("head:wd", (64, cz)))
-                        ops.conv_dgrad(dl, wd_head, 64, taps=1, mask=xin.data if xin.fused_relu else None, out0=g)
-                    if fw or fb:
-                        dw64 = self._buf("head:dw", (cz, 64, 1, 1), torch.float32)
-                        db64 = self._buf("head:db", (cz,), torch.float32)
-                        need = ops.lib().b2u_conv_wgrad_workspace(dl.shape[0], dl.shape[1], dl.shape[2], 64, cz, 1)
-                        ops.conv_wgrad(xin.data, dl, taps=1, dw=dw64, db=db64, ws=self._workspace("wgrad", need))
-                        if fw:
-                            ops.fold_head_groups(dw64, C, cin, grads[ins["w"]])
-                        if fb:
-                            ops.fold_head_groups(db64, C, cin, grads[ins["bias"]])
-                else:
-                    dl = dlogits.float().contiguous() if dlogits.dtype != torch.float32 else dlogits.contiguous()
-                    dwt = None
-                    if fw:
-                        dwt = grads[ins["w"]] if cin == 64 else self._buf("head:dwf", (C, 64, 1, 1), torch.float32)
-                    ops.head_bwd(dl, xin.data, wh, need_dx=g is not None, need_dw=fw or fb, relu_mask=xin.fused_relu, dx=g,
-                                 dw=dwt, db=grads[ins["bias"]] if fb else None,
-                                 ws=self._workspace("head", ops.lib().b2u_head_bwd_workspace_cls(C)))
-                    if fw and cin != 64:
-                        grads[ins["w"]].copy_(dwt[:, :cin])
+                self._head_bwd(dlogits, xin.data, params, grads, has, ins["w"], ins["bias"], ins.get("cin", 64), g,
+                               xin.data if xin.fused_relu else None)
                 if g is not None:
                     self._acc(xin, g)
                 ready(ins["w"], ins["bias"])
@@ -822,20 +759,12 @@ class GraphEngine(EngineBase):
                 res = T[ins["res"]] if ins["res"] else None
                 if t.grad is None:
                     continue
-                bnn, c = ins["bn"], ins["c"]
-                cp = zt.data.shape[3]
+                bnn = ins["bn"]
                 need_res = res is not None and res.needs_grad
                 gout = self._buf("g:" + ins["out"] + ">res", t.data.shape) if need_res else None
                 dz = self._buf("g:" + ins["z"], zt.data.shape)
-                direct = cp == c
-                dgam = grads[bnn + ".weight"] if (direct and has(bnn + ".weight")) else self._buf("dg:" + bnn, (cp,), torch.float32)
-                dbet = grads[bnn + ".bias"] if (direct and has(bnn + ".bias")) else self._buf("db:" + bnn, (cp,), torch.float32)
-                self._bn_bwd(t.grad, t.data, zt.data, t.aux, ins["relu"], dz, dgam, dbet, residual=res is not None, gout=gout)
-                if not direct:
-                    if has(bnn + ".weight"):
-                        grads[bnn + ".weight"].copy_(dgam[:c])
-                    if has(bnn + ".bias"):
-                        grads[bnn + ".bias"].copy_(dbet[:c])
+                self._bn_bwd(t.grad, t.data, zt.data, t.aux, ins["relu"], dz, grads, has, bnn, ins["c"], residual=res is not None,
+                             gout=gout)
                 ready(bnn + ".weight", bnn + ".bias")
                 if zt.needs_grad:
                     self._acc(zt, dz)
@@ -912,35 +841,8 @@ class GraphEngine(EngineBase):
                 xw = t.aux if (ins["stride"] == 2 and taps == 1) else xin.data          # wgrad's activation operand
                 c0p = xw.shape[3]
                 c1p = x1.data.shape[3] if x1 else 0
-                fused_db = (self.fused_db(coutp) and has(ins["w"]) and has(ins["bias"]) and taps == 9 and ins["out"] not in self._pre_bn
-                            and coutp == cout and c0p == c0r and c1p == c1r)
-                if has(ins["w"]):
-                    need = ops.lib().b2u_conv_wgrad_workspace(dz.shape[0], dz.shape[1], dz.shape[2], c0p + c1p, coutp, taps)
-                    ws = self._workspace("wgrad", need)
-                    if coutp == cout and c0p == c0r and c1p == c1r:
-                        ops.conv_wgrad(xw, dz, taps=taps, x1=x1.data if x1 else None, dw=grads[ins["w"]], ws=ws,
-                                       db=grads[ins["bias"]] if fused_db else None)
-                    else:       # padded operands: gradient of the padded weight, then keep the real rows/columns
-                        k = 3 if taps == 9 else 1
-                        tmp = self._buf("dw:" + ins["w"], (coutp, c0p + c1p, k, k), torch.float32)
-                        ops.conv_wgrad(xw, dz, taps=taps, x1=x1.data if x1 else None, dw=tmp, ws=ws)
-                        gw = grads[ins["w"]]
-                        gw[:, :c0r].copy_(tmp[:cout, :c0r])
-                        if ins["w"] in self.image_convs:          # + the lo half of the image split
-                            gw[:, :c0r].add_(tmp[:cout, c0r:2 * c0r])
-                        if c1r:
-                            gw[:, c0r:].copy_(tmp[:cout, c0p:c0p + c1r])
-                if has(ins["bias"]) and ins["out"] in self._pre_bn:
-                    # a bias in front of BatchNorm: the BN backward's dz sums to zero over the batch exactly, so the
-                    # gradient is 0 (the reference's autograd returns fp32 cancellation residue ~1e-8)
-                    grads[ins["bias"]].zero_()
-                elif has(ins["bias"]) and not fused_db:
-                    wsb = self._workspace("bias", ops.lib().b2u_bias_grad_workspace(coutp))
-                    if coutp == cout:
-                        ops.bias_grad(dz, db=grads[ins["bias"]], ws=wsb)
-                    else:
-                        tb = ops.bias_grad(dz, db=self._buf("dbias:" + ins["w"], (coutp,), torch.float32), ws=wsb)
-                        grads[ins["bias"]].copy_(tb[:cout])
+                self._conv_param_grads(xw, dz, grads, has, ins["w"], ins["bias"], cout, c0r, c1r, x1=x1.data if x1 else None,
+                                       taps=taps, pre_bn=ins["out"] in self._pre_bn, lo_half=ins["w"] in self.image_convs)
                 ready(ins["w"], ins["bias"])
                 need0, need1 = xin.needs_grad, (x1 is not None and x1.needs_grad)
                 if not (need0 or need1):
