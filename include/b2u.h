@@ -160,13 +160,16 @@ int b2u_bn_fwd_eval(const void* z, const void* residual, void* y, const float* g
                     const float* running_mean, const float* running_var, void* ws, size_t ws_bytes, long long P, int C,
                     float eps, int relu, void* stream);
 /* SyncBatchNorm building blocks (nn.SyncBatchNorm.convert_sync_batchnorm, train.py:335-336): the statistics and apply
- * passes as separate calls so the caller can all-reduce the [2][C] fp32 sums across ranks in between.  P_stat = rows over
- * all ranks.  b2u_bn_bwd_sums returns this rank's (dbeta, dgamma), which stay local (DDP averages them), like torch */
-int b2u_bn_sums(const void* z, float* sums, void* ws, size_t ws_bytes, long long P, int C, void* stream);
-int b2u_bn_fwd_train_sums(const void* z, const void* residual, void* y, const float* gamma, const float* beta,
-                          float* running_mean, float* running_var, float* save_mean, float* save_invstd, const float* sums,
-                          long long P_stat, void* ws, size_t ws_bytes, long long P, int C, float eps, float momentum, int relu,
-                          void* stream);
+ * passes as separate calls so the caller can exchange statistics across ranks in between.  Forward: b2u_bn_moments writes
+ * this rank's [2][C] fp32 (mean, biased variance); the caller all-gathers them into [world][2][C] and
+ * b2u_bn_fwd_train_moments combines them (every rank holds P rows).  Backward: the caller all-reduces the [2][C] sums of
+ * b2u_bn_bwd_sums; P_stat = rows over all ranks.  b2u_bn_bwd_sums returns this rank's (dbeta, dgamma), which stay local
+ * (DDP averages them), like torch */
+int b2u_bn_moments(const void* z, float* moments, void* ws, size_t ws_bytes, long long P, int C, void* stream);
+int b2u_bn_fwd_train_moments(const void* z, const void* residual, void* y, const float* gamma, const float* beta,
+                             float* running_mean, float* running_var, float* save_mean, float* save_invstd,
+                             const float* moments, int world, void* ws, size_t ws_bytes, long long P, int C, float eps,
+                             float momentum, int relu, void* stream);
 int b2u_bn_bwd_sums(const void* dy, const void* y, const void* z, const float* gamma, const float* beta, const float* save_mean,
                     const float* save_invstd, float* sums, void* ws, size_t ws_bytes, long long P, int C, int relu,
                     void* stream);

@@ -106,7 +106,7 @@ def test_validation_switch_routes_and_restores(b2u):
         with pytest.raises(_lib.B2UError):
             v.b2u_head_fwd_tc
         with pytest.raises(_lib.B2UError):
-            v.b2u_bn_sums                   # SyncBatchNorm building blocks are product-only
+            v.b2u_bn_moments                # SyncBatchNorm building blocks are product-only
     finally:
         ops.set_validation_fp32(False)
     assert not _lib.validation_fp32() and ops.act_dtype() == torch.bfloat16

@@ -129,8 +129,8 @@ def tile_sums(z, rows, tile_w=16, tile_h=8):
 
 # ------------------------------------------------------------------------------------------------- conv forward
 CONV_CASES = [
-    # N, H, W, C0, C1, Cout, taps.  Observed err / bound: y and z 0.96-0.99 (bf16 rounding), statistics rows <= 0.056,
-    # totals <= 5e-4.
+    # N, H, W, C0, C1, Cout, taps.  Observed err / bound: y, z and the scaled y 0.96-0.99 (bf16 rounding), statistics
+    # rows <= 0.056, totals <= 5e-4.
     (8, 256, 256, 64, 0, 64, 9),        # 1024 tiles with four stacked M tiles, 4096 with one
     (8, 128, 128, 128, 128, 128, 9),    # two sources; N tile 128 and 64 (two N tiles: bias parity)
     (8, 64, 64, 512, 0, 512, 9),        # N tiles 256 / 128 / 64: 2..8 N tiles per M tile
@@ -151,6 +151,19 @@ def _conv_case(b2u, dev, N, H, W, C0, C1, Cout, taps, seed):
     return x, x0, x1, w.to(BF), b, wf, wd
 
 
+def _folded_bn_coeffs(C, dev, seed):
+    """Per-channel scale s (|s| in [0.5, 1.5], both signs) and shift b' of a folded eval-mode BatchNorm."""
+    g = _gen(dev, seed)
+    s = (torch.rand((C,), generator=g, device=dev) + 0.5) * torch.where(torch.arange(C, device=dev) % 2 == 1, -1.0, 1.0)
+    return s, torch.randn((C,), generator=g, device=dev)
+
+
+def _scaled_ref(conv, A, s, bp):
+    """fp64 relu(s conv + b') of an NCHW conv result and its magnitude bound |s| A + |b'|."""
+    sh = (-1, 1, 1)
+    return (s.double().view(sh) * conv + bp.double().view(sh)).relu(), s.double().abs().view(sh) * A + bp.double().abs().view(sh)
+
+
 @pytest.mark.parametrize("N,H,W,C0,C1,Cout,taps", CONV_CASES)
 def test_conv_fprop_at_scale(b2u, cuda_device, N, H, W, C0, C1, Cout, taps):
     """conv + bias + ReLU in every tiling variant the launcher can pick, and the statistics epilogue (per-tile rows)."""
@@ -165,6 +178,14 @@ def test_conv_fprop_at_scale(b2u, cuda_device, N, H, W, C0, C1, Cout, taps):
         assert ops.conv_stat_rows(N, H, W, Cout, taps, bn) * n_tiles >= 3 * sms, f"variant {bn:#x} is not multi-tile"
         y = ops.conv_fprop(x0, wf, b, Cout, taps=taps, relu=True, x1=x1, bn=bn)
         check_bf16(f"fprop {N}x{H}x{W} {C0}+{C1}->{Cout} t{taps} bn={bn:#x}", y, ref, A)
+    # folded eval-mode BatchNorm in the epilogue: y = relu(s conv(x) + b'), s of both signs (a ReLU taken before the
+    # scale would pass every channel with s > 0)
+    s, bp = _folded_bn_coeffs(Cout, dev, 16)
+    ref_s, A_s = _scaled_ref(ref_z - b.double().view(-1, 1, 1), A, s, bp)
+    for bn in variants:
+        y = ops.conv_fprop_scaled(x0, wf, s, bp, Cout, taps=taps, relu=True, x1=x1, bn=bn)
+        check_bf16(f"fprop scaled {N}x{H}x{W} {C0}+{C1}->{Cout} t{taps} bn={bn:#x}", y, ref_s, A_s)
+    del ref_s, A_s
     for bn in (0, 1 << 16):
         rows = ops.conv_stat_rows(N, H, W, Cout, taps, bn)
         st = torch.full((rows * 2 * Cout,), float("nan"), device=dev)
@@ -178,6 +199,29 @@ def test_conv_fprop_at_scale(b2u, cuda_device, N, H, W, C0, C1, Cout, taps):
         check_sum(name + " rows sum", got[:, 0], s, a)
         check_sum(name + " rows sumsq", got[:, 1], q, q)
         check_sum(name + " total", got.double().sum(0)[0], s.sum(0), a.sum(0))
+
+
+def test_decoder_conv_scaled_at_scale(b2u, cuda_device):
+    """b2u_decoder_conv_fprop with a folded eval-mode BatchNorm (scale=...), the inference form of every BatchNorm decoder
+    stage: relu(s conv([skip, upsample2x(low)]) + b') against fp64 on the up-sampled bf16 operand the kernel interpolates
+    (bit-identical to b2u_upsample2x_fwd), s of both signs, in every N tile and M-tile stacking of a multi-tile launch.
+    Observed err / bound: <= 0.98 (bf16 rounding)."""
+    ops, dev, sms = b2u.ops, cuda_device, _sms(b2u)
+    N, H, W, C0, C1, Cout = 8, 128, 128, 128, 128, 128
+    g = _gen(dev, 17)
+    skip = _bf((N, H, W, C0), g, dev)
+    low = _bf((N, H // 2, W // 2, C1), g, dev)
+    w = torch.randn((Cout, C0 + C1, 3, 3), generator=g, device=dev) / ((C0 + C1) * 9) ** 0.5
+    wf, _ = ops.pack_weights(w)
+    x = torch.cat([skip, ops.upsample2x(low)], -1)
+    wb = w.to(BF)
+    s, bp = _folded_bn_coeffs(Cout, dev, 18)
+    ref_s, A_s = _scaled_ref(conv_ref(x, wb), conv_ref(x, wb, absolute=True), s, bp)
+    for bn in (0, 1 << 16, 64, (1 << 16) | 64):
+        units = ops.conv_stat_rows(N, H, W, Cout, 9, bn | (1 << 18)) * (Cout // ((bn & 0xffff) or default_bn(Cout)))
+        assert units >= 3 * sms, f"variant {bn:#x} is not multi-tile"
+        y = ops.decoder_conv_fprop(skip, low, wf, bp, Cout, relu=True, scale=s, bn=bn)
+        check_bf16(f"decoder scaled {N}x{H}x{W} {C0}+{C1}->{Cout} bn={bn:#x}", y, ref_s, A_s)
 
 
 # ------------------------------------------------------------------------------------------------- conv data gradient
@@ -432,6 +476,252 @@ def test_batchnorm_epilogue_statistics_at_scale(b2u, cuda_device):
         allowed = 2e-5 + (0.0 if centered else 2e-7) * ratio.double() ** 2
         assert (e_var <= allowed).all(), (e_var / allowed).max().item()
         assert ((rv.double() - (0.9 + 0.1 * v_ref * P / (P - 1))).abs() <= 0.1 * allowed * v_ref + 2e-6).all()
+
+
+# ------------------------------------------------------------------------------------------------- SyncBatchNorm
+BN_BLOCKS = 296            # bn.cu kBnBlocks: the column-sum grid (2 blocks of 256 threads per SM of a B200)
+
+
+def _colsum_passes(P, C, unroll):
+    """Grid-stride passes of the last, least loaded block of bn_colsum_kernel over P rows (0: some blocks get no row).
+    unroll: kBnUnroll, 8 for the forward statistics, 4 for the backward sums."""
+    rows = 256 // min(C // 8, 256)
+    first = (BN_BLOCKS - 1) * rows
+    return 0 if first >= P else -(-(P - first) // (unroll * BN_BLOCKS * rows))
+
+
+def _bn_ws(ops, C, dev):
+    return torch.empty(ops.lib().b2u_bn_workspace(C), dtype=torch.uint8, device=dev)
+
+
+def _sync_bn_fwd(ops, z, R, gamma, beta, rm0, rv0, residual=None):
+    """SyncBatchNorm forward on R emulated ranks holding one shard of whole images each: every rank's moments land in its
+    slot of one [R][2][C] buffer (what the all-gather delivers), then every rank applies with its own running statistics.
+    Returns the stitched y and, per rank, (save_mean, save_invstd, running_mean, running_var)."""
+    lib, ptr, check, sp = ops.lib(), ops.ptr, ops.check, ops.stream_ptr()
+    C = z.shape[-1]
+    zs = z.view(R, -1, C)
+    res = residual.view(R, -1, C) if residual is not None else [None] * R
+    Pr = zs.shape[1]
+    ws = _bn_ws(ops, C, z.device)
+    moments = torch.full((R, 2, C), float("nan"), device=z.device)
+    for r in range(R):
+        check(lib.b2u_bn_moments(ptr(zs[r]), ptr(moments[r]), ptr(ws), ws.numel(), Pr, C, sp))
+    y = torch.empty_like(z)
+    ys = y.view(R, -1, C)
+    per_rank = []
+    for r in range(R):
+        mean, invstd = torch.empty(C, device=z.device), torch.empty(C, device=z.device)
+        rm, rv = rm0.clone(), rv0.clone()
+        check(lib.b2u_bn_fwd_train_moments(ptr(zs[r]), ptr(res[r]), ptr(ys[r]), ptr(gamma), ptr(beta), ptr(rm), ptr(rv), ptr(mean),
+                                           ptr(invstd), ptr(moments), R, ptr(ws), ws.numel(), Pr, C, 1e-5, 0.1, 1, sp))
+        per_rank.append((mean, invstd, rm, rv))
+    return y, per_rank
+
+
+def _sync_bn_bwd(ops, dy, y, z, R, gamma, beta, mean, invstd):
+    """SyncBatchNorm backward on R emulated ranks: each rank's (sum g, sum g xhat), their sum (the all-reduce), then each
+    rank's dz and gout.  y=None recomputes the ReLU mask from z.  Returns (dz, gout, per-rank sums [R][2][C])."""
+    lib, ptr, check, sp = ops.lib(), ops.ptr, ops.check, ops.stream_ptr()
+    C = z.shape[-1]
+    dys, zs = dy.view(R, -1, C), z.view(R, -1, C)
+    yv = y.view(R, -1, C) if y is not None else [None] * R
+    Pr = zs.shape[1]
+    ws = _bn_ws(ops, C, z.device)
+    sums = torch.full((R, 2, C), float("nan"), device=z.device)
+    for r in range(R):
+        check(lib.b2u_bn_bwd_sums(ptr(dys[r]), ptr(yv[r]), ptr(zs[r]), ptr(gamma), ptr(beta), ptr(mean), ptr(invstd), ptr(sums[r]),
+                                  ptr(ws), ws.numel(), Pr, C, 1, sp))
+    total = sums.sum(0)
+    dz, gout = torch.full_like(z, float("nan")), torch.full_like(z, float("nan"))
+    dzs, gs = dz.view(R, -1, C), gout.view(R, -1, C)
+    for r in range(R):
+        check(lib.b2u_bn_bwd_apply_sums(ptr(dys[r]), ptr(yv[r]), ptr(zs[r]), ptr(gamma), ptr(beta), ptr(mean), ptr(invstd), ptr(dzs[r]),
+                                        ptr(gs[r]), ptr(total), R * Pr, ptr(ws), ws.numel(), Pr, C, 1, sp))
+    return dz, gout, sums
+
+
+def _bn_stat_errors(tag, mean, invstd, z, ratio):
+    """Per-shift errors of the statistics a BatchNorm normalised with (mean in standard deviations, var and invstd relative),
+    printed; asserted against the one-GPU bounds."""
+    m_ref, v_ref = _bn_ref_stats(z)
+    e_mean = (mean.double() - m_ref).abs() / v_ref.sqrt()
+    e_var = (invstd.double() ** -2 - 1e-5 - v_ref).abs() / v_ref
+    is_ref = (v_ref + 1e-5).rsqrt()
+    e_is = (invstd.double() - is_ref).abs() / is_ref
+    for r in sorted(set(ratio.tolist())):
+        sel = ratio == r
+        print(f"[{tag}] mean/std={r:+.0f}: mean err/std {e_mean[sel].max().item():.2e}  var rel {e_var[sel].max().item():.2e}  "
+              f"invstd rel {e_is[sel].max().item():.2e}")
+    assert e_mean.max().item() <= 2e-5, f"{tag}: mean err / std {e_mean.max().item():.3g}"
+    assert e_var.max().item() <= 2e-5 and e_is.max().item() <= 2e-5, f"{tag}: var rel {e_var.max().item():.3g}"
+    return m_ref, v_ref
+
+
+def _bn_fwd_ref(zd, mean, invstd, gamma, beta, residual=None):
+    """fp64 y = relu(gamma (z - mean) invstd + beta [+ residual]) of NCHW zd, and the magnitude A of its fp32 evaluation."""
+    sh = (-1, 1, 1)
+    m, s = mean.double().view(sh), invstd.double().view(sh)
+    gd, bd = gamma.double().view(sh), beta.double().view(sh)
+    v = gd * (zd - m) * s + bd
+    A = gd.abs() * (zd.abs() + m.abs()) * s + bd.abs()
+    if residual is not None:
+        rd = residual.double().permute(0, 3, 1, 2)
+        v, A = v + rd, A + rd.abs()
+    return v.relu(), A
+
+
+def _bn_bwd_check(tag, dz, gout, sums, dy, y, z, R, gamma, mean, invstd):
+    """dz and gout of the whole batch element by element (ReLU decisions: the kernel's own y > 0), and each rank's
+    (dbeta, dgamma) against fp64 sums over that rank's shard."""
+    N, C = z.shape[0], z.shape[-1]
+    P = z.numel() // C
+    sh = (-1, 1, 1)
+    keep = (y > 0).permute(0, 3, 1, 2)
+    gm = dy.double().permute(0, 3, 1, 2) * keep
+    assert torch.equal(gout, dy * (y > 0)), f"{tag}: gout is not the ReLU-masked dy"
+    xk = (z.double().permute(0, 3, 1, 2) - mean.double().view(sh)) * invstd.double().view(sh)
+    gx = gm * xk
+    n = N // R
+    for r in range(R):
+        part = slice(r * n, (r + 1) * n)
+        check_sum(f"{tag} rank {r} dbeta", sums[r, 0], gm[part].sum((0, 2, 3)), gm[part].abs().sum((0, 2, 3)))
+        check_sum(f"{tag} rank {r} dgamma", sums[r, 1], gx[part].sum((0, 2, 3)), gx[part].abs().sum((0, 2, 3)))
+    ref_db, ref_dg = gm.sum((0, 2, 3)), gx.sum((0, 2, 3))
+    a = (gamma.double() * invstd.double()).view(sh)
+    ref_dz = a * (gm - (ref_db / P).view(sh) - xk * (ref_dg / P).view(sh))
+    A_dz = a.abs() * (gm.abs() + (ref_db.abs() / P).view(sh) + xk.abs() * (ref_dg.abs() / P).view(sh))
+    check_bf16(f"{tag} dz", dz, ref_dz, A_dz)
+
+
+# N, H, W, C, R emulated ranks, least grid-stride passes per block of both column-sum kernels (0: a regime of idle blocks).
+# Observed err / bound: y, dz <= 0.992 (bf16 rounding); per-rank dgamma <= 0.031, dbeta <= 0.0038.  Statistics at every
+# shift and R: mean err <= 4.9e-6 std, var rel <= 8.0e-7, invstd rel <= 4.0e-7 (all-reduced raw fp32 sums, the earlier
+# design: var rel 1.2e-2 at 64 std with R = 1, 3.5e-4..8.6e-4 with R = 2..8).
+SYNC_BN_CASES = [
+    (16, 512, 512, 64, 1, 2),
+    (16, 512, 512, 64, 2, 2),
+    (16, 512, 512, 64, 8, 2),
+    (12, 256, 256, 256, 3, 2),
+    (8, 32, 32, 2048, 2, 2),          # one row per block and pass: the forward's last block takes exactly two passes
+    (8, 3, 5, 2560, 8, 0),            # 15 rows per rank: 281 of 296 blocks idle; C/8 = 320, a second channel chunk of 64
+]
+
+
+@pytest.mark.parametrize("N,H,W,C,R,passes", SYNC_BN_CASES)
+def test_sync_batchnorm_emulated_ranks(b2u, cuda_device, N, H, W, C, R, passes):
+    """SyncBatchNorm's four entry points on R ranks emulated on one GPU (shards of whole images), stitched together,
+    against fp64 BatchNorm over the whole batch: the statistics to the one-GPU bounds at channel means up to 64 standard
+    deviations, bit-identical on every rank; the running statistics with the unbiased factor of the global row count;
+    y with and without a residual; dz and gout element by element with the ReLU mask read from y and recomputed from z;
+    each rank's local dgamma / dbeta."""
+    ops, dev = b2u.ops, cuda_device
+    assert N % R == 0
+    P, Pr = N * H * W, N // R * H * W
+    if passes:
+        assert min(_colsum_passes(Pr, C, 8), _colsum_passes(Pr, C, 4)) >= passes
+    else:
+        assert Pr < BN_BLOCKS and C // 8 > 256 and (C // 8) % 256 != 0
+    z, ratio = _bn_data(dev, N, H, W, C, 11)
+    g = _gen(dev, 12)
+    sign = torch.where(torch.arange(C, device=dev) % 3 == 2, -1.0, 1.0)
+    gamma = (1 + 0.2 * torch.randn((C,), generator=g, device=dev)) * sign
+    beta = 0.1 * torch.randn((C,), generator=g, device=dev)
+    rm0, rv0 = 0.1 * torch.randn((C,), generator=g, device=dev), torch.rand((C,), generator=g, device=dev) + 0.5
+    residual = _bf((N, H, W, C), g, dev)
+    dy = _bf((N, H, W, C), g, dev)
+    tag = f"sync bn {N}x{H}x{W}x{C} R={R}"
+    y, ranks = _sync_bn_fwd(ops, z, R, gamma, beta, rm0, rv0)
+    mean, invstd, rm, rv = ranks[0]
+    for r, t in enumerate(ranks[1:], 1):
+        for a, b, what in zip(t, ranks[0], ("save_mean", "save_invstd", "running_mean", "running_var")):
+            assert torch.equal(a.view(torch.int32), b.view(torch.int32)), f"{tag}: {what} of rank {r} differs from rank 0"
+    m_ref, v_ref = _bn_stat_errors(tag, mean, invstd, z, ratio)
+    want_rv = 0.9 * rv0.double() + 0.1 * v_ref * P / (P - 1)
+    assert ((rv.double() - want_rv).abs() / want_rv).max().item() <= 2e-6
+    assert torch.allclose(rm.double(), 0.9 * rm0.double() + 0.1 * m_ref, rtol=1e-6, atol=1e-6 * v_ref.sqrt().max().item())
+    zd = z.double().permute(0, 3, 1, 2)
+    ref_y, A_y = _bn_fwd_ref(zd, m_ref, (v_ref + 1e-5).rsqrt(), gamma, beta)
+    check_bf16(f"{tag} y", y, ref_y, A_y)
+    del ref_y, A_y
+    y_res, ranks_res = _sync_bn_fwd(ops, z, R, gamma, beta, rm0, rv0, residual=residual)
+    assert torch.equal(ranks_res[0][1], invstd)
+    ref_y, A_y = _bn_fwd_ref(zd, m_ref, (v_ref + 1e-5).rsqrt(), gamma, beta, residual)
+    check_bf16(f"{tag} y residual", y_res, ref_y, A_y)
+    del ref_y, A_y, zd
+    # backward: ReLU mask recomputed from z (no residual), then read from y (residual added before the ReLU)
+    dz, gout, sums = _sync_bn_bwd(ops, dy, None, z, R, gamma, beta, mean, invstd)
+    _bn_bwd_check(f"{tag} bwd", dz, gout, sums, dy, y, z, R, gamma, mean, invstd)
+    dz, gout, sums = _sync_bn_bwd(ops, dy, y_res, z, R, gamma, beta, mean, invstd)
+    _bn_bwd_check(f"{tag} bwd residual", dz, gout, sums, dy, y_res, z, R, gamma, mean, invstd)
+
+
+# ------------------------------------------------------------------------------------------------- eval-mode BatchNorm
+# Observed err / bound: y, dz <= 0.992 (bf16 rounding); dgamma <= 0.0025, dbeta <= 8e-4.
+@pytest.mark.parametrize("N,H,W,C", BN_CASES)
+def test_batchnorm_eval_backward_at_scale(b2u, cuda_device, N, H, W, C):
+    """model.eval() + backward: y = relu(bn(z) [+ residual]) from the running statistics, then ops.bn_bwd_eval against
+    dz = gamma / sqrt(rv + eps) g (no batch-mean terms), dbeta = sum g, dgamma = sum g (z - rm) / sqrt(rv + eps), with g
+    the ReLU-masked dy; every fifth channel has rv = 1e-4, where eps moves invstd by 5 %."""
+    ops, dev = b2u.ops, cuda_device
+    z, _ = _bn_data(dev, N, H, W, C, 13)
+    g = _gen(dev, 14)
+    m_ref, v_ref = _bn_ref_stats(z)
+    gamma = (1 + 0.2 * torch.randn((C,), generator=g, device=dev)) * torch.where(torch.arange(C, device=dev) % 3 == 2, -1.0, 1.0)
+    beta = 0.1 * torch.randn((C,), generator=g, device=dev)
+    rm = (m_ref + 0.2 * v_ref.sqrt() * torch.randn((C,), generator=g, device=dev, dtype=F64)).float()
+    rv = (v_ref * (torch.rand((C,), generator=g, device=dev, dtype=F64) + 0.5)).float()
+    rv[::5] = 1e-4
+    residual = _bf((N, H, W, C), g, dev)
+    dy = _bf((N, H, W, C), g, dev)
+    sh = (-1, 1, 1)
+    is_ref = (rv.double() + 1e-5).rsqrt()
+    for res in (None, residual):
+        tag = f"bn eval bwd {N}x{H}x{W}x{C} residual={res is not None}"
+        y = ops.bn_fwd_eval(z, gamma, beta, rm, rv, relu=True, residual=res)
+        ref_y, A_y = _bn_fwd_ref(z.double().permute(0, 3, 1, 2), rm, is_ref, gamma, beta, res)
+        check_bf16(tag + " y", y, ref_y, A_y)
+        del ref_y, A_y
+        gout = torch.full_like(z, float("nan")) if res is not None else None
+        dz, dgam, dbet = ops.bn_bwd_eval(dy, y, z, gamma, beta, rm, rv, relu=True, gout=gout)
+        gm = dy.double().permute(0, 3, 1, 2) * (y > 0).permute(0, 3, 1, 2)
+        if gout is not None:
+            assert torch.equal(gout, dy * (y > 0)), f"{tag}: gout is not the ReLU-masked dy"
+        a = (gamma.double() * is_ref).view(sh)
+        check_bf16(tag + " dz", dz, a * gm, a.abs() * gm.abs())
+        gx = gm * (z.double().permute(0, 3, 1, 2) - rm.double().view(sh)) * is_ref.view(sh)
+        check_sum(tag + " dbeta", dbet, gm.sum((0, 2, 3)), gm.abs().sum((0, 2, 3)))
+        check_sum(tag + " dgamma", dgam, gx.sum((0, 2, 3)), gx.abs().sum((0, 2, 3)))
+        del gm, gx
+
+
+def test_bn_fold_against_float64(b2u, cuda_device):
+    """b2u_bn_fold (eval BatchNorm folded into the conv before it): scale = gamma / sqrt(rv + eps) and
+    bias = (conv_bias - rm) scale + beta to fp32 rounding, with gamma of both signs, rv from 1e-6 (eps dominates) to 10, and
+    each of gamma / beta / conv_bias absent.  Observed err / bound <= 0.52."""
+    ops, dev = b2u.ops, cuda_device
+    C = 1000                                  # not a multiple of the 128-thread block
+    g = _gen(dev, 15)
+    gamma = torch.randn((C,), generator=g, device=dev)
+    beta = torch.randn((C,), generator=g, device=dev)
+    rm = 3 * torch.randn((C,), generator=g, device=dev)
+    rv = 10 ** (7 * torch.rand((C,), generator=g, device=dev) - 6)
+    rv[:4] = torch.tensor([1e-6, 2e-6, 1e-5, 1e-4])
+    cb = torch.randn((C,), generator=g, device=dev)
+    assert (gamma < 0).any() and (rv < 1e-5).sum() >= 20
+    for drop in (None, "gamma", "beta", "conv_bias"):
+        ga, bt, b0 = (None if drop == "gamma" else gamma), (None if drop == "beta" else beta), (None if drop == "conv_bias" else cb)
+        s, b = ops.bn_fold(ga, bt, rm, rv, b0)
+        gd = ga.double() if ga is not None else torch.ones(C, dtype=F64, device=dev)
+        bd = bt.double() if bt is not None else torch.zeros(C, dtype=F64, device=dev)
+        cd = b0.double() if b0 is not None else torch.zeros(C, dtype=F64, device=dev)
+        ref_s = gd / (rv.double() + 1e-5).sqrt()
+        ref_b = (cd - rm.double()) * ref_s + bd
+        e_s = ((s.double() - ref_s).abs() / (2.0 ** -21 * ref_s.abs() + 1e-300)).max().item()
+        e_b = ((b.double() - ref_b).abs() / (2.0 ** -21 * ((cd - rm.double()).abs() * ref_s.abs() + bd.abs()) + 1e-300)).max().item()
+        _note(f"bn_fold without {drop} scale", e_s)
+        _note(f"bn_fold without {drop} bias", e_b)
+        assert e_s <= 1.0 and e_b <= 1.0, drop
 
 
 # ------------------------------------------------------------------------------------------------- grid-stride reductions

@@ -10,6 +10,7 @@ shows 2.8e-2; torch's own bf16 autocast 1.7e-2, SURVEY.md Appendix B), so that f
 storage model (<= 1e-2) and must not exceed 1.5x the model's own distance from fp32."""
 import os
 import re
+import socket
 
 import numpy as np
 import pytest
@@ -875,6 +876,102 @@ def test_sync_batchnorm_two_gpus(cuda_device):
         # two bf16 runs with different summation orders: the tensors next to the output agree closely; through the 14
         # BatchNorm backward passes the difference is amplified like any other bf16 rounding (see DESIGN.md section 5)
         assert near <= 2e-2 and gerr <= 0.15
+
+
+def _free_port():
+    s = socket.socket()
+    s.bind(("127.0.0.1", 0))
+    p = s.getsockname()[1]
+    s.close()
+    return p
+
+
+def _syncbn_gloo_worker(rank, world, port, z, dy, residual, gamma, beta, rm, rv, out_dir):
+    import torch.distributed as dist
+    import unet_pytorch_b200 as b2u
+    os.environ["MASTER_ADDR"] = "127.0.0.1"; os.environ["MASTER_PORT"] = str(port)
+    dist.init_process_group("gloo", rank=rank, world_size=world)
+    try:
+        dev = torch.device("cuda:0")
+        n = z.shape[0] // world
+        mine = slice(rank * n, (rank + 1) * n)
+        zr, dyr, g, bt = z[mine].to(dev), dy[mine].to(dev), gamma.to(dev), beta.to(dev)
+        res = {}
+        for tag, rr in (("plain", None), ("residual", residual[mine].to(dev))):
+            rmr, rvr = rm.to(dev), rv.to(dev)
+            y, mean, invstd = b2u.ops.bn_fwd_train_sync(zr, g, bt, rmr, rvr, dist.group.WORLD, residual=rr)
+            gout = torch.empty_like(zr)
+            dz, dgam, dbet = b2u.ops.bn_bwd_sync(dyr, y if rr is not None else None, zr, g, mean, invstd, dist.group.WORLD,
+                                                 gout=gout, beta=bt)
+            res[tag] = {k: v.cpu() for k, v in dict(y=y, mean=mean, invstd=invstd, rm=rmr, rv=rvr, dz=dz, gout=gout,
+                                                     dgamma=dgam, dbeta=dbet).items()}
+        torch.save(res, os.path.join(out_dir, f"rank{rank}.pt"))
+    finally:
+        dist.destroy_process_group()
+
+
+def test_sync_batchnorm_wrappers_gloo_one_gpu(b2u, cuda_device, tmp_path):
+    """ops.bn_fwd_train_sync / ops.bn_bwd_sync in a two-process gloo group whose ranks share cuda:0, half a batch each:
+    the collectives of the wrappers (all-gather of the moments, all-reduce of the backward sums, CUDA tensors through
+    gloo) give what ops.bn_fwd_train / ops.bn_bwd give on the whole batch, both held to fp64 BatchNorm with the bounds of
+    test_kernels_at_scale_gpu.py, at channel means up to 64 standard deviations."""
+    import torch.multiprocessing as mp
+    from test_kernels_at_scale_gpu import _bn_data, _bn_fwd_ref, _bn_stat_errors, check_bf16, check_sum
+    dev = cuda_device
+    N, H, W, C = 8, 64, 64, 128
+    P = N * H * W
+    z, ratio = _bn_data(dev, N, H, W, C, 19)
+    g = torch.Generator(device=dev).manual_seed(20)
+    gamma = (1 + 0.2 * torch.randn((C,), generator=g, device=dev)) * torch.where(torch.arange(C, device=dev) % 3 == 2, -1.0, 1.0)
+    beta = 0.1 * torch.randn((C,), generator=g, device=dev)
+    rm0, rv0 = 0.1 * torch.randn((C,), generator=g, device=dev), torch.rand((C,), generator=g, device=dev) + 0.5
+    residual = torch.randn((N, H, W, C), generator=g, device=dev).to(torch.bfloat16)
+    dy = torch.randn((N, H, W, C), generator=g, device=dev).to(torch.bfloat16)
+    mp.spawn(_syncbn_gloo_worker, args=(2, _free_port(), z.cpu(), dy.cpu(), residual.cpu(), gamma.cpu(), beta.cpu(), rm0.cpu(),
+                                        rv0.cpu(), str(tmp_path)), nprocs=2, join=True)
+    ranks = [torch.load(tmp_path / f"rank{r}.pt") for r in range(2)]
+    zd = z.double().permute(0, 3, 1, 2)
+    sh = (-1, 1, 1)
+    for tag, res in (("plain", None), ("residual", residual)):
+        got = {k: [ranks[r][tag][k].to(dev) for r in range(2)] for k in ranks[0][tag]}
+        for k in ("mean", "invstd", "rm", "rv"):
+            assert torch.equal(got[k][0], got[k][1]), f"{tag}: {k} differs between the ranks"
+        rm, rv = rm0.clone(), rv0.clone()
+        y1, mean1, invstd1 = b2u.ops.bn_fwd_train(z, gamma, beta, rm, rv, residual=res)
+        m_ref, v_ref = _bn_stat_errors(f"gloo sync bn {tag}", got["mean"][0], got["invstd"][0], z, ratio)
+        _bn_stat_errors(f"one GPU bn {tag}", mean1, invstd1, z, ratio)
+        want_rv = 0.9 * rv0.double() + 0.1 * v_ref * P / (P - 1)
+        for r_v in (got["rv"][0], rv):
+            assert ((r_v.double() - want_rv).abs() / want_rv).max().item() <= 2e-6
+        for r_m in (got["rm"][0], rm):
+            assert torch.allclose(r_m.double(), 0.9 * rm0.double() + 0.1 * m_ref, rtol=1e-6, atol=1e-6 * v_ref.sqrt().max().item())
+        ref_y, A_y = _bn_fwd_ref(zd, m_ref, (v_ref + 1e-5).rsqrt(), gamma, beta, res)
+        y_sync = torch.cat(got["y"])
+        check_bf16(f"gloo sync bn {tag} y", y_sync, ref_y, A_y)
+        check_bf16(f"one GPU bn {tag} y", y1, ref_y, A_y)
+        # backward from each path's own forward (ReLU mask from z without a residual, from y with one)
+        gout1 = torch.empty_like(z)
+        dz1, dg1, db1 = b2u.ops.bn_bwd(dy, y1 if res is not None else None, z, gamma, mean1, invstd1, gout=gout1, beta=beta)
+        for name, y_, dz_, gout_, mean_, invstd_ in (("gloo sync", y_sync, torch.cat(got["dz"]), torch.cat(got["gout"]),
+                                                      got["mean"][0], got["invstd"][0]),
+                                                     ("one GPU", y1, dz1, gout1, mean1, invstd1)):
+            assert torch.equal(gout_, dy * (y_ > 0)), f"{name} {tag}: gout"
+            gm = dy.double().permute(0, 3, 1, 2) * (y_ > 0).permute(0, 3, 1, 2)
+            xk = (zd - mean_.double().view(sh)) * invstd_.double().view(sh)
+            ref_db, ref_dg = gm.sum((0, 2, 3)), (gm * xk).sum((0, 2, 3))
+            a = (gamma.double() * invstd_.double()).view(sh)
+            ref_dz = a * (gm - (ref_db / P).view(sh) - xk * (ref_dg / P).view(sh))
+            A_dz = a.abs() * (gm.abs() + (ref_db.abs() / P).view(sh) + xk.abs() * (ref_dg.abs() / P).view(sh))
+            check_bf16(f"{name} bn {tag} dz", dz_, ref_dz, A_dz)
+            if name == "one GPU":
+                check_sum(f"one GPU bn {tag} dbeta", db1, ref_db, gm.abs().sum((0, 2, 3)))
+                check_sum(f"one GPU bn {tag} dgamma", dg1, ref_dg, (gm * xk).abs().sum((0, 2, 3)))
+            else:       # the affine gradients stay local to each rank, like nn.SyncBatchNorm's
+                for r in range(2):
+                    part = slice(r * N // 2, (r + 1) * N // 2)
+                    check_sum(f"gloo sync bn {tag} rank {r} dbeta", got["dbeta"][r], gm[part].sum((0, 2, 3)), gm[part].abs().sum((0, 2, 3)))
+                    check_sum(f"gloo sync bn {tag} rank {r} dgamma", got["dgamma"][r], (gm * xk)[part].sum((0, 2, 3)),
+                              (gm * xk)[part].abs().sum((0, 2, 3)))
 
 
 def _dp_trainer_worker(rank, world, port, sd, imgs, pngs, C, out):

@@ -32,8 +32,8 @@ SIGNATURES = {
     "b2u_letterbox_workspace": (SZ, [P, I, I, I]),
     "b2u_letterbox_bicubic": (I, [P, I, P, I, I, P, SZ, P]),
     "b2u_conv_fprop": (I, [P, I, P, I, P, P, P, I, I, I, I, I, I, I, P]),
-    "b2u_bn_sums": (I, [P, P, P, SZ, LL, I, P]),
-    "b2u_bn_fwd_train_sums": (I, [P, P, P, P, P, P, P, P, P, P, LL, P, SZ, LL, I, F, F, I, P]),
+    "b2u_bn_moments": (I, [P, P, P, SZ, LL, I, P]),
+    "b2u_bn_fwd_train_moments": (I, [P, P, P, P, P, P, P, P, P, P, I, P, SZ, LL, I, F, F, I, P]),
     "b2u_bn_bwd_sums": (I, [P, P, P, P, P, P, P, P, P, SZ, LL, I, I, P]),
     "b2u_bn_bwd_apply_sums": (I, [P, P, P, P, P, P, P, P, P, P, LL, P, SZ, LL, I, I, P]),
     "b2u_bn_fold": (I, [P, P, P, P, P, P, P, I, F, P]),

@@ -155,25 +155,28 @@ bn_rows_reduce_kernel(const float* __restrict__ rows, float* __restrict__ out, i
   }
 }
 
-// forward finalize: statistics -> (scale, shift) for the apply pass, saved mean/invstd, running-stat update.
+// (mean, biased variance) of channel c from the column sums of bn_colsum_kernel<0>, combined in fp64 in block order.
 // pivot_z (nullable): z itself when the sums are of z - K with K = row 0 of z (bn_colsum_kernel<0> with pivot set)
-__global__ void bn_fwd_finalize_kernel(const float* __restrict__ partial, const __nv_bfloat16* __restrict__ pivot_z, int blocks, int C, long long P,
-                                       const float* __restrict__ gamma, const float* __restrict__ beta,
-                                       float* __restrict__ running_mean, float* __restrict__ running_var,
-                                       float* __restrict__ save_mean, float* __restrict__ save_invstd,
-                                       float* __restrict__ scale, float* __restrict__ shift, float eps, float momentum,
-                                       int centered) {
-  const int c = blockIdx.x * blockDim.x + threadIdx.x;
-  if (c >= C) return;
+__device__ __forceinline__ void bn_sums_to_moments(const float* __restrict__ partial, const __nv_bfloat16* __restrict__ pivot_z,
+                                                   int blocks, int C, long long P, int c, double* mean, double* var) {
   double s = 0.0, ss = 0.0;
   for (int b = 0; b < blocks; ++b) {
     s += partial[static_cast<size_t>(b) * 2 * C + c];
     ss += partial[static_cast<size_t>(b) * 2 * C + C + c];
   }
   const double ms = s / static_cast<double>(P);      // mean of the shifted values
-  const double mean = (pivot_z ? static_cast<double>(__bfloat162float(pivot_z[c])) : 0.0) + ms;
-  double var = ss / static_cast<double>(P) - ms * ms;
-  if (var < 0.0) var = 0.0;
+  *mean = (pivot_z ? static_cast<double>(__bfloat162float(pivot_z[c])) : 0.0) + ms;
+  const double v = ss / static_cast<double>(P) - ms * ms;
+  *var = v < 0.0 ? 0.0 : v;
+}
+
+// the forward finalize from channel c's statistics over P rows: (scale, shift) for the apply pass, saved mean / invstd,
+// running-statistic update
+__device__ __forceinline__ void bn_fwd_finish(int c, double mean, double var, long long P, const float* __restrict__ gamma,
+                                              const float* __restrict__ beta, float* __restrict__ running_mean,
+                                              float* __restrict__ running_var, float* __restrict__ save_mean,
+                                              float* __restrict__ save_invstd, float* __restrict__ scale,
+                                              float* __restrict__ shift, float eps, float momentum, int centered) {
   const double invstd = 1.0 / sqrt(var + static_cast<double>(eps));
   const float mean_f = static_cast<float>(mean), invstd_f = static_cast<float>(invstd);
   save_mean[c] = mean_f;
@@ -190,6 +193,55 @@ __global__ void bn_fwd_finalize_kernel(const float* __restrict__ partial, const 
     const double unbiased = P > 1 ? var * static_cast<double>(P) / static_cast<double>(P - 1) : var;
     running_var[c] = (1.f - momentum) * running_var[c] + momentum * static_cast<float>(unbiased);
   }
+}
+
+// forward finalize from the column sums of bn_colsum_kernel<0> (`blocks` rows of [2][C])
+__global__ void bn_fwd_finalize_kernel(const float* __restrict__ partial, const __nv_bfloat16* __restrict__ pivot_z, int blocks, int C, long long P,
+                                       const float* __restrict__ gamma, const float* __restrict__ beta,
+                                       float* __restrict__ running_mean, float* __restrict__ running_var,
+                                       float* __restrict__ save_mean, float* __restrict__ save_invstd,
+                                       float* __restrict__ scale, float* __restrict__ shift, float eps, float momentum,
+                                       int centered) {
+  const int c = blockIdx.x * blockDim.x + threadIdx.x;
+  if (c >= C) return;
+  double mean, var;
+  bn_sums_to_moments(partial, pivot_z, blocks, C, P, c, &mean, &var);
+  bn_fwd_finish(c, mean, var, P, gamma, beta, running_mean, running_var, save_mean, save_invstd, scale, shift, eps, momentum,
+                centered);
+}
+
+// SyncBatchNorm, one rank: moments [2][C] = (mean, biased variance) of this rank's rows
+__global__ void bn_moments_kernel(const float* __restrict__ partial, const __nv_bfloat16* __restrict__ pivot_z, int blocks, int C,
+                                  long long P, float* __restrict__ moments) {
+  const int c = blockIdx.x * blockDim.x + threadIdx.x;
+  if (c >= C) return;
+  double mean, var;
+  bn_sums_to_moments(partial, pivot_z, blocks, C, P, c, &mean, &var);
+  moments[c] = static_cast<float>(mean);
+  moments[C + c] = static_cast<float>(var);
+}
+
+// SyncBatchNorm forward finalize from the moments [world][2][C] of `world` ranks of P rows each, combined in fp64 like
+// nn.SyncBatchNorm: mean = mean of the means, var = mean of (var_r + (mean_r - mean)^2); the running variance's unbiased
+// factor counts the rows of all ranks
+__global__ void bn_fwd_finalize_moments_kernel(const float* __restrict__ moments, int world, int C, long long P,
+                                               const float* __restrict__ gamma, const float* __restrict__ beta,
+                                               float* __restrict__ running_mean, float* __restrict__ running_var,
+                                               float* __restrict__ save_mean, float* __restrict__ save_invstd,
+                                               float* __restrict__ scale, float* __restrict__ shift, float eps, float momentum,
+                                               int centered) {
+  const int c = blockIdx.x * blockDim.x + threadIdx.x;
+  if (c >= C) return;
+  double mean = 0.0, var = 0.0;
+  for (int r = 0; r < world; ++r) mean += moments[static_cast<size_t>(r) * 2 * C + c];
+  mean /= world;
+  for (int r = 0; r < world; ++r) {
+    const double d = static_cast<double>(moments[static_cast<size_t>(r) * 2 * C + c]) - mean;
+    var += static_cast<double>(moments[static_cast<size_t>(r) * 2 * C + C + c]) + d * d;
+  }
+  var /= world;
+  bn_fwd_finish(c, mean, var, P * world, gamma, beta, running_mean, running_var, save_mean, save_invstd, scale, shift, eps,
+                momentum, centered);
 }
 
 __global__ void bn_eval_coeff_kernel(const float* __restrict__ gamma, const float* __restrict__ beta,
@@ -388,38 +440,40 @@ int b2u_bn_fwd_train_stats(const void* z, const void* residual, void* y, const f
 }
 
 // ---- SyncBatchNorm building blocks (nn.SyncBatchNorm.convert_sync_batchnorm, train.py:335-336): the statistics pass and the
-// apply pass as separate calls, so the caller can all-reduce the 2C per-layer sums across ranks in between.
-// sums [2][C] fp32 = (sum z, sum z^2) over this rank's P rows.  Unlike b2u_bn_fwd_train these are raw, unshifted sums: the
-// ranks add them up, and a per-rank pivot would not compose.  They keep the one-pass variance's loss of precision when a
-// channel's mean is large against its spread (the centred mode of the producing conv avoids that once running_mean is set).
-int b2u_bn_sums(const void* z, float* sums, void* ws, size_t ws_bytes, long long P, int C, void* stream) {
-  int rc = bn_check(P, C, ws, ws_bytes, "bn_sums");
+// apply pass as separate calls, so the caller can gather the per-rank moments in between.  A per-rank pivot does not survive
+// a sum across ranks, so the ranks exchange moments, not sums, and combine them the way nn.SyncBatchNorm does: each rank's
+// (mean, var) keeps the one-GPU path's accuracy at any channel mean, and so does their combination.
+// moments [2][C] fp32 = (mean, biased variance) of this rank's P rows, from the column sums about the row-0 pivot.
+int b2u_bn_moments(const void* z, float* moments, void* ws, size_t ws_bytes, long long P, int C, void* stream) {
+  int rc = bn_check(P, C, ws, ws_bytes, "bn_moments");
   if (rc) return rc;
+  if (!moments) return set_error(B2U_ERR_ARG, "bn_moments: moments missing");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   float* partial = static_cast<float*>(ws);
   bn_colsum_kernel<0><<<kBnBlocks, 256, 256 * 16 * sizeof(float), st>>>(static_cast<const uint4*>(z), nullptr, nullptr, nullptr,
-                                                                        nullptr, nullptr, nullptr, partial, P, C / 8, 0, 0);
+                                                                        nullptr, nullptr, nullptr, partial, P, C / 8, 0, 1);
   B2U_CHECK_LAUNCH("bn_colsum");
-  bn_rows_reduce_kernel<<<(2 * C + 31) / 32, 256, 0, st>>>(partial, sums, kBnBlocks, 2 * C);
-  B2U_CHECK_LAUNCH("bn_rows_reduce");
+  bn_moments_kernel<<<(C + 127) / 128, 128, 0, st>>>(partial, static_cast<const __nv_bfloat16*>(z), kBnBlocks, C, P, moments);
+  B2U_CHECK_LAUNCH("bn_moments");
   return 0;
 }
 
-// forward from given sums over P_stat rows (all ranks); running statistics and saved mean / invstd are the global ones
-int b2u_bn_fwd_train_sums(const void* z, const void* residual, void* y, const float* gamma, const float* beta,
-                          float* running_mean, float* running_var, float* save_mean, float* save_invstd, const float* sums,
-                          long long P_stat, void* ws, size_t ws_bytes, long long P, int C, float eps, float momentum, int relu,
-                          void* stream) {
-  int rc = bn_check(P, C, ws, ws_bytes, "bn_fwd_train_sums");
+// forward from the gathered moments [world][2][C] of `world` ranks holding P rows each; running statistics and saved
+// mean / invstd are the global ones
+int b2u_bn_fwd_train_moments(const void* z, const void* residual, void* y, const float* gamma, const float* beta,
+                             float* running_mean, float* running_var, float* save_mean, float* save_invstd, const float* moments,
+                             int world, void* ws, size_t ws_bytes, long long P, int C, float eps, float momentum, int relu,
+                             void* stream) {
+  int rc = bn_check(P, C, ws, ws_bytes, "bn_fwd_train_moments");
   if (rc) return rc;
   const int centered = (relu >> 1) & 1;      // bit 1 of `relu`: z is stored centred on the running mean (see finalize)
   relu &= 1;
-  if (!sums || P_stat < P) return set_error(B2U_ERR_ARG, "bn_fwd_train_sums: sums missing or P_stat < P");
+  if (!moments || world < 1) return set_error(B2U_ERR_ARG, "bn_fwd_train_moments: moments missing or world < 1");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   float* coef = static_cast<float*>(ws) + static_cast<size_t>(kBnBlocks) * 2 * C;
-  bn_fwd_finalize_kernel<<<(C + 127) / 128, 128, 0, st>>>(sums, nullptr, 1, C, P_stat, gamma, beta, running_mean, running_var,
-                                                          save_mean, save_invstd, coef, coef + C, eps, momentum, centered);
-  B2U_CHECK_LAUNCH("bn_fwd_finalize");
+  bn_fwd_finalize_moments_kernel<<<(C + 127) / 128, 128, 0, st>>>(moments, world, C, P, gamma, beta, running_mean, running_var,
+                                                                  save_mean, save_invstd, coef, coef + C, eps, momentum, centered);
+  B2U_CHECK_LAUNCH("bn_fwd_finalize_moments");
   const long long G = (P + kBnApplyRows - 1) / kBnApplyRows;
   bn_apply_kernel<<<static_cast<unsigned>((G * (C / 8) + 255) / 256), 256, 0, st>>>(static_cast<const uint4*>(z), static_cast<const uint4*>(residual),
                                                                                    static_cast<uint4*>(y), coef, coef + C, P, G, C / 8, relu);

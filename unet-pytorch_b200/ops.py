@@ -406,8 +406,9 @@ def bn_fwd_train(z, gamma, beta, running_mean, running_var, eps=1e-5, momentum=0
 
 def bn_fwd_train_sync(z, gamma, beta, running_mean, running_var, group, eps=1e-5, momentum=0.1, relu=True, out=None, ws=None,
                       residual=None, centered=False):
-    """SyncBatchNorm forward (train.py:335-336): this rank's column sums, one all-reduce of 2C floats over `group`, apply
-    with the global statistics.  Every rank is assumed to hold the same number of rows (DistributedSampler batches)."""
+    """SyncBatchNorm forward (train.py:335-336): this rank's (mean, biased var), one all-gather of 2C floats per rank over
+    `group`, apply with the combined statistics.  Every rank is assumed to hold the same number of rows (DistributedSampler
+    batches)."""
     import torch.distributed as dist
     _req(z, ACT, "z")
     C = z.shape[-1]
@@ -417,15 +418,16 @@ def bn_fwd_train_sync(z, gamma, beta, running_mean, running_var, group, eps=1e-5
         ws = _ws(need, z.device)
     if out is None:
         out = torch.empty_like(z)
-    sums = torch.empty((2, C), dtype=torch.float32, device=z.device)
-    check(lib().b2u_bn_sums(ptr(z), ptr(sums), ptr(ws), ws.numel() * ws.element_size(), P, C, stream_ptr()))
-    dist.all_reduce(sums, group=group)
+    mine = torch.empty((2, C), dtype=torch.float32, device=z.device)
+    check(lib().b2u_bn_moments(ptr(z), ptr(mine), ptr(ws), ws.numel() * ws.element_size(), P, C, stream_ptr()))
     world = dist.get_world_size(group)
+    moments = torch.empty((world, 2, C), dtype=torch.float32, device=z.device)
+    dist.all_gather(list(moments.unbind(0)), mine, group=group)
     mean = torch.empty((C,), dtype=torch.float32, device=z.device)
     invstd = torch.empty((C,), dtype=torch.float32, device=z.device)
-    check(lib().b2u_bn_fwd_train_sums(ptr(z), ptr(residual), ptr(out), ptr(gamma), ptr(beta), ptr(running_mean), ptr(running_var),
-                                      ptr(mean), ptr(invstd), ptr(sums), P * world, ptr(ws), ws.numel() * ws.element_size(), P, C, eps,
-                                      momentum, (1 if relu else 0) | (2 if centered else 0), stream_ptr()))
+    check(lib().b2u_bn_fwd_train_moments(ptr(z), ptr(residual), ptr(out), ptr(gamma), ptr(beta), ptr(running_mean), ptr(running_var),
+                                         ptr(mean), ptr(invstd), ptr(moments), world, ptr(ws), ws.numel() * ws.element_size(), P, C,
+                                         eps, momentum, (1 if relu else 0) | (2 if centered else 0), stream_ptr()))
     return out, mean, invstd
 
 
