@@ -133,6 +133,21 @@ int b2u_conv_wgrad(const void* x0, int C0, const void* x1, int C1, const void* d
 size_t b2u_bias_grad_workspace(int C);
 int b2u_bias_grad(const void* dz, float* db, void* ws, size_t ws_bytes, long long P, int C, void* stream);
 
+/* ---- gradient wrt the input image (x.grad of the drop-in modules, autograd of the first layer's nn.Conv2d) ------ */
+/* dx (NCHW fp32 [N][Cin][H][W], overwritten) = data gradient of the first 3x3 s1 p1 conv (nets/vgg.py:53,
+ * nets/TraditionalUnet.py:9), the one run over b2u_im2col_first rows: dz [N,H,W,Cz] = the gradient wrt its output (ReLU-masked
+ * or from the BatchNorm backward), w = its fp32 OIHW weight [Cout][Cin][3][3] (Cout <= Cz, Cz % 16 == 0, 9 Cin <= 64).  The
+ * gradient wrt the image is that of the hi columns of the two-term split alone.  Any H, W; dz (and x below) 16-byte aligned
+ * (B2U_ERR_ARG otherwise). */
+int b2u_first_conv_dgrad_input(const void* dz, int Cz, const float* w, float* dx, int N, int Cin, int H, int W, int Cout,
+                               void* stream);
+/* the same for the 7x7 s2 p3 ResNet stem (nets/resnet.py:109) run over b2u_im2col_stem rows: dz [N,ceil(H/2),ceil(W/2),Cz],
+ * w [Cout][Cin][7][7] (49 Cin <= 192); H, W = the image's */
+int b2u_stem_dgrad_input(const void* dz, int Cz, const float* w, float* dx, int N, int Cin, int H, int W, int Cout, void* stream);
+/* channels [0, C) of an NHWC tensor [N,H,W,Cpad] -> NCHW fp32 [N][C][H][W]: the gradient wrt an image that entered through
+ * b2u_nchw_f32_to_nhwc_bf16_padded (channels [C, 2C) hold the lo half of its split and carry the same gradient) */
+int b2u_nhwc_bf16_padded_to_nchw_f32(const void* x, float* y, int N, int C, int H, int W, int Cpad, void* stream);
+
 /* ---- pooling / upsampling ---------------------------------------------------------------------------------- */
 /* nn.MaxPool2d(2, 2) (nets/vgg.py:51).  H, W = dims of the un-pooled tensor. */
 int b2u_maxpool2x2_fwd(const void* x, void* y, int N, int H, int W, int C, void* stream);

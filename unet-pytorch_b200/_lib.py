@@ -52,6 +52,9 @@ SIGNATURES = {
     "b2u_conv_wgrad": (I, [P, I, P, I, P, I, P, P, P, SZ, I, I, I, I, I, I, P]),
     "b2u_bias_grad_workspace": (SZ, [I]),
     "b2u_bias_grad": (I, [P, P, P, SZ, LL, I, P]),
+    "b2u_first_conv_dgrad_input": (I, [P, I, P, P, I, I, I, I, I, P]),
+    "b2u_stem_dgrad_input": (I, [P, I, P, P, I, I, I, I, I, P]),
+    "b2u_nhwc_bf16_padded_to_nchw_f32": (I, [P, P, I, I, I, I, I, P]),
     "b2u_maxpool2x2_fwd": (I, [P, P, I, I, I, I, P]),
     "b2u_maxpool2x2_bwd": (I, [P, P, P, P, I, I, I, I, I, P]),
     "b2u_upsample2x_fwd": (I, [P, P, I, I, I, I, P]),

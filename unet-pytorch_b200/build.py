@@ -18,7 +18,7 @@ OUT_FP32 = os.path.join(HERE, "libb200unet_fp32.so")
 SOURCES_FP32 = ["runtime.cu", "head_loss.cu", "hist.cu", "optim.cu", "dw_se.cu", "letterbox.cu", "render.cu",
                 "validation_fp32.cu"]
 SOURCES = ["runtime.cu", "conv_igemm.cu", "conv_wgrad.cu", "elementwise.cu", "head_loss.cu", "hist.cu", "optim.cu", "bn.cu", "resnet_ops.cu", "dw_se.cu",
-           "letterbox.cu", "render.cu"]
+           "letterbox.cu", "render.cu", "input_grad.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "-Xptxas=-v",  # no --use_fast_math: precise math everywhere; -v prints registers/spills

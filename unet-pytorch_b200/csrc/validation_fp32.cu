@@ -701,6 +701,41 @@ __global__ void v32_nchw_to_nhwc_padded_kernel(const float* __restrict__ x, floa
   const long long n = p / HW, hw = p % HW;
   y[idx] = c < C ? x[(n * C + c) * HW + hw] : 0.f;
 }
+// the gradient wrt the input image (input_grad.cu in fp32): one thread per NCHW output element, gather over (co, tap)
+// dx[n,c,h,w] = sum over co and the taps (r, s) with (h + pad - r) and (w + pad - s) divisible by the stride of
+// dz[n, (h+pad-r)/stride, (w+pad-s)/stride, co] * W[co,c,r,s]
+__global__ void v32_conv_dgrad_input_kernel(const float* __restrict__ dz, int Cz, const float* __restrict__ w, float* __restrict__ dx,
+                                            int N, int Cin, int H, int W, int Hz, int Wz, int Cout, int K, int stride, int pad) {
+  const long long idx = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (idx >= static_cast<long long>(N) * Cin * H * W) return;
+  const int x = static_cast<int>(idx % W);
+  long long t = idx / W;
+  const int y = static_cast<int>(t % H); t /= H;
+  const int c = static_cast<int>(t % Cin);
+  const int n = static_cast<int>(t / Cin);
+  float acc = 0.f;
+  for (int r = 0; r < K; ++r) {
+    const int hs = y + pad - r;
+    if (hs < 0 || hs % stride) continue;
+    const int hz = hs / stride;
+    if (hz >= Hz) continue;
+    for (int s = 0; s < K; ++s) {
+      const int ws = x + pad - s;
+      if (ws < 0 || ws % stride) continue;
+      const int wz = ws / stride;
+      if (wz >= Wz) continue;
+      const float* g = dz + ((static_cast<size_t>(n) * Hz + hz) * Wz + wz) * Cz;
+      for (int co = 0; co < Cout; ++co) acc = fmaf(g[co], w[((static_cast<size_t>(co) * Cin + c) * K + r) * K + s], acc);
+    }
+  }
+  dx[idx] = acc;
+}
+__global__ void v32_nhwc_padded_to_nchw_kernel(const float* __restrict__ x, float* __restrict__ y, int N, int C, long long HW, int Cpad) {
+  const long long idx = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (idx >= static_cast<long long>(N) * C * HW) return;
+  const long long hw = idx % HW, nc = idx / HW;
+  y[idx] = x[((nc / C) * HW + hw) * Cpad + nc % C];
+}
 // F.interpolate(x, size, mode="bilinear", align_corners=True) on NCHW fp32 planes, and its adjoint (gather form)
 __global__ void v32_resize_fwd_kernel(const float* __restrict__ x, float* __restrict__ y, long long NC, int Hi, int Wi, int Ho, int Wo,
                                       float sh, float sw) {
@@ -1163,6 +1198,35 @@ int b2u_nchw_f32_to_nhwc_bf16_padded(const float* x, void* y, int N, int C, int 
   v32_nchw_to_nhwc_padded_kernel<<<blocks_for(N * HW * Cpad, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(x, static_cast<float*>(y), N, C,
                                                                                                               HW, Cpad);
   B2U_CHECK_LAUNCH("nchw_to_nhwc_padded_fp32");
+  return 0;
+}
+int b2u_first_conv_dgrad_input(const void* dz, int Cz, const float* w, float* dx, int N, int Cin, int H, int W, int Cout,
+                               void* stream) {
+  if (N <= 0 || H <= 0 || W <= 0 || Cin <= 0 || 9 * Cin > 64 || Cout <= 0 || Cout > Cz || Cz % 16 != 0)
+    return set_error(B2U_ERR_SHAPE, "first_conv_dgrad_input: bad shape (Cin=%d Cout=%d Cz=%d)", Cin, Cout, Cz);
+  if (reinterpret_cast<uintptr_t>(dz) % 16 != 0) return set_error(B2U_ERR_ARG, "first_conv_dgrad_input: dz must be 16-byte aligned");
+  v32_conv_dgrad_input_kernel<<<blocks_for(static_cast<long long>(N) * Cin * H * W, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+      static_cast<const float*>(dz), Cz, w, dx, N, Cin, H, W, H, W, Cout, 3, 1, 1);
+  B2U_CHECK_LAUNCH("first_conv_dgrad_input_fp32");
+  return 0;
+}
+int b2u_stem_dgrad_input(const void* dz, int Cz, const float* w, float* dx, int N, int Cin, int H, int W, int Cout, void* stream) {
+  if (N <= 0 || H <= 0 || W <= 0 || Cin <= 0 || 49 * Cin > 192 || Cout <= 0 || Cout > Cz || Cz % 16 != 0)
+    return set_error(B2U_ERR_SHAPE, "stem_dgrad_input: bad shape (Cin=%d Cout=%d Cz=%d)", Cin, Cout, Cz);
+  if (reinterpret_cast<uintptr_t>(dz) % 16 != 0) return set_error(B2U_ERR_ARG, "stem_dgrad_input: dz must be 16-byte aligned");
+  v32_conv_dgrad_input_kernel<<<blocks_for(static_cast<long long>(N) * Cin * H * W, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+      static_cast<const float*>(dz), Cz, w, dx, N, Cin, H, W, (H - 1) / 2 + 1, (W - 1) / 2 + 1, Cout, 7, 2, 3);
+  B2U_CHECK_LAUNCH("stem_dgrad_input_fp32");
+  return 0;
+}
+int b2u_nhwc_bf16_padded_to_nchw_f32(const void* x, float* y, int N, int C, int H, int W, int Cpad, void* stream) {
+  if (N <= 0 || C <= 0 || H <= 0 || W <= 0 || Cpad < C || Cpad % 8 != 0)
+    return set_error(B2U_ERR_SHAPE, "nhwc_bf16_padded_to_nchw_f32: bad shape (C=%d Cpad=%d)", C, Cpad);
+  if (reinterpret_cast<uintptr_t>(x) % 16 != 0) return set_error(B2U_ERR_ARG, "nhwc_bf16_padded_to_nchw_f32: x must be 16-byte aligned");
+  const long long HW = static_cast<long long>(H) * W;
+  v32_nhwc_padded_to_nchw_kernel<<<blocks_for(N * C * HW, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+      static_cast<const float*>(x), y, N, C, HW, Cpad);
+  B2U_CHECK_LAUNCH("nhwc_padded_to_nchw_fp32");
   return 0;
 }
 int b2u_resize_bilinear_f32_fwd(const float* x, float* y, long long NC, int Hi, int Wi, int Ho, int Wo, void* stream) {

@@ -18,6 +18,9 @@ dgrad epilogue and the weight-gradient side stream.
 Channel counts that are not multiples of 64 (the 32-channel layers of TraditionalUnet) are zero-padded to 64 in the
 activation buffers and operands; padded channels stay exactly zero in both directions.
 
+backward(dx=...) also returns the gradient wrt the input image: every layer then runs its data gradient (weight gradients
+still follow `trainable`), and the first conv's data gradient, b2u_first_conv_dgrad_input, writes it as NCHW fp32.
+
 Gradients are written straight into caller-provided fp32 OIHW tensors (normally views of one flat buffer), and
 `on_grads_ready(names)` is called after the launches that complete each layer's gradients so a data-parallel
 trainer can start that bucket's all-reduce while the remaining dgrad/wgrad kernels still run.
@@ -248,10 +251,10 @@ class UNetEngine(EngineBase):
         return out
 
     # ------------------------------------------------------------------ forward
-    def forward(self, x, params, save=True, training=None, trainable=None):
+    def forward(self, x, params, save=True, training=None, trainable=None, input_grad=False):
         """x: NCHW fp32 CUDA [N, Cin, H, W] -> logits NCHW fp32.  training (BN nets): batch statistics + running-stat
-        update (default: same as `save`).  trainable is accepted for interface parity with GraphEngine (backward decides
-        what to skip from the gradient names it is given)."""
+        update (default: same as `save`).  trainable and input_grad are accepted for interface parity with GraphEngine
+        (backward decides what to skip from the gradient names it is given, and whether to reach the image from its dx)."""
         if not x.is_cuda:
             raise ValueError("UNetEngine.forward: input must be a CUDA tensor (no CPU fallback)")
         if x.dtype != torch.float32:
@@ -307,10 +310,11 @@ class UNetEngine(EngineBase):
         return logits
 
     # ------------------------------------------------------------------ backward
-    def backward(self, dlogits, params, grads, trainable=None, on_grads_ready=None):
+    def backward(self, dlogits, params, grads, trainable=None, on_grads_ready=None, dx=None):
         """dlogits: NCHW fp32, or bf16 [N,H,W,64] from ops.loss_bwd(nhwc64=True).  grads: name -> fp32 tensor to
-        overwrite (missing / not in `trainable`: skipped).
-        Returns nothing; the input image gets no gradient (the reference never asks for one)."""
+        overwrite (missing / not in `trainable`: skipped).  dx (optional): NCHW fp32 buffer shaped like the input, which
+        receives the gradient wrt the image (x.grad); every layer then runs its data gradient, frozen ones included, while
+        weight gradients still follow `trainable`."""
         if self.saved is None:
             raise RuntimeError("backward() without a saved forward()")
         # Weight/bias gradients on a second stream (plain conv+ReLU nets): wgrad_L depends only on dz_L and the saved
@@ -338,12 +342,12 @@ class UNetEngine(EngineBase):
             self._workspace("bias", ops.lib().b2u_bias_grad_workspace(max(c.cout_p for c in self.convs)))
             side.wait_stream(torch.cuda.current_stream())
         try:
-            self._backward(dlogits, params, grads, trainable, on_grads_ready, side)
+            self._backward(dlogits, params, grads, trainable, on_grads_ready, side, dx)
         finally:
             if side is not None:
                 torch.cuda.current_stream().wait_stream(side)      # optimizer / next forward see every gradient
 
-    def _backward(self, dlogits, params, grads, trainable, on_grads_ready, side):
+    def _backward(self, dlogits, params, grads, trainable, on_grads_ready, side, dx):
         A, feats, (N, H, W) = self.saved
         if trainable is None:
             trainable = set(grads.keys())
@@ -355,11 +359,11 @@ class UNetEngine(EngineBase):
             return any(n in trainable for n in names)
         want = {c.name: wanted(c) for c in self.convs}
         want[self.head_name] = (self.head_name + ".weight") in trainable or (self.head_name + ".bias") in trainable
-        # data gradients are needed down to the first (in execution order) trainable conv
-        first_trainable = next((i for i, n in enumerate(order) if want[n]), len(order))
+        # data gradients are needed down to the first (in execution order) trainable conv, or to the image
+        first_trainable = -1 if dx is not None else next((i for i, n in enumerate(order) if want[n]), len(order))
         need_dx = {n: i > first_trainable for i, n in enumerate(order)}   # does layer n have to produce dx?
         n_enc = sum(len(b) for b in self.enc)
-        enc_trainable = first_trainable < n_enc
+        enc_trainable = first_trainable < n_enc       # the encoder's features need their skip gradients
 
         def ready(*names):
             if on_grads_ready is not None:
@@ -471,6 +475,8 @@ class UNetEngine(EngineBase):
                     nxt = self._buf("g:" + block[ci - 1].name, xin.shape)
                     dgrad_to(block[ci - 1], dz, c.wd, c.c0_p, None if bn else xin, nxt)
                     g = nxt
+                elif bi == 0:
+                    ops.first_conv_dgrad_input(dz, params[c.name + ".weight"], out=dx)
                 else:
                     dpool = self._buf(f"g:pool{bi}", xin.shape)
                     ops.conv_dgrad(dz, c.wd, c.c0_p, out0=dpool)

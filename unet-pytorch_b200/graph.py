@@ -453,7 +453,9 @@ class GraphEngine(EngineBase):
         self._pack_versions = versions
 
     # ------------------------------------------------------------------ forward
-    def forward(self, x, params, save=True, training=None, trainable=None):
+    def forward(self, x, params, save=True, training=None, trainable=None, input_grad=False):
+        """input_grad: backward() will be asked for the gradient wrt x, so the image (the input instruction's tensor, or
+        the stem's output) needs a gradient and every layer between it and the loss runs its data gradient."""
         if not x.is_cuda:
             raise ValueError("GraphEngine.forward: input must be a CUDA tensor (no CPU fallback)")
         x = x.float().contiguous() if x.dtype != torch.float32 else x.contiguous()
@@ -476,12 +478,13 @@ class GraphEngine(EngineBase):
                 shift = self._center_shift(ins, params, training, 64)
                 sbias = torch.neg(shift, out=self._buf("bc:" + ins["w"], (64,), torch.float32)) if shift is not None else None
                 ops.conv_fprop(col, self._stem_wf, sbias, 64, taps=1, relu=False, out=z)
-                t = _T(z, needs_grad=ins["w"] in trainable)
+                t = _T(z, needs_grad=ins["w"] in trainable or input_grad)
                 t.centered = shift is not None
                 t.aux = col
                 T[ins["out"]] = t
             elif op == "input":
-                T[ins["out"]] = _T(ops.nchw_to_nhwc_bf16_padded(x, 64, out=self._buf("x", (N, H, W, 64))))      # hi | lo split when 2C <= 64
+                T[ins["out"]] = _T(ops.nchw_to_nhwc_bf16_padded(x, 64, out=self._buf("x", (N, H, W, 64))),      # hi | lo split when 2C <= 64
+                                   needs_grad=input_grad)
             elif op == "conv":
                 xin = T[ins["x"]]
                 x1 = T[ins["x1"]] if ins["x1"] else None
@@ -644,7 +647,7 @@ class GraphEngine(EngineBase):
             elif op == "head":
                 logits = self._head_fwd(T[ins["x"]].data, params, ins["w"], ins["bias"], ins.get("cin", 64))
         if save:
-            self.saved = (T, (N, H, W), set(trainable))
+            self.saved = (T, (N, H, W), set(trainable), input_grad)
         return logits
 
     # ------------------------------------------------------------------ backward
@@ -654,10 +657,14 @@ class GraphEngine(EngineBase):
         else:
             ops.add_bf16(t.grad, g, out=t.grad)
 
-    def backward(self, dlogits, params, grads, trainable=None, on_grads_ready=None):
+    def backward(self, dlogits, params, grads, trainable=None, on_grads_ready=None, dx=None):
+        """grads: name -> fp32 tensor to overwrite (missing / not in `trainable`: skipped).  dx (optional, needs a forward
+        with input_grad=True): NCHW fp32 buffer shaped like the input, receives the gradient wrt the image."""
         if self.saved is None:
             raise RuntimeError("backward() without a saved forward()")
-        T, (N, H, W), fwd_trainable = self.saved
+        T, (N, H, W), fwd_trainable, input_grad = self.saved
+        if dx is not None and not input_grad:
+            raise RuntimeError("backward(dx=...) needs a forward(input_grad=True)")
         if trainable is None:
             trainable = set(grads.keys())
         for t in T.values():
@@ -670,6 +677,7 @@ class GraphEngine(EngineBase):
             if on_grads_ready is not None:
                 on_grads_ready([n for n in names if n in grads])
 
+        dx_written = False
         for ins in reversed(self.program):
             op = ins["op"]
             if op == "head":
@@ -717,9 +725,10 @@ class GraphEngine(EngineBase):
                 if t.grad is None or not xin.needs_grad:
                     continue
                 if t.aux is None:
-                    self._acc(xin, t.grad)
+                    g = t.grad
                 else:
-                    self._acc(xin, ops.scale_nc(t.grad, t.aux, out=self._buf("g:" + ins["out"] + ">", xin.data.shape)))
+                    g = ops.scale_nc(t.grad, t.aux, out=self._buf("g:" + ins["out"] + ">", xin.data.shape))
+                self._acc(xin, self._relu_mask(xin, g, ins["out"]))
             elif op == "se":
                 t, xin = T[ins["out"]], T[ins["x"]]
                 if t.grad is None:
@@ -735,7 +744,8 @@ class GraphEngine(EngineBase):
                                         dw2=grads[names[2]] if has(names[2]) else None, db2=grads[names[3]] if has(names[3]) else None)
                 ready(*names)
                 if xin.needs_grad:
-                    self._acc(xin, ops.scale_nc(t.grad, sc, add=dpooled, out=self._buf("g:" + ins["out"] + ">", xin.data.shape)))
+                    g = ops.scale_nc(t.grad, sc, add=dpooled, out=self._buf("g:" + ins["out"] + ">", xin.data.shape))
+                    self._acc(xin, self._relu_mask(xin, g, ins["out"]))
             elif op == "dw":
                 t, xin = T[ins["out"]], T[ins["x"]]
                 if t.grad is None:
@@ -867,12 +877,31 @@ class GraphEngine(EngineBase):
                     self._acc(xin, d0)
             elif op == "stem":
                 t = T[ins["out"]]
-                if t.grad is None or not has(ins["w"]):
+                if t.grad is None:
                     continue
-                col = t.aux
-                need = ops.lib().b2u_conv_wgrad_workspace(col.shape[0], col.shape[1], col.shape[2], 192, 64, 1)
-                ops.conv_wgrad_im2col(col, t.grad, 3, 49, dw=grads[ins["w"]], ws=self._workspace("wgrad", need))
-                ready(ins["w"])
+                if has(ins["w"]):
+                    col = t.aux
+                    need = ops.lib().b2u_conv_wgrad_workspace(col.shape[0], col.shape[1], col.shape[2], 192, 64, 1)
+                    ops.conv_wgrad_im2col(col, t.grad, 3, 49, dw=grads[ins["w"]], ws=self._workspace("wgrad", need))
+                    ready(ins["w"])
+                if dx is not None:
+                    ops.stem_dgrad_input(t.grad, params[ins["w"]], H, W, out=dx)
+                    dx_written = True
+            elif op == "input":
+                t = T[ins["out"]]
+                if dx is not None and t.grad is not None:
+                    # channels [C, 2C) (the lo half of the image split) meet the same weights: their gradient equals [0, C)'s
+                    ops.nhwc_padded_to_nchw_f32(t.grad, ins["c"], out=dx)
+                    dx_written = True
+        if dx is not None and not dx_written:
+            dx.zero_()          # no path from the image reached the loss: its gradient is zero, not whatever dx held
+
+    def _relu_mask(self, t, g, key):
+        """g, a gradient for t, made wrt t's pre-activation when t is a fused-ReLU conv output (ImprovedSegNet's deploy form
+        feeds those to SE and Dropout2d, which cannot mask in their own pass)."""
+        if not t.fused_relu:
+            return g
+        return ops.relu_bwd(g, t.data, out=self._buf("g:" + key + ">relu", g.shape))
 
     def _acc_masked(self, t, g):
         """Gradient from a split (two-output) dgrad, which cannot mask in its epilogue."""

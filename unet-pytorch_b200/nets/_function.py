@@ -12,19 +12,22 @@ class EngineFunction(torch.autograd.Function):
         tensors = dict(zip(names, params))
         tensors.update(module._named_buffer_tensors())        # BatchNorm running statistics (updated in place)
         needs = any(ctx.needs_input_grad[2:])
+        input_grad = ctx.needs_input_grad[1]          # x.grad: saliency maps, adversarial inputs, trainable modules in front
         trainable = {n for n, need in zip(names, ctx.needs_input_grad[2:]) if need}
         if needs or module.training:
             # parameters of a training module change between calls (optimizer steps, and in-place `.data` writes such as
             # weights_init / EMA that do not bump Tensor._version): always re-pack the bf16 operands (one launch)
             engine.invalidate_packed_weights()
-        logits = engine.forward(x, tensors, save=needs, training=module.training, trainable=trainable)
-        if needs:
+        save = needs or input_grad
+        logits = engine.forward(x, tensors, save=save, training=module.training, trainable=trainable, input_grad=input_grad)
+        if save:
             engine._generation = getattr(engine, "_generation", 0) + 1
             ctx.generation = engine._generation
             ctx.engine = engine
             ctx.names = names
             ctx.params = params
             ctx.tensors = tensors
+            ctx.x_meta = (x.shape, x.dtype)
         return logits
 
     @staticmethod
@@ -35,8 +38,14 @@ class EngineFunction(torch.autograd.Function):
         # zero-initialised: a gradient the engine legitimately leaves untouched (a tensor that cannot receive one) reads as
         # 0, never as uninitialised memory
         grads = {n: torch.zeros_like(p) for n, p, need in zip(ctx.names, ctx.params, ctx.needs_input_grad[2:]) if need}
-        engine.backward(dlogits, ctx.tensors, grads)
-        return (None, None) + tuple(grads.get(n) for n in ctx.names)
+        dx = None
+        if ctx.needs_input_grad[1]:
+            shape, dtype = ctx.x_meta
+            dx = torch.empty(shape, dtype=torch.float32, device=dlogits.device)
+        engine.backward(dlogits, ctx.tensors, grads, dx=dx)
+        if dx is not None and dtype != torch.float32:
+            dx = dx.to(dtype)
+        return (None, dx) + tuple(grads.get(n) for n in ctx.names)
 
 
 class EngineModuleMixin:

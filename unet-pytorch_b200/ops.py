@@ -168,6 +168,54 @@ def nchw_to_nhwc_bf16_padded(x, cpad, out=None):
     return out
 
 
+# ---------------------------------------------------------------------------------------------- gradient wrt the image
+def _image_grad_out(out, shape, device):
+    if out is None:
+        return torch.empty(shape, dtype=torch.float32, device=device)
+    _req(out, torch.float32, "dx")
+    if tuple(out.shape) != tuple(shape):
+        raise ValueError(f"dx: expected shape {tuple(shape)}, got {tuple(out.shape)}")
+    return out
+
+
+def first_conv_dgrad_input(dz, w, out=None):
+    """Gradient wrt the NCHW fp32 image of the first 3x3 conv (the one over im2col_first rows): dz [N,H,W,Cz] (gradient wrt
+    its output), w fp32 OIHW [Cout, Cin, 3, 3] -> dx [N, Cin, H, W] fp32."""
+    N, H, W, Cz = dz.shape
+    Cout, Cin, kh, kw = w.shape
+    if (kh, kw) != (3, 3):
+        raise ValueError("first_conv_dgrad_input: expected a 3x3 weight")
+    _req(dz, ACT, "dz"); _req(w, torch.float32, "weight")
+    out = _image_grad_out(out, (N, Cin, H, W), dz.device)
+    check(lib().b2u_first_conv_dgrad_input(ptr(dz), Cz, ptr(w), ptr(out), N, Cin, H, W, Cout, stream_ptr()))
+    return out
+
+
+def stem_dgrad_input(dz, w, H, W, out=None):
+    """Gradient wrt the H x W NCHW fp32 image of the 7x7 stride-2 stem: dz [N, ceil(H/2), ceil(W/2), Cz], w fp32
+    [Cout, Cin, 7, 7] -> dx [N, Cin, H, W] fp32."""
+    N, Ho, Wo, Cz = dz.shape
+    Cout, Cin, kh, kw = w.shape
+    if (kh, kw) != (7, 7) or (Ho, Wo) != ((H + 1) // 2, (W + 1) // 2):
+        raise ValueError("stem_dgrad_input: expected a 7x7 weight and dz at half the image size")
+    _req(dz, ACT, "dz"); _req(w, torch.float32, "weight")
+    out = _image_grad_out(out, (N, Cin, H, W), dz.device)
+    check(lib().b2u_stem_dgrad_input(ptr(dz), Cz, ptr(w), ptr(out), N, Cin, H, W, Cout, stream_ptr()))
+    return out
+
+
+def nhwc_padded_to_nchw_f32(x, C, out=None):
+    """Channels [0, C) of NHWC x [N,H,W,Cpad] -> NCHW fp32 [N, C, H, W] (the gradient wrt an image that entered through
+    nchw_to_nhwc_bf16_padded)."""
+    N, H, W, Cpad = x.shape
+    if not 0 < C <= Cpad:
+        raise ValueError(f"nhwc_padded_to_nchw_f32: C = {C} must be in [1, {Cpad}]")
+    _req(x, ACT, "x")
+    out = _image_grad_out(out, (N, C, H, W), x.device)
+    check(lib().b2u_nhwc_bf16_padded_to_nchw_f32(ptr(x), ptr(out), N, C, H, W, Cpad, stream_ptr()))
+    return out
+
+
 # ---------------------------------------------------------------------------------------------- convs
 def conv_fprop(x0, wf, bias, Cout, taps=9, relu=True, x1=None, out=None, bn=0, stats=None):
     """stats: optional fp32 buffer [>= conv_stat_rows(...)][2][Cout]; the conv then also writes the per-tile sums of z and
